@@ -1,15 +1,13 @@
 """GPU parity at the BASELINE.json sizes (through the C ABI).
 
-  configs[1]  P = 1000, 64-beam scan (143k points), 30 iterations: against the REFERENCE ITSELF running on this GPU
-              (oracle/_ref/libsvnicp_ref_cuda.so = its unmodified sources + its vendored knn.cu), asserted.
+  configs[1]  P = 1000, 64-beam scan (143k points), 30 iterations: against the stored outputs of that scan
+              (tests/golden/bench_full_p1000.npz): the particle mean of the REFERENCE ITSELF run on a B200 (its unmodified
+              sources + its vendored knn.cu) and the particles of the fp64 oracle, asserted.
   configs[2]  P = 4096 (16 particle groups), 128-beam scan (~250k points): correspondence indices bit-exact and a short scan
               against the fp64 oracle on a 4096-point subsample of that scan; the full-size scan through size-independent
               properties (deterministic, finite, recovers the planted motion, history consistent with the particles).
 """
-import json
 import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
@@ -23,29 +21,34 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 POSE_TOL = 1e-5
 
 
-def test_config1_full_size_against_the_reference_on_this_gpu(tmp_path):
+def check_golden_inputs(g, pb, src):
+    """The seeded bench problem is still the one the golden outputs were computed on (tests/golden/make_golden_bench.py)."""
+    np.testing.assert_array_equal(g["in_n"], [len(src), len(pb.target)])
+    for k, v in (("in_gt_rel", pb.gt_rel), ("in_R0", pb.R0), ("in_t0", pb.t0), ("in_init_pose", pb.init_pose)):
+        np.testing.assert_allclose(v, g[k], rtol=0, atol=1e-12, err_msg=k)
+    np.testing.assert_allclose(src.sum(0), g["in_source_sum"], rtol=1e-12, err_msg="source")
+    np.testing.assert_allclose(pb.target.sum(0), g["in_target_sum"], rtol=1e-12, err_msg="target")
+
+
+def test_config1_full_size_against_the_reference_on_this_gpu():
     """Per-particle poses <= 5e-5, particle mean <= 1e-5 after 30 iterations at P = 1000, N_s = 143k (near-tie
-    correspondence flips -- 1.6e-6 of the pairs -- compound through the repulsive dynamics, hence the per-particle bar)."""
+    correspondence flips -- 1.6e-6 of the pairs -- compound through the repulsive dynamics, hence the per-particle bar).
+    Against tests/golden/bench_full_p1000.npz: the particle mean of the reference's own sources run on a B200 on this scan,
+    and the particles of the fp64 C restatement on the same scan."""
     import bench
-    if not orc.ref_cuda_available():
-        pytest.skip("oracle/_ref/libsvnicp_ref_cuda.so not built (needs /root/reference at build time)")
+    g = np.load(os.path.join(ROOT, "tests", "golden", "bench_full_p1000.npz"))
     P, I = 1000, 30
-    out_npy = os.path.join(tmp_path, "ref_particles.npy")
-    r = subprocess.run([sys.executable, "-m", "oracle.ref_gpu_run", str(P), str(I), "0", out_npy], cwd=ROOT, capture_output=True, text=True,
-                       timeout=900)
-    info = json.loads(r.stdout.strip().splitlines()[-1])
-    if not info.get("ok"):
-        pytest.skip(f"the reference could not run the full-size scan on this box: {info}")
     pb, _ = bench.make_problem(P)
+    check_golden_inputs(g, pb, pb.source)
     W = bench.WORKLOAD
     icp = sv.SVNICP(sv.SteinICPParam(iterations=I, KNN_count=W["K"], max_dist=W["max_dist"], lr=W["lr"], SVN_full_grad=True), pb.init_pose)
     icp.add_cloud(pb.source, pb.target, pb.init_pose)
     icp.set_initial_mean(pb.R0, pb.t0)
     assert icp.stein_align() == sv.ALIGN_SUCCESS
-    theirs = np.load(out_npy)
     ours = icp.get_particles().reshape(6, P)
-    np.testing.assert_allclose(ours, theirs, atol=5 * POSE_TOL, rtol=0)
-    np.testing.assert_allclose(icp.get_transformation(), np.array(info["mean"]), atol=POSE_TOL, rtol=0)
+    np.testing.assert_allclose(ours, g["oracle_particles"], atol=5 * POSE_TOL, rtol=0)
+    np.testing.assert_allclose(icp.get_transformation(), g["reference_mean"], atol=POSE_TOL, rtol=0)
+    np.testing.assert_allclose(icp.get_transformation(), g["oracle_mean"], atol=POSE_TOL, rtol=0)
 
 
 @pytest.fixture(scope="module")

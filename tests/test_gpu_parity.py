@@ -397,31 +397,23 @@ def test_set_k_keeps_the_clouds(oracle, small):
     np.testing.assert_array_equal(idx, oidx)
 
 
-def test_against_the_reference_running_on_this_gpu(tmp_path):
-    """The reference's OWN sources + its vendored knn.cu built against libtorch CUDA (oracle/_ref/libsvnicp_ref_cuda.so, built
-    where /root/reference exists) run the same scan on this GPU in a subprocess; our particles must agree within the scan
-    tolerance and the mean within POSE_TOL.  (bench.py reports the same figure at the full BASELINE size.)"""
-    import json
+def test_bench_subsample_against_stored_fp64_scan():
+    """The bench problem (64-beam scan against its voxel map, K = 100) on a 6000-point subsample, P = 64, 12 iterations, against
+    the stored fp64 oracle outputs of the same scan (tests/golden/bench_sub6000_p64.npz, make_golden_bench.py): our particles
+    must agree within the scan tolerance and the mean within POSE_TOL.  (tests/test_gpu_fullsize.py checks the full BASELINE size.)"""
     import os
-    import subprocess
-    import sys
     import bench
-    if not orc.ref_cuda_available():
-        pytest.skip("oracle/_ref/libsvnicp_ref_cuda.so not built")
+    from test_gpu_fullsize import check_golden_inputs
+    g = np.load(os.path.join(bench.ROOT, "tests", "golden", "bench_sub6000_p64.npz"))
     P, I, cap = 64, 12, 6000
-    out_npy = os.path.join(tmp_path, "ref_particles.npy")
-    r = subprocess.run([sys.executable, "-m", "oracle.ref_gpu_run", str(P), str(I), str(cap), out_npy], cwd=bench.ROOT, capture_output=True,
-                       text=True, timeout=600)
-    info = json.loads(r.stdout.strip().splitlines()[-1])
-    assert info.get("ok"), info
     pb, _ = bench.make_problem(P)
     src = bench._subsample(pb, cap)
+    check_golden_inputs(g, pb, src)
     W = bench.WORKLOAD
     icp = sv.SVNICP(sv.SteinICPParam(iterations=I, KNN_count=W["K"], max_dist=W["max_dist"], lr=W["lr"], SVN_full_grad=W["svn_full_grad"]),
                     pb.init_pose)
     icp.add_cloud(src, pb.target, pb.init_pose)
     icp.set_initial_mean(pb.R0, pb.t0)
     assert icp.stein_align() == sv.ALIGN_SUCCESS
-    theirs = np.load(out_npy)
-    np.testing.assert_allclose(icp.get_particles().reshape(6, P), theirs, atol=5 * POSE_TOL, rtol=0)
-    np.testing.assert_allclose(icp.get_transformation(), np.array(info["mean"]), atol=POSE_TOL, rtol=0)
+    np.testing.assert_allclose(icp.get_particles().reshape(6, P), g["oracle_particles"], atol=5 * POSE_TOL, rtol=0)
+    np.testing.assert_allclose(icp.get_transformation(), g["oracle_mean"], atol=POSE_TOL, rtol=0)
