@@ -309,7 +309,7 @@ static int alloc_particle_state(svnicp_handle h) {
   h->pt.n_ranks = 1; h->pt.rank = 0;
   h->pt.rec[0] = h->rec; h->pt.flag[0] = h->flags_dev;
   h->pt.timeout_ns = 4000000000ull;
-  CU(h->xs.ensure(39 * P));  // SoA copy of x (SVGD-ICP class: of the gathered record, RT_ROWS x P)
+  CU(h->xs.ensure(6 * P));  // SoA copy of x at the head of the iteration (k_head_*)
   CU(h->delta.ensure(6 * P, true));
   CU(h->Hbar_inv.ensure(36));
   CU(h->stats.ensure(48));
@@ -811,6 +811,7 @@ static int align_begin(svnicp_handle h, AlignState &S) {
   sa.Hbar_inv = h->Hbar_inv.p; sa.hist = h->hist.p; sa.history = h->history.p; sa.ctrl = h->ctrl.p;
   sa.stats = h->stats.p; sa.particles = h->particles.p; sa.sm_count = h->sm_count;
   sa.kept_hist = h->kept_hist.p;
+  if (svgd) sa.rec_stride = 0;  // one record buffer: k_head_* read buffer 0 whatever the iteration's parity
   sa.prep_scratch_d = h->prep_scratch_d.p;
   sa.prep_scratch_i = h->prep_scratch_i.p;
   sa.stamps = h->profile ? h->stamps.p : nullptr;
@@ -964,8 +965,9 @@ static int align_step(svnicp_handle h, AlignState &S) {
       int rc = do_allgather(h);
       if (rc) return rc;
       PROF(5);
-      h->launches += launch_decide(sa, st, 0);
-      h->launches += launch_median(sa, st);
+      const int n = launch_head(sa, pt, 0u, 0, st);
+      if (n < 0) return fail(h, SVNICP_ERR_CUDA, "launch of k_head failed: %s", cudaGetErrorString(cudaGetLastError()));
+      h->launches += n;
       h->launches += launch_stein_first(sa, st);
       h->launches += launch_update_opt(sa, sv, e + 1, st);
     } else {
@@ -1015,8 +1017,9 @@ static int align_epilogue(svnicp_handle h, AlignState &S) {
     h->launches += launch_svgd_rec(h->rec, h->pose6.p, h->dnorm.p, h->p_lo, h->P_l, h->p_lo, st);
     int rc = do_allgather(h);
     if (rc) return rc;
-    h->launches += launch_decide(sa, st, 1);
-    h->launches += launch_stats_svgd(sa, h->prev.p, st);
+    const int n = launch_head(sa, pt, 0u, 1, st);
+    if (n < 0) return fail(h, SVNICP_ERR_CUDA, "launch of k_head failed: %s", cudaGetErrorString(cudaGetLastError()));
+    h->launches += n + launch_stats_svgd(sa, h->prev.p, st);
   } else {
     // the final x of every particle already sits in the record buffer of parity (updates applied & 1) on every rank
     if (!overlap && h->n_ranks > 1)

@@ -105,76 +105,11 @@ __device__ __forceinline__ float warp_min(float v) {
 }
 
 // ---- 6x6 dense helpers in fp64 (Stein step, finalize) ------------------------------------------
-// LU with partial pivoting; solves A X = B (nrhs columns), row-major, in place on B.
-__device__ inline void lu_solve6(double *A, double *B, int nrhs) {
-  for (int k = 0; k < 6; k++) {
-    int p = k;
-    double mx = fabs(A[k * 6 + k]);
-    for (int i = k + 1; i < 6; i++) {
-      double v = fabs(A[i * 6 + k]);
-      if (v > mx) { mx = v; p = i; }
-    }
-    if (p != k) {
-      for (int j = 0; j < 6; j++) { double t = A[k * 6 + j]; A[k * 6 + j] = A[p * 6 + j]; A[p * 6 + j] = t; }
-      for (int j = 0; j < nrhs; j++) { double t = B[k * nrhs + j]; B[k * nrhs + j] = B[p * nrhs + j]; B[p * nrhs + j] = t; }
-    }
-    const double d = A[k * 6 + k];
-    for (int i = k + 1; i < 6; i++) {
-      const double l = A[i * 6 + k] / d;
-      for (int j = k + 1; j < 6; j++) A[i * 6 + j] -= l * A[k * 6 + j];
-      for (int j = 0; j < nrhs; j++) B[i * nrhs + j] -= l * B[k * nrhs + j];
-    }
-  }
-  for (int k = 5; k >= 0; k--)
-    for (int j = 0; j < nrhs; j++) {
-      double s = B[k * nrhs + j];
-      for (int i = k + 1; i < 6; i++) s -= A[k * 6 + i] * B[i * nrhs + j];
-      B[k * nrhs + j] = s / A[k * 6 + k];
-    }
-}
-
-// The same solve (one right-hand side) with every index a compile-time constant: A and b stay in registers (nvcc leaves
-// `#pragma unroll` loops of this depth rolled and puts A on the stack, hence the template recursion).  The pivot of column k
-// is brought up by compare-and-swap of whole rows (i = k+1 .. 5 against row k): the same pivot VALUES as a classic arg-max
-// search, and each remaining row sees identical arithmetic, so the solution has the same bits (exact ties aside).
+// Compile-time loop: every index below is a constant, so the 6x6 operands stay in registers (nvcc leaves `#pragma unroll`
+// loops of this depth rolled and puts the matrix on the stack, hence the template recursion).
 template <int I, int N, class F>
 __device__ __forceinline__ void static_for(F &&f) {
   if constexpr (I < N) { f(std::integral_constant<int, I>{}); static_for<I + 1, N>(f); }
-}
-__device__ __forceinline__ void lu_solve6_reg(double (&A)[36], double (&b)[6]) {
-  static_for<0, 6>([&](auto K) {
-    constexpr int k = decltype(K)::value;
-    static_for<k + 1, 6>([&](auto I_) {
-      constexpr int i = decltype(I_)::value;
-      const bool sw = fabs(A[i * 6 + k]) > fabs(A[k * 6 + k]);
-      static_for<k, 6>([&](auto J) {
-        constexpr int j = decltype(J)::value;
-        const double u = A[k * 6 + j], v = A[i * 6 + j];
-        A[k * 6 + j] = sw ? v : u;
-        A[i * 6 + j] = sw ? u : v;
-      });
-      const double u = b[k], v = b[i];
-      b[k] = sw ? v : u;
-      b[i] = sw ? u : v;
-    });
-    // ONE division per pivot; the multipliers and the back substitution multiply by the reciprocal (fp64 division is a ~30
-    // instruction dependent sequence: 21 of them made this solve 13 us of the 17 us per-particle chain of k_tail).  x * (1/d)
-    // differs from x / d by at most one rounding: 1e-16 relative on the step, far inside every parity bar.
-    const double inv = 1.0 / A[k * 6 + k];
-    A[k * 6 + k] = inv;  // the diagonal now holds the reciprocal pivot
-    static_for<k + 1, 6>([&](auto I_) {
-      constexpr int i = decltype(I_)::value;
-      const double l = A[i * 6 + k] * inv;
-      static_for<k + 1, 6>([&](auto J) { constexpr int j = decltype(J)::value; A[i * 6 + j] -= l * A[k * 6 + j]; });
-      b[i] -= l * b[k];
-    });
-  });
-  static_for<0, 6>([&](auto KK) {
-    constexpr int k = 5 - decltype(KK)::value;
-    double s = b[k];
-    static_for<k + 1, 6>([&](auto I_) { constexpr int i = decltype(I_)::value; s -= A[k * 6 + i] * b[i]; });
-    b[k] = s * A[k * 6 + k];
-  });
 }
 
 // Symmetric positive definite 6x6 solve A x = b by LDL^T, every index a compile-time constant (registers only), one reciprocal

@@ -123,8 +123,8 @@ struct SteinArgs {
   int svn_full_grad, check_early_stop;
   double lr, threshold;
   double *rec;       // [2][rec_stride] (see IterArgs)
-  size_t rec_stride;
-  double *xs;        // [6][P] SoA copy of x (SVGD-ICP class: [39][P] copy of the gathered record)
+  size_t rec_stride; // SVN-ICP class: doubles per record buffer; SVGD-ICP class: 0, one buffer
+  double *xs;        // [6][P] SoA copy of x at the head of the iteration (median sweeps, get_gn_system of the SVGD-ICP class)
   double *delta;     // [P_l][6]
   double *dnorm;     // [P_l]
   double *R, *t;
@@ -140,14 +140,11 @@ struct SteinArgs {
   double *stamps;                 // [8] globaltimer stamps of k_tail's phases (tuning aid; null = off)
   int sm_count;
 };
-// SVN-ICP class, Stein phase (tail2.cu): k_head_* = early-stop decision + history row + exact median bandwidth (a chain of
-// small ordinary kernels, off the critical path); k_tail = Stein step + pose update + next iteration's transforms and pruning ball.
+// Stein phase (tail2.cu): k_head_* = early-stop decision + history row + exact median bandwidth (a chain of small ordinary
+// kernels; both classes), k_tail = Stein step + pose update + next iteration's transforms and pruning ball (SVN-ICP class).
 // seq_x / seq_h / seq_x_out: sequence numbers of the peer exchange (0 = nothing to wait for).  Return launches or -1.
 int launch_head(const SteinArgs &a, const PeerTable &pt, unsigned seq_x, int epilogue, cudaStream_t st);
 int launch_tail(const SteinArgs &a, const IterArgs &ia, const PeerTable &pt, unsigned seq_h, unsigned seq_x_out, cudaStream_t st);
-// SVGD-ICP class: separate kernels on the gathered record (stein_kernels.cu, svgd_class.cu)
-int launch_decide(const SteinArgs &a, cudaStream_t st, int epilogue);
-int launch_median(const SteinArgs &a, cudaStream_t st);
 // getters from the record buffer; parity_from_ctrl: read the buffer of parity (iters_done & 1) (SVN-ICP class)
 int launch_stats(const SteinArgs &a, int parity_from_ctrl, cudaStream_t st);
 // restart of the device-side iteration state at the head of every stein_align (poses are kept)

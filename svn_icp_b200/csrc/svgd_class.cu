@@ -3,9 +3,9 @@
 //   to_rotation_tensor   :226-260  ZYX Euler -> R                                  (k_svgd_init, k_update_opt)
 //   transform + get_correspondence_fast + point_filter :94-101, :300-333           (k_prep/k_filter/k_gn, shared)
 //   partial_derivative + sgd_grad :335-455                                         (k_gn<FIRST> + k_finalize_first)
-//   rbf_kernel + svgd_grad :457-474                                                (k_decide/k_median_pass shared, k_stein_first)
+//   rbf_kernel + svgd_grad :457-474                                                (k_head_* shared, k_stein_first)
 //   pose_update :476-494 = torch::optim::{Adam,RMSprop,SGD,Adagrad}::step          (k_update_opt)
-//   early stop :123-131, history :133, getters :497-534                            (k_decide shared, k_stats_svgd)
+//   early stop :123-131, history :133, getters :497-534                            (k_head_* shared, k_stats_svgd)
 //
 // Why the SVN-ICP correspondence kernel serves unchanged: each Euler partial is dR/dtheta_k = [omega_k]x R with
 //   omega_roll = R(:,0) of Rz Ry = (cp cy, cp sy, -sp),  omega_pitch = (-sy, cy, 0),  omega_yaw = (0, 0, 1),
@@ -92,6 +92,7 @@ __global__ void k_svgd_rec(double *rec, const double *src6, const double *dnorm,
 
 // SVGDICP::svgd_grad (:457-462): stein_i = ( sum_j K_ij (-g_j) + (2/h) sum_j (x_i - x_j) K_ij ) / P ; P == 1: -g (:112)
 constexpr int SF_WARPS = 8, SF_TJ = 32;
+static_assert(REC_X == 0 && REC_B == 6, "k_stein_first stages x and b as record doubles 0..11");
 __global__ void __launch_bounds__(SF_WARPS * 32) k_stein_first(SteinArgs a) {
   Ctrl *c = a.ctrl;
   if (c->stop) return;
@@ -115,8 +116,8 @@ __global__ void __launch_bounds__(SF_WARPS * 32) k_stein_first(SteinArgs a) {
   for (int j0 = 0; j0 < a.P; j0 += SF_TJ) {
     __syncthreads();
     for (int e = tid; e < 12 * SF_TJ; e += blockDim.x) {
-      const int q = e / SF_TJ, jj = e % SF_TJ;  // SoA rows 0..5 = x, 6..11 = b (the gradient)
-      s_rec[q][jj] = (j0 + jj < a.P) ? a.xs[(size_t)q * a.P + j0 + jj] : 0.0;
+      const int q = e / SF_TJ, jj = e % SF_TJ;  // s_rec rows 0..5 = x, 6..11 = b (the gradient)
+      s_rec[q][jj] = (j0 + jj < a.P) ? a.rec[(size_t)(j0 + jj) * REC + q] : 0.0;
     }
     __syncthreads();
     if (active && j0 + lane < a.P) {
@@ -187,7 +188,10 @@ __global__ void k_update_opt(SteinArgs a, SvgdArgs s, int step) {  // step = epo
     for (int i = 0; i < 3; i++) a.t[3 * (size_t)p + i] = x[i];
     a.dnorm[l] = sqrt(n2);                                               // :124 norm(2, 0)
   }
-  if (l == 0) c->iter = step;
+  if (l == 0) {
+    if (a.kept_hist) a.kept_hist[step - 1] = c->kept_total;  // candidates kept by this iteration's pruning pass
+    c->iter = step;
+  }
 }
 
 // getters (:497-524): plain mean, UNBIASED variance (torch::var), covariance / P; also refreshes pose_particles_ (`prev`)

@@ -77,15 +77,19 @@ def test_one_iteration_vs_oracle(oracle, lidar, optimizer, lr):
     np.testing.assert_allclose(icp.get_transformation(), ref["mean"], atol=POSE_TOL, rtol=0)
 
 
-@pytest.mark.parametrize("optimizer,lr", [("Adam", 0.03), ("RMSprop", 0.01)])
-def test_full_scan_vs_oracle(oracle, lidar, optimizer, lr):
+# P = 300 (> 64) runs the multi-CTA head chain: k_head_prep and, from iteration 1 on, the fast median path
+@pytest.mark.parametrize("optimizer,lr,P", [("Adam", 0.03, 64), ("RMSprop", 0.01, 64), ("Adam", 0.03, 300)],
+                         ids=["Adam-0.03", "RMSprop-0.01", "Adam-0.03-300"])
+def test_full_scan_vs_oracle(oracle, lidar, optimizer, lr, P):
     pb = lidar
-    P = pb.init_pose.shape[1]
+    init = pb.init_pose if P == pb.init_pose.shape[1] else synth.init_particles(P, np.random.default_rng(P))
     I = 12
-    icp = make_icp(pb, iterations=I, KNN_count=33, max_dist=3.0, lr=lr, optimizer=optimizer)
+    icp = sv.SVGDICP(sv.SteinICPParam(iterations=I, KNN_count=33, max_dist=3.0, lr=lr, optimizer=optimizer), init)
+    icp.add_cloud(pb.source, pb.target, init)
+    icp.set_initial_mean(pb.R0, pb.t0)
     assert icp.stein_align() == sv.ALIGN_SUCCESS
     prm = orc.make_svgd_params(iterations=I, lr=lr, max_dist=3.0, knn_count=33, optimizer=optimizer)
-    ref = oracle.svgd_align(prm, pb.source, pb.target, pb.init_pose, pb.init_pose, pb.R0, pb.t0)
+    ref = oracle.svgd_align(prm, pb.source, pb.target, init, init, pb.R0, pb.t0)
     got = icp.get_particles().reshape(6, P)
     # Adam / RMSprop divide the gradient by its running RMS: a near-threshold mask flip (test_first_order_gradient (3))
     # that changes a small gradient component by a few percent moves that parameter by a few percent of lr per step,
