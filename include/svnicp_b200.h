@@ -181,6 +181,24 @@ int svnicp_get_tail_stamps(svnicp_handle h, double out8[8]);
 /* number of kernel launches issued by the last svnicp_align */
 int svnicp_get_launch_count(svnicp_handle h, int64_t *out);
 
+/* Registration objective of the LAST scan at M caller-given poses (no reference counterpart): a fitness score to gate the map
+ * update on, to compare hypotheses (e.g. an IMU prediction against the registered pose), and the information matrix H at a pose.
+ * poses: [6][M] host doubles in the handle's particle convention (SVN-ICP: [t ; Log R]; SVGD-ICP: x,y,z,roll,pitch,yaw ZYX
+ *   Euler), relative to the scan's initial mean exactly like the particles: T_world = T0 * T(x).  get_transformation() and
+ *   all-zeros (= T0) are valid inputs.
+ * For every pose, against the candidate table of the last stein_align (1-NN among the K candidates of each source point,
+ *   the same fp32 arithmetic and tie-break as the registration; mask d^2 < max_dist, Q1; the current set_threshold value):
+ *   out_stats [M][3]  {inlier count, inlier fraction = count / N_s, inlier RMSE in metres (0 when there are no inliers)}
+ *   out_H [M][36], out_b [M][6]  (may be NULL)  Newton_grad_right at that pose (SVNICP.cpp:116-164, with Q1-Q3), in the
+ *     layout of svnicp_get_gn_system -- for both classes (right perturbation in [t ; omega])
+ *   out_mask [M][N_s] (may be NULL)  1 where the source point is an inlier
+ *   out_idx [M][N_s]  (may be NULL; needs debug_corr)  global map index of the chosen candidate
+ * Blocking, on the handle's stream; changes no state of the handle (particles, getters, history, timing, launch count).
+ * Sharded handles hold the whole table: rank-local, no communication, the same result on every rank.
+ * SVNICP_ERR_INVALID before the first stein_align, or after add_cloud / set_initial_mean / set_k until the next one. */
+int svnicp_evaluate(svnicp_handle h, int n_poses, const double *poses_6xM, double *out_stats, double *out_H, double *out_b,
+                    uint8_t *out_mask, int32_t *out_idx);
+
 /* ---------------------------------------------------------------------------------------------
  * Throughput mode: S independent odometry streams on one GPU (BASELINE.json configs[3]; no reference counterpart -- the
  * reference runs one SVNICP instance per node process).  A batch owns one SVN-ICP handle per stream; use

@@ -89,7 +89,7 @@ EXPORTS = [
     "svnicp_initialize_particles", "svnicp_initialize_particles_gaussian", "svnicp_iterations_done", "svnicp_get_candidates",
     "svnicp_get_source_f32", "svnicp_get_correspondences", "svnicp_get_gn_system", "svnicp_get_stein", "svnicp_get_prune_stats",
     "svnicp_get_timing", "svnicp_get_slice", "svnicp_get_launch_count", "svnicp_set_profiling", "svnicp_get_phase_times",
-    "svnicp_get_scan_info", "svnicp_get_tail_stamps",
+    "svnicp_get_scan_info", "svnicp_get_tail_stamps", "svnicp_evaluate",
     "svnicp_map_create", "svnicp_map_destroy", "svnicp_map_last_error", "svnicp_map_clear", "svnicp_map_add_cloud", "svnicp_map_get",
     "svnicp_map_download", "svnicp_map_size",
     "svnicp_pre_create", "svnicp_pre_destroy", "svnicp_pre_last_error", "svnicp_pre_crop", "svnicp_pre_downsample_uniform",
@@ -149,6 +149,7 @@ def _ARGTYPES(V, I, L, D):
         "svnicp_get_gn_system": [V, V, V, V], "svnicp_get_stein": [V, V, V], "svnicp_get_prune_stats": [V, V, V],
         "svnicp_get_timing": [V, V], "svnicp_get_slice": [V, V, V], "svnicp_get_launch_count": [V, V],
         "svnicp_get_tail_stamps": [V, V], "svnicp_set_profiling": [V, I], "svnicp_get_phase_times": [V, V], "svnicp_get_scan_info": [V, V],
+        "svnicp_evaluate": [V, I, V, V, V, V, V, V],
         "svnicp_map_create": [V, D, D, I, L, I], "svnicp_map_clear": [V], "svnicp_map_add_cloud": [V, V, L, I, I, V, V],
         "svnicp_map_get": [V, V, D, V, V], "svnicp_map_download": [V, V, L], "svnicp_map_size": [V, V, V],
         "svnicp_pre_create": [V, L, I], "svnicp_pre_crop": [V, V, L, I, D, D, V, V, V],
@@ -344,6 +345,29 @@ class SVNICP:
 
     def set_threshold(self, max_dist: float):
         self._check(self._lib.svnicp_set_threshold(self._h, C.c_double(max_dist)), "set_threshold")
+
+    def evaluate(self, poses, want_system: bool = True, want_mask: bool = False, want_idx: bool = False) -> dict:
+        """Registration objective of the last scan at caller-given poses (svnicp_evaluate; no reference counterpart).
+        poses: (6,) or (6, M) in the particle convention of the class, relative to the scan's initial mean (get_transformation()
+        and zeros are valid).  Returns numpy arrays: inliers [M] int64, fitness [M] (inlier fraction), rmse [M] (metres);
+        with want_system H [M, 6, 6], b [M, 6] (the Gauss-Newton system of svnicp_get_gn_system's layout); with want_mask
+        mask [M, N_s] uint8; with want_idx (handle created with debug_corr) idx [M, N_s] int32 global map indices.
+        A (6,) input drops the leading M axis.  Changes no state of the handle."""
+        x = np.asarray(poses, dtype=np.float64)
+        single = x.ndim == 1
+        x = np.ascontiguousarray(x.reshape(6, -1))
+        M = x.shape[1]
+        stats = np.zeros((M, 3))
+        H = np.zeros((M, 6, 6)) if want_system else None
+        b = np.zeros((M, 6)) if want_system else None
+        mask = np.zeros((M, self.n_s), dtype=np.uint8) if want_mask else None
+        idx = np.zeros((M, self.n_s), dtype=np.int32) if want_idx else None
+        self._check(self._lib.svnicp_evaluate(self._h, C.c_int(M), _p(x), _p(stats), _p(H), _p(b), _p(mask), _p(idx)), "evaluate")
+        out = dict(inliers=stats[:, 0].astype(np.int64), fitness=stats[:, 1].copy(), rmse=stats[:, 2].copy())
+        for k, v in (("H", H), ("b", b), ("mask", mask), ("idx", idx)):
+            if v is not None:
+                out[k] = v
+        return {k: v[0] for k, v in out.items()} if single else out
 
     # -- parity / debug taps ----------------------------------------------------------------------
     def iterations_done(self) -> int:

@@ -157,6 +157,13 @@ struct svnicp_handle_t {
   // launch shape
   int TB = 16, stages = 3, n_slices = 1, n_pgroups = 1, PG = 512, RG = 1;
   size_t gn_smem = 0;
+  // svnicp_evaluate: the candidate table (cand, sp, R0, K) of the last stein_align is still the scan's current one -- set by a
+  // completed stein_align, cleared by add_cloud / set_initial_mean / set_k / init_sharding; and the evaluation's own scratch
+  bool eval_ok = false;
+  DevBuf<double> ev_pose, ev_R, ev_part, ev_out;
+  DevBuf<float> ev_xf;
+  DevBuf<uint8_t> ev_mask;
+  DevBuf<int32_t> ev_idx;
 };
 
 static int fail(svnicp_handle h, int code, const char *fmt, ...) {
@@ -390,6 +397,7 @@ int svnicp_create(svnicp_handle *out, const svnicp_params *params, int particle_
     CU(cudaEventCreateWithFlags(&h->ev_chead, cudaEventDisableTiming));
     for (int i = 0; i < 4; i++) CU(cudaEventCreate(&h->ev[i]));
     init_iter_kernels();
+    init_eval_kernels();
     CU(cudaGetLastError());
     int r = alloc_particle_state(h);
     if (r) return r;
@@ -445,6 +453,7 @@ void svnicp_destroy(svnicp_handle h) {
   h->counts.release(); h->starts.release(); h->fill.release(); h->pt_slot.release(); h->sidx.release(); h->misc.release();
   h->keys.release(); h->kept_hist.release(); h->xf.release(); h->dbg_xf.release(); h->history.release(); h->hist.release(); h->ctrl.release();
   h->dbg_idx.release(); h->dbg_mask.release();
+  h->ev_pose.release(); h->ev_R.release(); h->ev_part.release(); h->ev_out.release(); h->ev_xf.release(); h->ev_mask.release(); h->ev_idx.release();
   if (h->h_stats) cudaFreeHost(h->h_stats);
   if (h->h_particles) cudaFreeHost(h->h_particles);
   if (h->h_history) cudaFreeHost(h->h_history);
@@ -498,6 +507,7 @@ int svnicp_init_sharding(svnicp_handle h, const void *unique_id128, int rank, in
   int r = alloc_particle_state(h);
   if (r) return r;
   h->have_cloud = false;
+  h->eval_ok = false;
   h->peer_mode = false;
   if (n_ranks > 1 && n_ranks <= MAX_RANKS && h->class_type == SVNICP_CLASS_SVNICP && !(h->prm.flags & SVNICP_FLAG_NCCL_GATHER)) {
     // Peer-memory exchange: map every rank's record block here through CUDA IPC (handles travel over the NCCL communicator
@@ -645,11 +655,13 @@ int svnicp_add_cloud(svnicp_handle h, const double *source, int64_t n_s, int sou
   if (rc) return rc;
   h->have_cloud = true;
   h->aligned = false;
+  h->eval_ok = false;
   return upload_particles(h, init_pose);  // SVGDICP.cpp:47-61 (also synchronises the cloud copies)
 }
 
 int svnicp_set_initial_mean(svnicp_handle h, const double R0[9], const double t0[3]) {
   if (!h || !R0 || !t0) return SVNICP_ERR_INVALID;
+  h->eval_ok = false;  // the candidate table is relative to the previous initial mean
   memcpy(h->sc.R0, R0, 9 * sizeof(double));
   memcpy(h->sc.t0, t0, 3 * sizeof(double));
   return SVNICP_OK;
@@ -658,7 +670,8 @@ int svnicp_set_initial_mean(svnicp_handle h, const double R0[9], const double t0
 int svnicp_set_k(svnicp_handle h, int k) {
   if (!h) return SVNICP_ERR_INVALID;
   if (k < 1 || k > 256) return fail(h, SVNICP_ERR_INVALID, "set_k: K must be in [1,256]");
-  if (k != h->K) h->shape_dirty = true;  // SVGDICP.h:98: K_source_ takes effect at the next stein_align; the stored clouds stay
+  if (k != h->K) h->shape_dirty = true;
+  h->eval_ok = false;  // SVGDICP.h:98: K_source_ takes effect at the next stein_align; the stored clouds stay
   h->K = k;
   return SVNICP_OK;
 }
@@ -698,6 +711,7 @@ struct AlignState {
 
 static int align_begin(svnicp_handle h, AlignState &S) {
   if (!h->have_cloud) return fail(h, SVNICP_ERR_INVALID, "stein_align before add_cloud");
+  h->eval_ok = false;  // the candidate table is rebuilt (or, NO_OPTIMIZER, not built): valid again once the scan completes
   CU(cudaSetDevice(h->device));
   cudaStream_t st = h->stream;
   const int I = S.I = h->prm.iterations;
@@ -1085,6 +1099,7 @@ static int align_finish(svnicp_handle h, AlignState &S) {
   CU(cudaMemcpy(misc, h->misc.p, sizeof(misc), cudaMemcpyDeviceToHost));
   h->fallback_queries = misc[1];
   h->aligned = true;
+  h->eval_ok = true;
   return SVNICP_ALIGN_SUCCESS;
 }
 
@@ -1350,6 +1365,62 @@ int svnicp_get_tail_stamps(svnicp_handle h, double out8[8]) {
 int svnicp_get_launch_count(svnicp_handle h, int64_t *out) {
   if (!h || !out) return SVNICP_ERR_INVALID;
   *out = h->launches;
+  return SVNICP_OK;
+}
+
+// ---- svnicp_evaluate: registration objective of the last scan at caller-given poses (eval_kernels.cu) ----
+// Reads the candidate table, the fp32 source and R0 of the last stein_align; writes only its own scratch (ev_*).  No launch
+// is counted in launch_count() and no event of the scan's timing is recorded.
+int svnicp_evaluate(svnicp_handle h, int n_poses, const double *poses_6xM, double *out_stats, double *out_H, double *out_b,
+                    uint8_t *out_mask, int32_t *out_idx) {
+  if (!h) return SVNICP_ERR_INVALID;
+  if (n_poses < 1) return fail(h, SVNICP_ERR_INVALID, "evaluate: n_poses must be >= 1 (got %d)", n_poses);
+  if (!poses_6xM || !out_stats) return fail(h, SVNICP_ERR_INVALID, "evaluate: null poses or out_stats");
+  if (!h->eval_ok)
+    return fail(h, SVNICP_ERR_INVALID, "evaluate: no candidate table of the current scan (stein_align must complete after add_cloud / "
+                                       "set_initial_mean / set_k)");
+  if (out_idx && !h->prm.debug_corr)
+    return fail(h, SVNICP_ERR_INVALID, "evaluate: out_idx needs a handle created with debug_corr (the map-index table is only kept for it)");
+  CU(cudaSetDevice(h->device));
+  cudaStream_t st = h->stream;
+  const int M = n_poses, n_s = (int)h->n_s;
+  const int n_blk = M < EV_BLOCK ? M : EV_BLOCK;
+  CU(h->ev_pose.ensure((size_t)6 * M));
+  CU(h->ev_xf.ensure((size_t)12 * M));
+  CU(h->ev_R.ensure((size_t)9 * M));
+  CU(h->ev_out.ensure((size_t)EV_OUT * M));
+  CU(h->ev_part.ensure((size_t)eval_parts(n_s, h->K, h->sm_count) * n_blk * EV_NS));
+  if (out_mask) CU(h->ev_mask.ensure((size_t)n_blk * n_s));
+  if (out_idx) CU(h->ev_idx.ensure((size_t)n_blk * n_s));
+  CU(cudaMemcpyAsync(h->ev_pose.p, poses_6xM, (size_t)6 * M * sizeof(double), cudaMemcpyHostToDevice, st));
+  launch_eval_prep(h->ev_pose.p, M, h->class_type == SVNICP_CLASS_SVGDICP ? 1 : 0, h->sc, h->ev_xf.p, h->ev_R.p, st);
+  EvalArgs a;
+  memset(&a, 0, sizeof(a));
+  a.n_s = n_s; a.K = h->K; a.max_dist = (float)h->max_dist;
+  a.sp = h->sp.p; a.cand = h->cand.p; a.cand_idx = out_idx ? h->cand_idx.p : nullptr;
+  a.part = h->ev_part.p;
+  a.mask = out_mask ? h->ev_mask.p : nullptr;
+  a.idx = out_idx ? h->ev_idx.p : nullptr;
+  for (int m0 = 0; m0 < M; m0 += EV_BLOCK) {
+    a.MB = M - m0 < EV_BLOCK ? M - m0 : EV_BLOCK;
+    a.G = 1;
+    while (a.G < a.MB) a.G <<= 1;
+    a.xf = h->ev_xf.p + (size_t)12 * m0;
+    launch_eval_block(a, out_H || out_b, h->sc, h->ev_R.p + (size_t)9 * m0, h->ev_out.p + (size_t)EV_OUT * m0, h->sm_count, st);
+    CU(cudaGetLastError());
+    // [M][n_s] outputs: the rows of this block are contiguous in the caller's array
+    if (out_mask) CU(cudaMemcpyAsync(out_mask + (size_t)m0 * n_s, h->ev_mask.p, (size_t)a.MB * n_s, cudaMemcpyDeviceToHost, st));
+    if (out_idx) CU(cudaMemcpyAsync(out_idx + (size_t)m0 * n_s, h->ev_idx.p, (size_t)a.MB * n_s * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  }
+  std::vector<double> res((size_t)EV_OUT * M);
+  CU(cudaMemcpyAsync(res.data(), h->ev_out.p, res.size() * sizeof(double), cudaMemcpyDeviceToHost, st));
+  CU(cudaStreamSynchronize(st));
+  for (int m = 0; m < M; m++) {
+    const double *r = res.data() + (size_t)EV_OUT * m;
+    memcpy(out_stats + (size_t)3 * m, r, 3 * sizeof(double));
+    if (out_H) memcpy(out_H + (size_t)36 * m, r + 3, 36 * sizeof(double));
+    if (out_b) memcpy(out_b + (size_t)6 * m, r + 39, 6 * sizeof(double));
+  }
   return SVNICP_OK;
 }
 

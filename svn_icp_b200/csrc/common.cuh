@@ -190,6 +190,87 @@ __device__ inline void so3_log(const double R[9], double w[3]) {
   }
 }
 
+// ZYX Euler angles x6[3..5] = (roll, pitch, yaw) -> R, exactly as SVGDICP::to_rotation_tensor (SVGDICP.cpp:226-260)
+__device__ __forceinline__ void euler_R(const double *x6, double *R) {
+  double sr, cr, sp, cp, sy, cy;
+  sincos(x6[3], &sr, &cr);
+  sincos(x6[4], &sp, &cp);
+  sincos(x6[5], &sy, &cy);
+  R[0] = cp * cy; R[1] = sr * sp * cy - cr * sy; R[2] = sr * sy + cr * sp * cy;
+  R[3] = cp * sy; R[4] = cr * cy + sr * sp * sy; R[5] = cr * sp * sy - sr * cy;
+  R[6] = -sp;     R[7] = sr * cp;                R[8] = cr * cp;
+}
+
+// fp32 transform of one pose (R, t) in coordinates relative to the scan's initial-guess query q0:
+// xf[0..9) = A' = R0 (R - I) R0^T (row-major), xf[9..12) = tau = R0 t, so that q_pb - q0_b = A' (R0 s_b) + tau.
+// The one place this is computed: k_prep (iteration 0), k_tail (iterations >= 1) and k_eval_prep (svnicp_evaluate).
+__device__ __forceinline__ void rel_transform_f32(const double *R0, const double R[9], const double t[3], float xf[12]) {
+  double D[9], T[9], M[9];
+#pragma unroll
+  for (int i = 0; i < 9; i++) D[i] = R[i] - ((i % 4 == 0) ? 1.0 : 0.0);
+#pragma unroll
+  for (int r = 0; r < 3; r++)
+#pragma unroll
+    for (int c = 0; c < 3; c++) T[3 * r + c] = R0[3 * r] * D[c] + R0[3 * r + 1] * D[3 + c] + R0[3 * r + 2] * D[6 + c];
+#pragma unroll
+  for (int r = 0; r < 3; r++)
+#pragma unroll
+    for (int c = 0; c < 3; c++) M[3 * r + c] = T[3 * r] * R0[3 * c] + T[3 * r + 1] * R0[3 * c + 1] + T[3 * r + 2] * R0[3 * c + 2];
+#pragma unroll
+  for (int i = 0; i < 9; i++) xf[i] = __double2float_rn(M[i]);
+#pragma unroll
+  for (int r = 0; r < 3; r++) xf[9 + r] = __double2float_rn(R0[3 * r] * t[0] + R0[3 * r + 1] * t[1] + R0[3 * r + 2] * t[2]);
+}
+
+// The 16 Gauss-Newton sums of one pose (v: W, S1, S2, E, C in the world-oriented frame, see k_gn) -> the reference's system
+// H (full 6x6, row-major) and b of Newton_grad_right (SVNICP.cpp:116-164, quirks Q2 and Q3).  Rp: the pose's rotation.
+__device__ __forceinline__ void gn_assemble(const double *R0, const double Rp[9], const double v[NACC], double H[36], double b[6]) {
+  double Rt[9];
+#pragma unroll
+  for (int r = 0; r < 3; r++)
+#pragma unroll
+    for (int c = 0; c < 3; c++) Rt[3 * r + c] = R0[3 * r] * Rp[c] + R0[3 * r + 1] * Rp[3 + c] + R0[3 * r + 2] * Rp[6 + c];
+  const double W = v[0];
+  // world-oriented -> sensor frame: S1 = R0^T S1', S2 = R0^T S2' R0
+  const double S1p[3] = {v[1], v[2], v[3]};
+  const double S2p[9] = {v[4], v[5], v[6], v[5], v[7], v[8], v[6], v[8], v[9]};
+  double S1[3], T[9], S2[9];
+#pragma unroll
+  for (int c = 0; c < 3; c++) S1[c] = R0[c] * S1p[0] + R0[3 + c] * S1p[1] + R0[6 + c] * S1p[2];
+#pragma unroll
+  for (int r = 0; r < 3; r++)
+#pragma unroll
+    for (int c = 0; c < 3; c++) T[3 * r + c] = R0[r] * S2p[c] + R0[3 + r] * S2p[3 + c] + R0[6 + r] * S2p[6 + c];
+#pragma unroll
+  for (int r = 0; r < 3; r++)
+#pragma unroll
+    for (int c = 0; c < 3; c++) S2[3 * r + c] = T[3 * r] * R0[c] + T[3 * r + 1] * R0[3 + c] + T[3 * r + 2] * R0[6 + c];
+#pragma unroll
+  for (int i = 0; i < 36; i++) H[i] = 0.0;
+  const double trS2 = S2[0] + S2[4] + S2[8];
+#pragma unroll
+  for (int i = 0; i < 3; i++) {
+    H[7 * i] = W + 1e-6;  // SVNICP.cpp:153 (Q3); translation block = sum(rho') + #masked (Q2)
+#pragma unroll
+    for (int j = 0; j < 3; j++) H[6 * (3 + i) + 3 + j] = ((i == j) ? trS2 : 0.0) - S2[3 * i + j];
+    H[7 * (3 + i)] += 1e-6;
+  }
+  // H_tr = -[S1]x
+  H[0 * 6 + 4] = S1[2];  H[0 * 6 + 5] = -S1[1];
+  H[1 * 6 + 3] = -S1[2]; H[1 * 6 + 5] = S1[0];
+  H[2 * 6 + 3] = S1[1];  H[2 * 6 + 4] = -S1[0];
+#pragma unroll
+  for (int i = 0; i < 3; i++)
+#pragma unroll
+    for (int j = 0; j < 3; j++) H[6 * (3 + i) + j] = H[6 * j + 3 + i];
+  // b_t = R~^T E, b_r = R~^T C
+#pragma unroll
+  for (int c = 0; c < 3; c++) {
+    b[c] = Rt[c] * v[10] + Rt[3 + c] * v[11] + Rt[6 + c] * v[12];
+    b[3 + c] = Rt[c] * v[13] + Rt[3 + c] * v[14] + Rt[6 + c] * v[15];
+  }
+}
+
 // largest eigenvalue of M^T M (M 3x3 row-major) = sigma_max(M)^2, rounded up; NaN propagates
 __device__ inline double sym3_max_eig_MtM(const double M[9]) {
   double B[6];  // 00 01 02 11 12 22

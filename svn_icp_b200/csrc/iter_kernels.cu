@@ -57,27 +57,11 @@ __global__ void __launch_bounds__(1024) k_prep(IterArgs a, int all_x, const doub
 #pragma unroll
     for (int i = 0; i < 3; i++) { rec[REC_X + i] = t[i]; rec[REC_X + 3 + i] = w[i]; }
     rec[REC_DNORM] = a.dnorm[l];
-    // A' = R0 (R - I) R0^T, tau = R0 t   (so that q_pb - q0_b = A' (R0 s_b) + tau)
-    double D[9], T[9], M[9];
-#pragma unroll
-    for (int i = 0; i < 9; i++) D[i] = R[i] - ((i % 4 == 0) ? 1.0 : 0.0);
-#pragma unroll
-    for (int r = 0; r < 3; r++)
-#pragma unroll
-      for (int c = 0; c < 3; c++) T[3 * r + c] = R0[3 * r] * D[c] + R0[3 * r + 1] * D[3 + c] + R0[3 * r + 2] * D[6 + c];
-#pragma unroll
-    for (int r = 0; r < 3; r++)
-#pragma unroll
-      for (int c = 0; c < 3; c++) M[3 * r + c] = T[3 * r] * R0[3 * c] + T[3 * r + 1] * R0[3 * c + 1] + T[3 * r + 2] * R0[3 * c + 2];
+    float f[12];
+    rel_transform_f32(R0, R, t, f);  // A' = R0 (R - I) R0^T, tau = R0 t
     float *xf = a.xf + (size_t)l * 12;
 #pragma unroll
-    for (int i = 0; i < 9; i++) { const float f = __double2float_rn(M[i]); xf[i] = f; acc[i] += (double)f; }
-#pragma unroll
-    for (int r = 0; r < 3; r++) {
-      const float f = __double2float_rn(R0[3 * r] * t[0] + R0[3 * r + 1] * t[1] + R0[3 * r + 2] * t[2]);
-      xf[9 + r] = f;
-      acc[9 + r] += (double)f;
-    }
+    for (int i = 0; i < 12; i++) { xf[i] = f[i]; acc[i] += (double)f[i]; }
   }
   if (all_x)
     for (int p = tid; p < a.P; p += blockDim.x) {
@@ -775,55 +759,10 @@ __global__ void __launch_bounds__(FIN_WARPS * 32) k_finalize(IterArgs a, PeerTab
   SVN_CHECK(ctl, l < a.P_l && p < a.P && (size_t)(p + 1) * REC <= a.rec_stride, 20);
   const size_t buf_off = (size_t)(ctl->iter & 1) * a.rec_stride;
   if (threadIdx.x == 0) {
-    const double *R0 = a.sc.R0;
-    double Rp[9], Rt[9];
+    double Rp[9], H[36], b[6];
 #pragma unroll
     for (int i = 0; i < 9; i++) Rp[i] = a.R[9 * (size_t)p + i];
-#pragma unroll
-    for (int r = 0; r < 3; r++)
-#pragma unroll
-      for (int c = 0; c < 3; c++) Rt[3 * r + c] = R0[3 * r] * Rp[c] + R0[3 * r + 1] * Rp[3 + c] + R0[3 * r + 2] * Rp[6 + c];
-    const double W = v[0];
-    // world-oriented -> sensor frame: S1 = R0^T S1', S2 = R0^T S2' R0
-    const double S1p[3] = {v[1], v[2], v[3]};
-    const double S2p[9] = {v[4], v[5], v[6], v[5], v[7], v[8], v[6], v[8], v[9]};
-    double S1[3], T[9], S2[9];
-#pragma unroll
-    for (int c = 0; c < 3; c++) S1[c] = R0[c] * S1p[0] + R0[3 + c] * S1p[1] + R0[6 + c] * S1p[2];
-#pragma unroll
-    for (int r = 0; r < 3; r++)
-#pragma unroll
-      for (int c = 0; c < 3; c++) T[3 * r + c] = R0[r] * S2p[c] + R0[3 + r] * S2p[3 + c] + R0[6 + r] * S2p[6 + c];
-#pragma unroll
-    for (int r = 0; r < 3; r++)
-#pragma unroll
-      for (int c = 0; c < 3; c++) S2[3 * r + c] = T[3 * r] * R0[c] + T[3 * r + 1] * R0[3 + c] + T[3 * r + 2] * R0[6 + c];
-    double H[36];
-#pragma unroll
-    for (int i = 0; i < 36; i++) H[i] = 0.0;
-    const double trS2 = S2[0] + S2[4] + S2[8];
-#pragma unroll
-    for (int i = 0; i < 3; i++) {
-      H[7 * i] = W + 1e-6;  // SVNICP.cpp:153 (Q3); translation block = sum(rho') + #masked (Q2)
-#pragma unroll
-      for (int j = 0; j < 3; j++) H[6 * (3 + i) + 3 + j] = ((i == j) ? trS2 : 0.0) - S2[3 * i + j];
-      H[7 * (3 + i)] += 1e-6;
-    }
-    // H_tr = -[S1]x
-    H[0 * 6 + 4] = S1[2];  H[0 * 6 + 5] = -S1[1];
-    H[1 * 6 + 3] = -S1[2]; H[1 * 6 + 5] = S1[0];
-    H[2 * 6 + 3] = S1[1];  H[2 * 6 + 4] = -S1[0];
-#pragma unroll
-    for (int i = 0; i < 3; i++)
-#pragma unroll
-      for (int j = 0; j < 3; j++) H[6 * (3 + i) + j] = H[6 * j + 3 + i];
-    double b[6];
-    // b_t = R~^T E, b_r = R~^T C
-#pragma unroll
-    for (int c = 0; c < 3; c++) {
-      b[c] = Rt[c] * v[10] + Rt[3 + c] * v[11] + Rt[6 + c] * v[12];
-      b[3 + c] = Rt[c] * v[13] + Rt[3 + c] * v[14] + Rt[6 + c] * v[15];
-    }
+    gn_assemble(a.sc.R0, Rp, v, H, b);
 #pragma unroll
     for (int i = 0; i < 6; i++) s_out[REC_B + i] = b[i];
 #pragma unroll

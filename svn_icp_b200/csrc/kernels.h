@@ -153,6 +153,27 @@ int launch_init_particles(double *R, double *t, const double *init_pose_dev, int
                           cudaStream_t st);
 
 
+// ---- svnicp_evaluate (eval_kernels.cu): registration objective of the last scan's candidate table at given poses ----
+constexpr int EV_NS = NACC + 2;  // per-pose sums: the 16 Gauss-Newton sums, inlier count, sum of inlier d^2
+constexpr int EV_OUT = 45;       // per-pose result: {count, fraction, rmse}, H [36], b [6]
+constexpr int EV_BLOCK = 32;     // poses per pass over the table
+struct EvalArgs {
+  int n_s, K;
+  float max_dist;
+  const float4 *sp, *cand;
+  const int *cand_idx;  // [n_s][K] global map index per slot (only read when idx != null)
+  const float *xf;      // [MB][12] fp32 transforms of the block's poses
+  int MB, G;            // poses in the block (<= EV_BLOCK); lane groups = MB rounded up to a power of two
+  double *part;         // [eval_parts][MB][EV_NS] per-CTA partial sums
+  uint8_t *mask;        // [MB][n_s] or null
+  int32_t *idx;         // [MB][n_s] or null
+};
+int eval_parts(int n_s, int K, int sm_count);  // CTAs of the correspondence pass = partial slots per pose
+int launch_eval_prep(const double *poses, int M, int euler, const ScanConst &sc, float *xf, double *R, cudaStream_t st);
+int launch_eval_block(const EvalArgs &a, bool want_system, const ScanConst &sc, const double *R_blk, double *out_blk, int sm_count,
+                      cudaStream_t st);
+void init_eval_kernels();
+
 // ---- SVGD-ICP class (class_type = SVGDICP, svgd_class.cu): first-order gradient + torch::optim-style update ----
 enum { SVGD_OPT_ADAM = 0, SVGD_OPT_RMSPROP = 1, SVGD_OPT_SGD = 2, SVGD_OPT_ADAGRAD = 3 };
 struct SvgdArgs {

@@ -16,16 +16,6 @@
 
 namespace svn {
 
-__device__ __forceinline__ void euler_R(const double *x6, double *R) {  // SVGDICP.cpp:226-260
-  double sr, cr, sp, cp, sy, cy;
-  sincos(x6[3], &sr, &cr);
-  sincos(x6[4], &sp, &cp);
-  sincos(x6[5], &sy, &cy);
-  R[0] = cp * cy; R[1] = sr * sp * cy - cr * sy; R[2] = sr * sy + cr * sp * cy;
-  R[3] = cp * sy; R[4] = cr * cy + sr * sp * sy; R[5] = cr * sp * sy - sr * cy;
-  R[6] = -sp;     R[7] = sr * cp;                R[8] = cr * cp;
-}
-
 // SVGDICP::add_cloud (:46-61): parameters from init_pose [6][P]; optimizer moments cleared (set_optimizer, :73, :142-170)
 __global__ void k_svgd_init(SvgdArgs s, const double *init_pose, double *R, double *t, double *dnorm, Ctrl *ctrl) {
   const int p = blockIdx.x * blockDim.x + threadIdx.x;

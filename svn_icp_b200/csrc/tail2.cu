@@ -690,26 +690,11 @@ __global__ void __launch_bounds__(TL_THREADS, 1) k_tail(SteinArgs a, IterArgs ia
       }
       if (pt.n_ranks > 1) __threadfence_system();
       // fp32 transforms relative to q0 (as k_prep)
-      double D[9], T[9], M[9];
-#pragma unroll
-      for (int q = 0; q < 9; q++) D[q] = Rn[q] - ((q % 4 == 0) ? 1.0 : 0.0);
-#pragma unroll
-      for (int r = 0; r < 3; r++)
-#pragma unroll
-        for (int cc = 0; cc < 3; cc++) T[3 * r + cc] = R0[3 * r] * D[cc] + R0[3 * r + 1] * D[3 + cc] + R0[3 * r + 2] * D[6 + cc];
-#pragma unroll
-      for (int r = 0; r < 3; r++)
-#pragma unroll
-        for (int cc = 0; cc < 3; cc++) M[3 * r + cc] = T[3 * r] * R0[3 * cc] + T[3 * r + 1] * R0[3 * cc + 1] + T[3 * r + 2] * R0[3 * cc + 2];
+      float f[12];
+      rel_transform_f32(R0, Rn, t, f);
       float *xf = ia.xf + (size_t)l * 12;
 #pragma unroll
-      for (int q = 0; q < 9; q++) { const float f = __double2float_rn(M[q]); xf[q] = f; xfd[q] = (double)f; }
-#pragma unroll
-      for (int r = 0; r < 3; r++) {
-        const float f = __double2float_rn(R0[3 * r] * t[0] + R0[3 * r + 1] * t[1] + R0[3 * r + 2] * t[2]);
-        xf[9 + r] = f;
-        xfd[9 + r] = (double)f;
-      }
+      for (int q = 0; q < 12; q++) { xf[q] = f[q]; xfd[q] = (double)f[q]; }
     }
     if (ii < TL_WARPS)
 #pragma unroll

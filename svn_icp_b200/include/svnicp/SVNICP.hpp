@@ -141,6 +141,38 @@ class SVGDICP {  // the base interface the node holds (OdometryPipeline.h:125)
   void set_k(const int k) { check(svnicp_set_k(h_, k), "set_k"); }
   void set_threshold(const double max_dist) { check(svnicp_set_threshold(h_, max_dist), "set_threshold"); }
 
+  /** Registration objective of the last scan at M poses (svnicp_evaluate; no reference counterpart).  poses_6xM: [6][M] in the
+   *  class's particle convention, relative to the initial mean (get_transformation() and zeros are valid).  Per pose: inlier
+   *  count, fitness = inlier fraction, inlier RMSE (m); with want_system the Gauss-Newton system H [M][36], b [M][6]; with
+   *  want_mask the inlier mask [M][N_s].  Changes no state of the instance. */
+  struct Evaluation {
+    int n_poses = 0;
+    std::vector<int64_t> inliers;
+    std::vector<double> fitness, rmse;
+    std::vector<double> H, b;
+    std::vector<uint8_t> mask;
+  };
+  Evaluation evaluate(const std::vector<double> &poses_6xM, bool want_system = true, bool want_mask = false) const {
+    if (poses_6xM.empty() || poses_6xM.size() % 6 != 0) throw Error("evaluate: poses must hold 6*M doubles");
+    Evaluation r;
+    r.n_poses = (int)(poses_6xM.size() / 6);
+    const size_t M = (size_t)r.n_poses;
+    int64_t info[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+    check(svnicp_get_scan_info(h_, info), "evaluate");
+    std::vector<double> stats(3 * M);
+    if (want_system) { r.H.resize(36 * M); r.b.resize(6 * M); }
+    if (want_mask) r.mask.resize(M * (size_t)info[0]);
+    check(svnicp_evaluate(h_, r.n_poses, poses_6xM.data(), stats.data(), want_system ? r.H.data() : nullptr,
+                          want_system ? r.b.data() : nullptr, want_mask ? r.mask.data() : nullptr, nullptr),
+          "evaluate");
+    for (size_t m = 0; m < M; m++) {
+      r.inliers.push_back((int64_t)stats[3 * m]);
+      r.fitness.push_back(stats[3 * m + 1]);
+      r.rmse.push_back(stats[3 * m + 2]);
+    }
+    return r;
+  }
+
   svnicp_handle native_handle() const { return h_; }
 
  protected:
