@@ -243,6 +243,28 @@ int svnicp_map_get(svnicp_map m, const double position[3], double max_range, con
 int svnicp_map_download(svnicp_map m, double *out_xyz, int64_t n);
 /* Size() / Empty() (VoxelHashMap.h:55-56): live voxels and stored points */
 int svnicp_map_size(svnicp_map m, int64_t *voxels, int64_t *points);
+/* Registration objective of a scan at M caller-given poses against the map itself (no reference counterpart): score initial
+ * guesses before registration, gate a scan against the map, check relocalisation or loop-closure poses.
+ * source: [n][3] sensor-frame points, float (dtype_f64 = 0) or double, host or device (as svnicp_map_add_cloud).
+ * poses: [6][M] host doubles x = [t ; omega] relative to T0 = (R0 row-major, t0), the SVN-ICP particle convention:
+ *   T_world = T0 * (Exp(omega), t), i.e. R~ = R0 Exp(omega), t~ = t0 + R0 t.  x = 0 scores T0 itself.
+ * Per pose and source point: q = R~ s + t~ in fp64 (the fma order of the scan's q0; x = 0 gives q0 bit for bit) and the
+ *   EXACT nearest stored map point m (float widened to double, d^2 in the fp64 fma order of the candidate builder) among those
+ *   with d^2 < max_dist; an exact tie goes to the lexicographically smallest (x, y, z).  The same choice as a brute-force sweep
+ *   over GetMap().  max_dist has the registration's meaning (squared metres, Q1) and is also the robust scale D.
+ *   A non-finite query has no correspondence.
+ *   out_stats [M][3]  {inlier count, count / n, inlier RMSE in metres (0 without inliers)}
+ *   out_H [M][36], out_b [M][6]  (may be NULL)  Newton_grad_right at that pose on these correspondences (Q1-Q3: points without
+ *     a correspondence add I3 to the translation block), the layout of svnicp_get_gn_system
+ *   out_mask [M][n]  (may be NULL)  1 where the point has a correspondence
+ *   out_nearest [M][n][3]  (may be NULL)  float coordinates of the chosen map point, zeros where there is none
+ * Each pose's outputs are the same bits whatever M, its position among the poses, or the call.  Blocking, on the map's stream;
+ * changes no state of the map (Size(), the table, the last svnicp_map_get result stay valid).
+ * SVNICP_ERR_INVALID for null pointers, n outside [1, 2^30], n_poses < 1, a non-finite or non-positive max_dist, and a search
+ * radius sqrt(max_dist) beyond 4 voxels (ceil(sqrt(max_dist) / voxel_size) > 4). */
+int svnicp_map_evaluate(svnicp_map m, const void *source, int64_t n, int dtype_f64, int on_device, const double R0[9],
+                        const double t0[3], int n_poses, const double *poses_6xM, double max_dist, double *out_stats,
+                        double *out_H, double *out_b, uint8_t *out_mask, float *out_nearest);
 
 /* ---------------------------------------------------------------------------------------------
  * Scan pre-processing on the device, the step right before add_cloud in the reference's node

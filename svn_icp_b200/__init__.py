@@ -91,7 +91,7 @@ EXPORTS = [
     "svnicp_get_timing", "svnicp_get_slice", "svnicp_get_launch_count", "svnicp_set_profiling", "svnicp_get_phase_times",
     "svnicp_get_scan_info", "svnicp_get_tail_stamps", "svnicp_evaluate",
     "svnicp_map_create", "svnicp_map_destroy", "svnicp_map_last_error", "svnicp_map_clear", "svnicp_map_add_cloud", "svnicp_map_get",
-    "svnicp_map_download", "svnicp_map_size",
+    "svnicp_map_download", "svnicp_map_size", "svnicp_map_evaluate",
     "svnicp_pre_create", "svnicp_pre_destroy", "svnicp_pre_last_error", "svnicp_pre_crop", "svnicp_pre_downsample_uniform",
     "svnicp_pre_to_f64", "svnicp_pre_download", "svnicp_pre_deskew", "svnicp_pose_compose",
     "svnicp_batch_create", "svnicp_batch_destroy", "svnicp_batch_last_error", "svnicp_batch_size", "svnicp_batch_stream", "svnicp_batch_align",
@@ -152,6 +152,7 @@ def _ARGTYPES(V, I, L, D):
         "svnicp_evaluate": [V, I, V, V, V, V, V, V],
         "svnicp_map_create": [V, D, D, I, L, I], "svnicp_map_clear": [V], "svnicp_map_add_cloud": [V, V, L, I, I, V, V],
         "svnicp_map_get": [V, V, D, V, V], "svnicp_map_download": [V, V, L], "svnicp_map_size": [V, V, V],
+        "svnicp_map_evaluate": [V, V, L, I, I, V, V, I, V, D, V, V, V, V, V],
         "svnicp_pre_create": [V, L, I], "svnicp_pre_crop": [V, V, L, I, D, D, V, V, V],
         "svnicp_pre_downsample_uniform": [V, V, L, I, D, V, V], "svnicp_pre_to_f64": [V, V, L, V], "svnicp_pre_download": [V, V, L, V],
         "svnicp_pre_deskew": [V, V, L, I, V, I, I, V, V, V, V, V, V], "svnicp_pose_compose": [V, V, V, V, V],
@@ -589,6 +590,44 @@ class VoxelHashMap:
         out = np.zeros((n, 3))
         self._check(self._lib.svnicp_map_download(self._m, _p(out), C.c_int64(n)), "GetMap")
         return out
+
+    def Evaluate(self, source, R0, t0, poses, max_dist: float, want_system: bool = True, want_mask: bool = False,
+                 want_nearest: bool = False) -> dict:
+        """Registration objective of a scan at caller-given poses against this map (svnicp_map_evaluate; no reference
+        counterpart).  source: [n,3] float32 or float64 sensor-frame points, host.  poses: (6,) or (6, M) x = [t ; omega]
+        relative to T0 = (R0, t0) as the SVN-ICP particles (T_world = T0 * (Exp(omega), t); zeros score T0 itself).  Each point's
+        exact nearest map point with d^2 < max_dist (max_dist as in the registration, squared metres).  Returns the dict of
+        SVNICP.evaluate: inliers [M] int64, fitness [M], rmse [M] (metres); with want_system H [M, 6, 6], b [M, 6]; with want_mask
+        mask [M, n] uint8; with want_nearest nearest [M, n, 3] float32 (zeros where there is none).  A (6,) pose drops the M axis.
+        Changes no state of the map."""
+        a = np.asarray(source)
+        f64 = a.dtype != np.float32
+        a = np.ascontiguousarray(a, dtype=np.float64 if f64 else np.float32).reshape(-1, 3)
+        return self._evaluate(_p(a), len(a), f64, False, R0, t0, poses, max_dist, want_system, want_mask, want_nearest)
+
+    def EvaluateDevice(self, ptr: int, n: int, f64: bool, R0, t0, poses, max_dist: float, want_system: bool = True,
+                       want_mask: bool = False, want_nearest: bool = False) -> dict:
+        """Evaluate for a device cloud: ptr to [n,3] float32 (f64 = False, e.g. a ScanPreprocessor output) or float64."""
+        return self._evaluate(C.c_void_p(ptr), n, f64, True, R0, t0, poses, max_dist, want_system, want_mask, want_nearest)
+
+    def _evaluate(self, src, n, f64, on_device, R0, t0, poses, max_dist, want_system, want_mask, want_nearest):
+        x = np.asarray(poses, dtype=np.float64)
+        single = x.ndim == 1
+        x = np.ascontiguousarray(x.reshape(6, -1))
+        M = x.shape[1]
+        stats = np.zeros((M, 3))
+        H = np.zeros((M, 6, 6)) if want_system else None
+        b = np.zeros((M, 6)) if want_system else None
+        mask = np.zeros((M, n), dtype=np.uint8) if want_mask else None
+        near = np.zeros((M, n, 3), dtype=np.float32) if want_nearest else None
+        self._check(self._lib.svnicp_map_evaluate(self._m, src, C.c_int64(n), C.c_int(int(f64)), C.c_int(int(on_device)),
+                                                  _p(_f64(R0).reshape(9)), _p(_f64(t0).reshape(3)), C.c_int(M), _p(x),
+                                                  C.c_double(max_dist), _p(stats), _p(H), _p(b), _p(mask), _p(near)), "Evaluate")
+        out = dict(inliers=stats[:, 0].astype(np.int64), fitness=stats[:, 1].copy(), rmse=stats[:, 2].copy())
+        for k, v in (("H", H), ("b", b), ("mask", mask), ("nearest", near)):
+            if v is not None:
+                out[k] = v
+        return {k: v[0] for k, v in out.items()} if single else out
 
 
 class ScanPreprocessor:

@@ -58,7 +58,7 @@ __global__ void k_q0(const double *__restrict__ src, int n_s, ScanConst sc, doub
   double r[3];
 #pragma unroll
   for (int a = 0; a < 3; a++) {
-    q0[3 * i + a] = fma(sc.R0[3 * a], x, fma(sc.R0[3 * a + 1], y, fma(sc.R0[3 * a + 2], z, sc.t0[a])));
+    q0[3 * i + a] = affine_row_fma(sc.R0, sc.t0, a, x, y, z);
     r[a] = fma(sc.R0[3 * a], x, fma(sc.R0[3 * a + 1], y, sc.R0[3 * a + 2] * z));
   }
   const float fx = __double2float_rn(r[0]), fy = __double2float_rn(r[1]), fz = __double2float_rn(r[2]);
@@ -262,11 +262,6 @@ __device__ int warp_cut(Ent *buf, int count, int K, double *cut_scale, int *cut_
   *cut_scale = scale;
   *cut_bin = tbin;
   return m_out;
-}
-
-__device__ __forceinline__ double dist2(const double q[3], const double *__restrict__ m) {
-  const double dx = q[0] - m[0], dy = q[1] - m[1], dz = q[2] - m[2];
-  return fma(dz, dz, fma(dy, dy, dx * dx));  // knn.cu:101-106 after nvcc's fma contraction
 }
 
 __global__ void __launch_bounds__(KNN_WARPS * 32)

@@ -201,6 +201,18 @@ __device__ __forceinline__ void euler_R(const double *x6, double *R) {
   R[6] = -sp;     R[7] = sr * cp;                R[8] = cr * cp;
 }
 
+// Row a of q = R s + t in fp64, in the fma order of k_q0 (the scan's q0 = R0 s + t0, SVGDICP.cpp:204) and of
+// oracle_transform_q0.  Shared by k_q0 and k_map_eval (svnicp_map_evaluate), so a pose x = 0 queries the map at exactly q0.
+__device__ __forceinline__ double affine_row_fma(const double *R, const double *t, int a, double x, double y, double z) {
+  return fma(R[3 * a], x, fma(R[3 * a + 1], y, fma(R[3 * a + 2], z, t[a])));
+}
+
+// Squared distance in fp64 (knn.cu:101-106 after nvcc's fma contraction): k_knn's candidate sets and k_map_eval's nearest map point.
+__device__ __forceinline__ double dist2(const double q[3], const double *__restrict__ m) {
+  const double dx = q[0] - m[0], dy = q[1] - m[1], dz = q[2] - m[2];
+  return fma(dz, dz, fma(dy, dy, dx * dx));
+}
+
 // fp32 transform of one pose (R, t) in coordinates relative to the scan's initial-guess query q0:
 // xf[0..9) = A' = R0 (R - I) R0^T (row-major), xf[9..12) = tau = R0 t, so that q_pb - q0_b = A' (R0 s_b) + tau.
 // The one place this is computed: k_prep (iteration 0), k_tail (iterations >= 1) and k_eval_prep (svnicp_evaluate).

@@ -248,8 +248,14 @@ int launch_eval_block(const EvalArgs &a, bool want_system, const ScanConst &sc, 
   const size_t smem = eval_smem_bytes(a.G, a.K);
   if (want_system) go_corr<true>(a, grid, smem, st);
   else go_corr<false>(a, grid, smem, st);
-  k_eval_fin<<<a.MB, EV_NS * 32, 0, st>>>(a.part, grid, a.MB, a.n_s, sc, R_blk, out_blk);
+  launch_eval_fin(a.part, grid, a.MB, a.n_s, sc, R_blk, out_blk, st);
   return 2;
+}
+
+int launch_eval_fin(const double *part, int n_parts, int MB, int n_s, const ScanConst &sc, const double *R_blk, double *out_blk,
+                    cudaStream_t st) {
+  k_eval_fin<<<MB, EV_NS * 32, 0, st>>>(part, n_parts, MB, n_s, sc, R_blk, out_blk);
+  return 1;
 }
 
 }  // namespace svn

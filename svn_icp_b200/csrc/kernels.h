@@ -172,6 +172,10 @@ int eval_parts(int n_s, int K, int sm_count);  // CTAs of the correspondence pas
 int launch_eval_prep(const double *poses, int M, int euler, const ScanConst &sc, float *xf, double *R, cudaStream_t st);
 int launch_eval_block(const EvalArgs &a, bool want_system, const ScanConst &sc, const double *R_blk, double *out_blk, int sm_count,
                       cudaStream_t st);
+// k_eval_fin alone: per-CTA partials part [n_parts][MB][EV_NS] -> out_blk [MB][EV_OUT] (stats, then H and b by gn_assemble with
+// sc.R0 and the poses' rotations R_blk [MB][9]).  Also the back end of svnicp_map_evaluate (voxel_map.cu).
+int launch_eval_fin(const double *part, int n_parts, int MB, int n_s, const ScanConst &sc, const double *R_blk, double *out_blk,
+                    cudaStream_t st);
 void init_eval_kernels();
 
 // ---- SVGD-ICP class (class_type = SVGDICP, svgd_class.cu): first-order gradient + torch::optim-style update ----

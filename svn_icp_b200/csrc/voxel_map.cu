@@ -13,15 +13,22 @@
 // index as the voxel's walker; pass 2 lets the walker keep the (cap - count) lowest indices, ascending.
 // The table is open addressing (linear probing) over packed 3x21-bit voxel indices; RemoveFar rebuilds into the twin table
 // (no tombstones).  Point output order of GetMap is slot order: arbitrary like the reference's robin_map iteration.
+//
+// svnicp_map_evaluate (DESIGN.md section 10b) scores a scan at caller-given poses against the table itself: an exact
+// nearest-map-point search per (source point, pose) by read-only probes of the same hash (k_map_eval), then the fixed-order
+// reduction of svnicp_evaluate (k_eval_fin, eval_kernels.cu).
 #include <cuda_runtime.h>
 #include <limits.h>
+#include <math.h>
 #include <stdint.h>
 #include <stdio.h>
 #include <string.h>
 
 #include <string>
+#include <vector>
 
 #include "../../include/svnicp_b200.h"
+#include "kernels.h"
 
 namespace {
 
@@ -242,6 +249,193 @@ __global__ void k_fill_i32(int *p, int v, size_t n) {
   if (i < n) p[i] = v;
 }
 
+// ---- svnicp_map_evaluate ----------------------------------------------------------------------------------------------------
+constexpr int MEV_THREADS = 128;     // 4 warps; a warp holds 32 consecutive source points of one pose (ring order: shared voxels)
+constexpr int MEV_CTAS_PER_SM = 8;   // partial slots per SM (the grid-stride over the source points depends on n and SMs only)
+constexpr int MEV_MAX_REACH = 4;     // ceil(sqrt(max_dist) / voxel_size) allowed: at most 9^3 voxels per query
+constexpr int MEV_SPAN = 2 * MEV_MAX_REACH + 4;  // voxels per axis of a search box beyond which a query sweeps the whole table
+constexpr double MEV_MARGIN = 1.0 + 1e-12;       // search radii exceed sqrt(d^2) by far more than dist2's rounding (< 4 ulp)
+
+// Read-only probe: the slot holding key, or -1 when the voxel is absent or holds no point.  There are no tombstones (far voxels
+// leave by a rebuild into the twin table), so the walk may stop at the first empty slot.
+__device__ __forceinline__ int map_find(const MapTable &t, int slots_mask, unsigned long long key) {
+  unsigned slot = hash_key(key) & (unsigned)slots_mask;
+  for (int probe = 0; probe <= slots_mask; probe++) {
+    const unsigned long long k = __ldg(t.keys + slot);
+    if (k == key) return __ldg(t.count + slot) > 0 ? (int)slot : -1;
+    if (k == EMPTY_KEY) return -1;
+    slot = (slot + 1) & (unsigned)slots_mask;
+  }
+  return -1;
+}
+
+// Per pose of a block, x = [t ; omega] relative to T0 = (R0, t0): R~ = R0 Exp(omega), t~ = t0 + R0 t -> Rt [MB][12], and
+// R_p = Exp(omega) -> Rp [MB][9] for gn_assemble.  x = 0 gives R_p = I exactly, and (R0, t0) is stored as given, so the
+// query of a pose x = 0 is q0 bit for bit (the products would turn a -0 entry of R0 into +0).
+__global__ void k_map_eval_prep(const double *x6 /*[MB][6]*/, int MB, svn::ScanConst sc, double *Rt, double *Rp) {
+  const int p = threadIdx.x;
+  if (p >= MB) return;
+  const double *x = x6 + 6 * p;
+  double R[9];
+  svn::so3_exp(x + 3, R, nullptr);
+  const bool zero = x[0] == 0.0 && x[1] == 0.0 && x[2] == 0.0 && x[3] == 0.0 && x[4] == 0.0 && x[5] == 0.0;
+  double *o = Rt + 12 * p;
+#pragma unroll
+  for (int r = 0; r < 3; r++) {
+#pragma unroll
+    for (int c = 0; c < 3; c++)
+      o[3 * r + c] = zero ? sc.R0[3 * r + c] : sc.R0[3 * r] * R[c] + sc.R0[3 * r + 1] * R[3 + c] + sc.R0[3 * r + 2] * R[6 + c];
+    o[9 + r] = zero ? sc.t0[r] : sc.t0[r] + (sc.R0[3 * r] * x[0] + sc.R0[3 * r + 1] * x[1] + sc.R0[3 * r + 2] * x[2]);
+  }
+#pragma unroll
+  for (int i = 0; i < 9; i++) Rp[9 * p + i] = R[i];
+}
+
+// Voxel range [lo, hi] of one axis that holds every stored point p with |p_a - q_a| <= rad.  A point was filed under
+// trunc(fl32(p_a / v)) (k_map_insert_link, VoxelHashMap.cpp:30).  With lo_f = fl32 of (q_a - rad) rounded down, both roundings
+// downward, and hi_f likewise upward, lo_f <= p_a <= hi_f, because p_a is itself a float.  fp32 division by v > 0 (round to
+// nearest) is monotone and so is truncation toward zero, hence trunc(fl32(lo_f / v)) <= voxel_a(p) <= trunc(fl32(hi_f / v)).
+// Truncation files (-v, v) under voxel 0, which is twice as wide as the others; monotonicity holds across it, so a box that
+// straddles zero contains voxel 0 and none of its points are skipped.  Saturating conversions (|q| beyond 2^31 v) stay monotone.
+__device__ __forceinline__ void box_axis(double q, double rad, float v, int &lo, int &hi) {
+  lo = (int)__fdiv_rn(__double2float_rd(__dsub_rd(q, rad)), v);
+  hi = (int)__fdiv_rn(__double2float_ru(__dadd_ru(q, rad)), v);
+}
+
+struct NearestState {
+  double q[3];
+  double bd;  // best d^2 so far (max_dist until a point qualifies: d^2 < max_dist)
+  float bx, by, bz;
+  bool found;
+};
+
+// every point of one voxel: smaller d^2 wins, an exact tie goes to the lexicographically smaller (x, y, z) -- data only
+__device__ __forceinline__ void visit_slot(const MapTable &t, int cap, int slot, NearestState &s) {
+  const int c = __ldg(t.count + slot);
+  const float *p = t.pts + (size_t)slot * cap * 3;
+  for (int k = 0; k < c; k++) {
+    const float px = __ldg(p + 3 * k), py = __ldg(p + 3 * k + 1), pz = __ldg(p + 3 * k + 2);
+    const double mp[3] = {(double)px, (double)py, (double)pz};
+    const double d = svn::dist2(s.q, mp);
+    const bool lex = px < s.bx || (px == s.bx && (py < s.by || (py == s.by && pz < s.bz)));
+    if (d < s.bd || (s.found && d == s.bd && lex)) { s.bd = d; s.bx = px; s.by = py; s.bz = pz; s.found = true; }
+  }
+}
+
+// Exact nearest stored point of a finite query within d^2 < max_dist (the same choice as a brute-force sweep over GetMap()).
+// The query's own voxel first; then the box shrinks to the best distance found and every other voxel of it is visited.
+__device__ __forceinline__ void map_nearest(const MapDev &m, double r, NearestState &s) {
+  const float v = m.voxel_size_f;
+  int lo[3], hi[3];
+  bool wide = false;
+#pragma unroll
+  for (int a = 0; a < 3; a++) {
+    box_axis(s.q[a], r, v, lo[a], hi[a]);
+    wide |= (long long)hi[a] - lo[a] >= MEV_SPAN;
+  }
+  if (wide) {  // float spacing of q coarser than the voxels (|q| >~ 2^24 v): sweep the table, still exact
+    for (int slot = 0; slot <= m.slots_mask; slot++)
+      if (__ldg(m.tab.keys + slot) != EMPTY_KEY) visit_slot(m.tab, m.cap, slot, s);
+    return;
+  }
+  int own[3];
+#pragma unroll
+  for (int a = 0; a < 3; a++) own[a] = (int)__fdiv_rn(__double2float_rn(s.q[a]), v);
+  int slot = map_find(m.tab, m.slots_mask, pack_key(own[0], own[1], own[2]));
+  if (slot >= 0) visit_slot(m.tab, m.cap, slot, s);
+  if (s.found) {
+    const double rb = fmin(r, sqrt(s.bd) * MEV_MARGIN);
+#pragma unroll
+    for (int a = 0; a < 3; a++) box_axis(s.q[a], rb, v, lo[a], hi[a]);
+  }
+  for (int z = lo[2]; z <= hi[2]; z++)
+    for (int y = lo[1]; y <= hi[1]; y++)
+      for (int x = lo[0]; x <= hi[0]; x++) {
+        if (x == own[0] && y == own[1] && z == own[2]) continue;
+        slot = map_find(m.tab, m.slots_mask, pack_key(x, y, z));
+        if (slot >= 0) visit_slot(m.tab, m.cap, slot, s);
+      }
+}
+
+// One thread per (source point, pose): grid.x = partial slots (grid-stride over the points), grid.y = the poses of the block.
+// Sums per pose, as k_eval_corr: the 16 Gauss-Newton sums in the world-oriented frame (s' = R0 s, e = q - m, R~ s), the inlier
+// count and the inlier sum of d^2; fp64 per thread, a fixed butterfly per warp, the warps in ascending order per CTA.
+// Queries without a correspondence (no point with d^2 < max_dist, or a non-finite query) add only +1 to W (Q2).
+// Launch bounds: with the system 128 registers (4 CTAs per SM), without it 64 (8 CTAs); below that ptxas spills.
+template <typename T, bool SYS>
+__global__ void __launch_bounds__(MEV_THREADS, SYS ? 4 : 8) k_map_eval(MapDev m, const T *__restrict__ src, int n, const double *__restrict__ Rt,
+                                                          svn::ScanConst sc, double max_dist, double r, double *part,
+                                                          uint8_t *mask, float *nearest) {
+  using svn::EV_NS;
+  __shared__ double s_w[MEV_THREADS / 32][EV_NS];
+  const int p = blockIdx.y, MB = gridDim.y;
+  const double *P = Rt + 12 * p;
+  double Rtl[9], ttl[3];
+#pragma unroll
+  for (int i = 0; i < 9; i++) Rtl[i] = P[i];
+#pragma unroll
+  for (int i = 0; i < 3; i++) ttl[i] = P[9 + i];
+  const double D = max_dist;
+  double acc[EV_NS];
+#pragma unroll
+  for (int j = 0; j < EV_NS; j++) acc[j] = 0.0;
+  for (int i = blockIdx.x * MEV_THREADS + threadIdx.x; i < n; i += gridDim.x * MEV_THREADS) {
+    const double x = (double)src[3 * (size_t)i], y = (double)src[3 * (size_t)i + 1], z = (double)src[3 * (size_t)i + 2];
+    NearestState s;
+#pragma unroll
+    for (int a = 0; a < 3; a++) s.q[a] = svn::affine_row_fma(Rtl, ttl, a, x, y, z);
+    s.bd = max_dist;
+    s.bx = s.by = s.bz = 0.f;
+    s.found = false;
+    if (isfinite(s.q[0]) && isfinite(s.q[1]) && isfinite(s.q[2])) map_nearest(m, r, s);
+    if (mask) mask[(size_t)p * n + i] = s.found ? 1 : 0;
+    if (nearest) {
+      float *o = nearest + ((size_t)p * n + i) * 3;
+      o[0] = s.bx; o[1] = s.by; o[2] = s.bz;
+    }
+    if (!s.found) {
+      if (SYS) acc[0] += 1.0;  // masked: +1 on the translation block (Q2); nothing else, so a NaN never reaches the sums
+      continue;
+    }
+    acc[16] += 1.0;
+    acc[17] += s.bd;
+    if (SYS) {
+      double sp[3], w[3];
+#pragma unroll
+      for (int a = 0; a < 3; a++) {
+        sp[a] = fma(sc.R0[3 * a], x, fma(sc.R0[3 * a + 1], y, sc.R0[3 * a + 2] * z));  // s' = R0 s
+        w[a] = fma(Rtl[3 * a], x, fma(Rtl[3 * a + 1], y, Rtl[3 * a + 2] * z));        // R~ s
+      }
+      const double e[3] = {s.q[0] - (double)s.bx, s.q[1] - (double)s.by, s.q[2] - (double)s.bz};
+      const double wq = D / (D + 3.0 * sqrt(s.bd));
+      const double rho = wq * wq;  // (D / (D + 3 |e|))^2, SVNICP.cpp:120-122
+      acc[0] += rho;
+      const double g[3] = {rho * sp[0], rho * sp[1], rho * sp[2]};
+      acc[1] += g[0]; acc[2] += g[1]; acc[3] += g[2];
+      acc[4] += g[0] * sp[0]; acc[5] += g[0] * sp[1]; acc[6] += g[0] * sp[2];
+      acc[7] += g[1] * sp[1]; acc[8] += g[1] * sp[2]; acc[9] += g[2] * sp[2];
+      const double f[3] = {rho * e[0], rho * e[1], rho * e[2]};
+      acc[10] += f[0]; acc[11] += f[1]; acc[12] += f[2];
+      acc[13] += w[1] * f[2] - w[2] * f[1];
+      acc[14] += w[2] * f[0] - w[0] * f[2];
+      acc[15] += w[0] * f[1] - w[1] * f[0];
+    }
+  }
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+  for (int j = 0; j < EV_NS; j++) {
+    const double v = svn::warp_sum(acc[j]);
+    if (lane == 0) s_w[warp][j] = v;
+  }
+  __syncthreads();
+  if (threadIdx.x < EV_NS) {
+    double t = 0.0;
+#pragma unroll
+    for (int w = 0; w < MEV_THREADS / 32; w++) t += s_w[w][threadIdx.x];
+    part[((size_t)blockIdx.x * MB + p) * EV_NS + threadIdx.x] = t;
+  }
+}
+
 }  // namespace
 
 struct svnicp_map_t {
@@ -265,6 +459,14 @@ struct svnicp_map_t {
   size_t out_cap = 0;
   int *block_sums = nullptr;
   long long last_n = 0;
+  // svnicp_map_evaluate scratch (grown on demand; nothing above is touched by it)
+  void *ev_src = nullptr;
+  double *ev_pose = nullptr;  // [EV_BLOCK][6] x, [EV_BLOCK][12] R~ t~, [EV_BLOCK][9] R_p
+  double *ev_part = nullptr, *ev_out = nullptr;
+  uint8_t *ev_mask = nullptr;
+  float *ev_near = nullptr;
+  size_t ev_src_cap = 0, ev_part_cap = 0, ev_mask_cap = 0, ev_near_cap = 0;
+  int sm_count = 148;
   cudaStream_t stream = nullptr;
   std::string err;
 };
@@ -318,6 +520,7 @@ int svnicp_map_create(svnicp_map *out, double voxel_size, double max_range, int 
   m->slots = slots;
   auto body = [&]() -> int {
     MCU(cudaSetDevice(device));
+    MCU(cudaDeviceGetAttribute(&m->sm_count, cudaDevAttrMultiProcessorCount, device));
     MCU(cudaStreamCreateWithFlags(&m->stream, cudaStreamNonBlocking));
     for (int w = 0; w < 2; w++) {
       MCU(cudaMalloc((void **)&m->tab[w].keys, slots * sizeof(unsigned long long)));
@@ -328,6 +531,8 @@ int svnicp_map_create(svnicp_map *out, double voxel_size, double max_range, int 
     MCU(cudaMalloc((void **)&m->walker, slots * sizeof(int)));
     MCU(cudaMalloc((void **)&m->counters, 4 * sizeof(long long)));
     MCU(cudaMalloc((void **)&m->d_pose, 16 * sizeof(double)));
+    MCU(cudaMalloc((void **)&m->ev_pose, (size_t)svn::EV_BLOCK * 27 * sizeof(double)));
+    MCU(cudaMalloc((void **)&m->ev_out, (size_t)svn::EV_BLOCK * svn::EV_OUT * sizeof(double)));
     MCU(cudaMalloc((void **)&m->block_sums, ((slots + SCAN_BLOCK - 1) / SCAN_BLOCK + 1) * sizeof(int)));
     MCU(cudaMallocHost((void **)&m->h_counters, 4 * sizeof(long long)));
     memset(m->h_counters, 0, 4 * sizeof(long long));
@@ -351,6 +556,7 @@ void svnicp_map_destroy(svnicp_map m) {
   for (int w = 0; w < 2; w++) { cudaFree(m->tab[w].keys); cudaFree(m->tab[w].count); cudaFree(m->tab[w].pts); }
   cudaFree(m->head); cudaFree(m->walker); cudaFree(m->counters); cudaFree(m->d_pose); cudaFree(m->block_sums);
   cudaFree(m->batch_in); cudaFree(m->wxyz); cudaFree(m->pt_slot); cudaFree(m->next); cudaFree(m->out);
+  cudaFree(m->ev_src); cudaFree(m->ev_pose); cudaFree(m->ev_part); cudaFree(m->ev_out); cudaFree(m->ev_mask); cudaFree(m->ev_near);
   if (m->h_counters) cudaFreeHost(m->h_counters);
   if (m->stream) cudaStreamDestroy(m->stream);
   delete m;
@@ -486,3 +692,97 @@ int svnicp_map_size(svnicp_map m, int64_t *voxels, int64_t *points) {  // VoxelH
 }
 
 }  // extern "C"
+
+// device scratch of svnicp_map_evaluate: (re)allocate *p to hold at least `bytes`
+static int ev_grow(svnicp_map m, void **p, size_t *cap, size_t bytes) {
+  if (bytes <= *cap) return SVNICP_OK;
+  cudaFree(*p);
+  *p = nullptr;
+  *cap = 0;
+  MCU(cudaMalloc(p, bytes));
+  *cap = bytes;
+  return SVNICP_OK;
+}
+
+template <bool SYS>
+static void go_map_eval(const MapDev &d, const void *src, int dtype_f64, dim3 grid, int n, const double *Rt, const svn::ScanConst &sc,
+                        double max_dist, double r, double *part, uint8_t *mask, float *nearest, cudaStream_t st) {
+  if (dtype_f64)
+    k_map_eval<double, SYS><<<grid, MEV_THREADS, 0, st>>>(d, (const double *)src, n, Rt, sc, max_dist, r, part, mask, nearest);
+  else
+    k_map_eval<float, SYS><<<grid, MEV_THREADS, 0, st>>>(d, (const float *)src, n, Rt, sc, max_dist, r, part, mask, nearest);
+}
+
+extern "C" int svnicp_map_evaluate(svnicp_map m, const void *source, int64_t n, int dtype_f64, int on_device, const double R0[9],
+                                   const double t0[3], int n_poses, const double *poses_6xM, double max_dist, double *out_stats,
+                                   double *out_H, double *out_b, uint8_t *out_mask, float *out_nearest) {
+  using svn::EV_BLOCK;
+  using svn::EV_NS;
+  using svn::EV_OUT;
+  if (!m) return SVNICP_ERR_INVALID;
+  if (!source || !R0 || !t0 || !poses_6xM || !out_stats)
+    return mfail(m, SVNICP_ERR_INVALID, "svnicp_map_evaluate: null source, R0, t0, poses or out_stats");
+  if (n < 1 || n > (1ll << 30)) return mfail(m, SVNICP_ERR_INVALID, "svnicp_map_evaluate: need 1 <= n <= 2^30 source points");
+  if (n_poses < 1) return mfail(m, SVNICP_ERR_INVALID, "svnicp_map_evaluate: n_poses must be >= 1");
+  if (!isfinite(max_dist) || !(max_dist > 0)) return mfail(m, SVNICP_ERR_INVALID, "svnicp_map_evaluate: max_dist must be finite and > 0");
+  const double r = sqrt(max_dist);
+  if (ceil(r / m->voxel_size) > MEV_MAX_REACH) {
+    char buf[256];
+    snprintf(buf, sizeof(buf), "svnicp_map_evaluate: search radius sqrt(max_dist) = %g m spans %g voxels of %g m on each side of the "
+             "query; at most %d are supported", r, ceil(r / m->voxel_size), m->voxel_size, MEV_MAX_REACH);
+    return mfail(m, SVNICP_ERR_INVALID, buf);
+  }
+  MCU(cudaSetDevice(m->device));
+  cudaStream_t st = m->stream;
+  const int ni = (int)n, M = n_poses;
+  const int mb_max = M < EV_BLOCK ? M : EV_BLOCK;
+  int parts = (int)((n + MEV_THREADS - 1) / MEV_THREADS);
+  if (parts > m->sm_count * MEV_CTAS_PER_SM) parts = m->sm_count * MEV_CTAS_PER_SM;
+  const size_t esz = dtype_f64 ? sizeof(double) : sizeof(float);
+  int rc;
+  if ((rc = ev_grow(m, (void **)&m->ev_part, &m->ev_part_cap, (size_t)parts * mb_max * EV_NS * sizeof(double))) ||
+      (!on_device && (rc = ev_grow(m, &m->ev_src, &m->ev_src_cap, (size_t)n * 3 * esz))) ||
+      (out_mask && (rc = ev_grow(m, (void **)&m->ev_mask, &m->ev_mask_cap, (size_t)mb_max * n))) ||
+      (out_nearest && (rc = ev_grow(m, (void **)&m->ev_near, &m->ev_near_cap, (size_t)mb_max * n * 3 * sizeof(float)))))
+    return rc;
+  const void *src = source;
+  if (!on_device) {
+    MCU(cudaMemcpyAsync(m->ev_src, source, (size_t)n * 3 * esz, cudaMemcpyHostToDevice, st));
+    src = m->ev_src;
+  }
+  svn::ScanConst sc;
+  memcpy(sc.R0, R0, sizeof(sc.R0));
+  memcpy(sc.t0, t0, sizeof(sc.t0));
+  double *x_blk = m->ev_pose, *Rt_blk = m->ev_pose + 6 * EV_BLOCK, *Rp_blk = m->ev_pose + 18 * EV_BLOCK;
+  const MapDev d = dev_view(m, m->cur);
+  const bool sys = out_H || out_b;
+  std::vector<double> hx((size_t)6 * EV_BLOCK), res((size_t)EV_OUT * EV_BLOCK);
+  for (int m0 = 0; m0 < M; m0 += EV_BLOCK) {
+    const int MB = M - m0 < EV_BLOCK ? M - m0 : EV_BLOCK;
+    for (int j = 0; j < MB; j++)
+      for (int c = 0; c < 6; c++) hx[(size_t)6 * j + c] = poses_6xM[(size_t)c * M + m0 + j];
+    MCU(cudaMemcpyAsync(x_blk, hx.data(), (size_t)6 * MB * sizeof(double), cudaMemcpyHostToDevice, st));
+    k_map_eval_prep<<<1, EV_BLOCK, 0, st>>>(x_blk, MB, sc, Rt_blk, Rp_blk);
+    const dim3 grid((unsigned)parts, (unsigned)MB);
+    uint8_t *mk = out_mask ? m->ev_mask : nullptr;
+    float *nr = out_nearest ? m->ev_near : nullptr;
+    if (sys) go_map_eval<true>(d, src, dtype_f64, grid, ni, Rt_blk, sc, max_dist, r * MEV_MARGIN, m->ev_part, mk, nr, st);
+    else go_map_eval<false>(d, src, dtype_f64, grid, ni, Rt_blk, sc, max_dist, r * MEV_MARGIN, m->ev_part, mk, nr, st);
+    svn::launch_eval_fin(m->ev_part, parts, MB, ni, sc, Rp_blk, m->ev_out, st);
+    MCU(cudaGetLastError());
+    MCU(cudaMemcpyAsync(res.data(), m->ev_out, (size_t)EV_OUT * MB * sizeof(double), cudaMemcpyDeviceToHost, st));
+    // [M][n] outputs: the rows of this block are contiguous in the caller's arrays
+    if (out_mask) MCU(cudaMemcpyAsync(out_mask + (size_t)m0 * n, m->ev_mask, (size_t)MB * n, cudaMemcpyDeviceToHost, st));
+    if (out_nearest)
+      MCU(cudaMemcpyAsync(out_nearest + (size_t)m0 * n * 3, m->ev_near, (size_t)MB * n * 3 * sizeof(float), cudaMemcpyDeviceToHost, st));
+    MCU(cudaStreamSynchronize(st));  // the host block buffers are refilled next
+    for (int j = 0; j < MB; j++) {
+      const double *o = res.data() + (size_t)EV_OUT * j;
+      const size_t g = (size_t)m0 + j;
+      memcpy(out_stats + 3 * g, o, 3 * sizeof(double));
+      if (out_H) memcpy(out_H + 36 * g, o + 3, 36 * sizeof(double));
+      if (out_b) memcpy(out_b + 6 * g, o + 39, 6 * sizeof(double));
+    }
+  }
+  return SVNICP_OK;
+}

@@ -63,6 +63,31 @@ struct VoxelHashMap {
     return v;
   }
 
+  /** Registration objective of a scan at M poses against this map (svnicp_map_evaluate; no reference counterpart).  xyz: n float
+   *  xyz triples in the sensor frame (host, or device with on_device).  poses_6xM: [6][M] x = [t ; omega] relative to T0, the
+   *  SVN-ICP particle convention (zeros score T0 itself).  Each point's exact nearest map point with d^2 < max_dist (squared
+   *  metres, as the registration's threshold).  Returns the result type of SVGDICP::evaluate.  Changes no state of the map. */
+  SVGDICP::Evaluation Evaluate(const float *xyz, int64_t n, const InitialMean &T0, const std::vector<double> &poses_6xM, double max_dist,
+                               bool want_system = true, bool want_mask = false, bool on_device = false) {
+    if (poses_6xM.empty() || poses_6xM.size() % 6 != 0) throw Error("Evaluate: poses must hold 6*M doubles");
+    SVGDICP::Evaluation r;
+    r.n_poses = (int)(poses_6xM.size() / 6);
+    const size_t M = (size_t)r.n_poses;
+    std::vector<double> stats(3 * M);
+    if (want_system) { r.H.resize(36 * M); r.b.resize(6 * M); }
+    if (want_mask && n > 0) r.mask.resize(M * (size_t)n);
+    check(svnicp_map_evaluate(m_, xyz, n, 0, on_device, T0.R.data(), T0.t.data(), r.n_poses, poses_6xM.data(), max_dist, stats.data(),
+                              want_system ? r.H.data() : nullptr, want_system ? r.b.data() : nullptr,
+                              want_mask ? r.mask.data() : nullptr, nullptr),
+          "Evaluate");
+    for (size_t m = 0; m < M; m++) {
+      r.inliers.push_back((int64_t)stats[3 * m]);
+      r.fitness.push_back(stats[3 * m + 1]);
+      r.rmse.push_back(stats[3 * m + 2]);
+    }
+    return r;
+  }
+
  private:
   void check(int rc, const char *what) const {
     if (rc < 0) throw Error(std::string(what) + ": " + svnicp_map_last_error(m_));
