@@ -703,11 +703,6 @@ struct AlignState {
   unsigned seq0 = 0;
   int I = 0, e = 0;
 };
-#define ALIGN_LOCALS                                                                                                     \
-  IterArgs &ia = S.ia; SteinArgs &sa = S.sa; const SvgdArgs &sv = S.sv; PeerTable &pt = S.pt;                            \
-  const bool svgd = S.svgd, overlap = S.overlap; const unsigned seq0 = S.seq0; const int I = S.I;                        \
-  cudaStream_t st = h->stream, hs = h->head_stream;                                                                      \
-  (void)ia; (void)sa; (void)sv; (void)pt; (void)svgd; (void)overlap; (void)seq0; (void)I; (void)st; (void)hs;
 
 static int align_begin(svnicp_handle h, AlignState &S) {
   if (!h->have_cloud) return fail(h, SVNICP_ERR_INVALID, "stein_align before add_cloud");
@@ -862,200 +857,208 @@ static int align_begin(svnicp_handle h, AlignState &S) {
   return SVNICP_OK;
 }
 
-// enqueue iteration S.e (SVNICP.cpp:52-108)
+// Sequence number s of the peer exchange.  Without the exchange (pt.n_ranks == 1) no kernel waits on or publishes one, so it is
+// 0 there: a captured iteration then depends on e only through its list-buffer parity, and one graph per parity replays all.
+static unsigned peer_seq(const AlignState &S, int s) { return S.pt.n_ranks > 1 ? S.seq0 + (unsigned)s : 0u; }
+
+// The head chain of iteration e (epilogue: after the last one) on stream s; adds its launches to n.  Iteration 0 waits for no
+// peer: every rank's k_prep wrote the x of all particles.
+static int head_chain(svnicp_handle h, const AlignState &S, int e, int epilogue, cudaStream_t s, int &n) {
+  const int k = launch_head(S.sa, S.pt, e > 0 ? peer_seq(S, e) : 0u, epilogue, s);
+  if (k < 0) return fail(h, SVNICP_ERR_CUDA, "launch of k_head failed: %s", cudaGetErrorString(cudaGetLastError()));
+  n += k;
+  return SVNICP_OK;
+}
+
+// List buffers of iteration e.  With list reuse they ping-pong by parity: iteration e prunes the lists of iteration e-1
+// wherever its ball still covers this one's.
+static void select_lists(svnicp_handle h, IterArgs &ia, int e) {
+  const int cur = h->filter_reuse ? e & 1 : 0;
+  ia.clist = cur ? h->clist2.p : h->clist.p;
+  ia.hdr = cur ? h->hdr2.p : h->hdr.p;
+  if (!h->filter_reuse) return;
+  ia.cbase = h->cbase[cur].p;
+  ia.ball = h->ball[cur].p;
+  ia.clist_prev = e > 0 ? (cur ? h->clist.p : h->clist2.p) : nullptr;
+  ia.cbase_prev = h->cbase[cur ^ 1].p;
+  ia.ball_prev = h->ball[cur ^ 1].p;
+  ia.kept_hist = h->kept_hist.p;
+}
+
+// Before phase k of iteration e: the per-phase event (svnicp_set_profiling), and with SVNICP_FLAG_DEBUG_SYNC a wait for the
+// device that is reported on stderr (localises a hang or a fault).  Both keep a scan off the graphs, so neither runs in a capture.
+static int phase_mark(svnicp_handle h, int e, int k) {
+  if (h->profile) CU(cudaEventRecord(h->prof_events[(size_t)e * 7 + k], h->stream));
+  if (h->prm.flags & SVNICP_FLAG_DEBUG_SYNC) {
+    fprintf(stderr, "[svnicp] iteration %d: before phase %d ...", e, k);
+    fflush(stderr);
+    const cudaError_t e1 = cudaStreamSynchronize(h->stream), e2 = cudaStreamSynchronize(h->head_stream);
+    fprintf(stderr, " main %s, head %s\n", cudaGetErrorString(e1), cudaGetErrorString(e2));
+    fflush(stderr);
+  }
+  return SVNICP_OK;
+}
+
+// Enqueue iteration e (SVNICP.cpp:52-108) of either class; returns its number of launches or a negative status.  Graph capture
+// and direct launches both run this code.  The side-stream head chain (overlap) forks from ev_fork, recorded on the main stream
+// in the same capture (or outside any), and joins it through ev_join.
+static int enqueue_iteration(svnicp_handle h, AlignState &S, int e, cudaEvent_t ev_fork, cudaEvent_t ev_join) {
+  IterArgs &ia = S.ia;
+  SteinArgs &sa = S.sa;
+  cudaStream_t st = h->stream, hs = h->head_stream;
+  int n = 0;
+  if (int rc = phase_mark(h, e, 0)) return rc;
+  if (S.svgd) n += launch_prep(ia, st, 0, nullptr);
+  else if (S.overlap) {
+    CU(cudaStreamWaitEvent(hs, ev_fork, 0));
+    if (int rc = head_chain(h, S, e, 0, hs, n)) return rc;
+    CU(cudaEventRecord(ev_join, hs));
+  }
+  if (int rc = phase_mark(h, e, 1)) return rc;
+  select_lists(h, ia, e);
+  n += launch_filter(ia, st);
+  if (int rc = phase_mark(h, e, 2)) return rc;
+  n += launch_gn(ia, st);
+  if (h->prm.debug_corr) {  // parity tap: the transforms this iteration's correspondences were computed with
+    CU(h->dbg_xf.ensure((size_t)(h->P_l > 0 ? h->P_l : 1) * 12));
+    CU(cudaMemcpyAsync(h->dbg_xf.p, h->xf.p, (size_t)h->P_l * 12 * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  }
+  if (int rc = phase_mark(h, e, 3)) return rc;
+  if (S.svgd) {
+    n += launch_finalize_first(ia, S.sv, st);
+    if (int rc = phase_mark(h, e, 4)) return rc;
+    if (int rc = do_allgather(h)) return rc;
+    if (int rc = phase_mark(h, e, 5)) return rc;
+    if (int rc = head_chain(h, S, e, 0, st, n)) return rc;
+    n += launch_stein_first(sa, st);
+    n += launch_update_opt(sa, S.sv, e + 1, st);
+  } else {
+    // k_finalize does not wait for the head chain: it needs neither the bandwidth nor (for correctness) the stop flag -- if
+    // the stop fires concurrently it writes one more (b, H) into the record buffer of the NEXT parity, which nobody reads
+    n += launch_finalize(ia, S.pt, peer_seq(S, e + 1), st);
+    if (int rc = phase_mark(h, e, 4)) return rc;
+    if (!S.overlap) {
+      if (int rc = do_allgather(h, e & 1)) return rc;  // NCCL fallback: whole records (x of this iteration + b, H, g)
+      if (int rc = head_chain(h, S, e, 0, st, n)) return rc;
+    }
+    if (int rc = phase_mark(h, e, 5)) return rc;
+    if (S.overlap) CU(cudaStreamWaitEvent(st, ev_join, 0));  // stop flag and bandwidth of this iteration
+    n += launch_tail(sa, ia, S.pt, peer_seq(S, e + 1), peer_seq(S, e + 1), st);
+  }
+  if (int rc = phase_mark(h, e, 6)) return rc;
+  CU(cudaGetLastError());
+  return n;
+}
+
+// Capture iteration e into the CUDA graph of its parity and return whether that graph can be replayed.  A failure (e.g. a
+// caller's stream that cannot be captured) is not an error of the scan: its error is cleared, direct launches take over.
+static bool capture_iteration(svnicp_handle h, AlignState &S, int e) {
+  const int par = e & 1;
+  cudaStream_t st = h->stream;
+  const std::string err = h->err;
+  cudaGraph_t g = nullptr;
+  int n = -1;
+  if (cudaStreamBeginCapture(st, cudaStreamCaptureModeRelaxed) == cudaSuccess) {
+    // fork from an event recorded in this capture: waiting on ev_x, recorded outside it, would invalidate the capture
+    if (cudaEventRecord(h->ev_cfork, st) == cudaSuccess) n = enqueue_iteration(h, S, e, h->ev_cfork, h->ev_chead);
+    if (cudaStreamEndCapture(st, &g) != cudaSuccess) n = -1;  // always end the capture, also after a failure inside it
+  }
+  bool ok = n >= 0 && g;
+  if (ok && h->gexec[par]) {  // same topology as the last scan's: patch the arguments in place
+    cudaGraphExecUpdateResultInfo info;
+    if (cudaGraphExecUpdate(h->gexec[par], g, &info) != cudaSuccess) {
+      cudaGraphExecDestroy(h->gexec[par]);
+      h->gexec[par] = nullptr;
+    }
+  }
+  if (ok && !h->gexec[par]) ok = cudaGraphInstantiate(&h->gexec[par], g, 0) == cudaSuccess;
+  if (g) cudaGraphDestroy(g);
+  cudaGetLastError();
+  h->err = err;
+  h->glaunches[par] = ok ? n : 0;
+  return ok;
+}
+
+// enqueue iteration S.e: replay its graph or launch it directly, then what the host follows it by (ev_x, stop flag)
 static int align_step(svnicp_handle h, AlignState &S) {
-  ALIGN_LOCALS
   const int LAG = 3;
   const int e = S.e;
-    if (h->prm.check_early_stop && e >= LAG) {
-      // deterministic host cut: the stop flag as of the END of iteration e-LAG decides (identical on every rank)
-      CU(cudaEventSynchronize(h->iter_events[e - LAG]));
-      if (h->h_stop[e - LAG]) { S.enqueue_done = true; return SVNICP_OK; }
-    }
-// SVNICP_FLAG_DEBUG_SYNC: wait for the device after every launch group and say so on stderr (localises a hang or a fault)
-#define PROF(k)                                                                                          \
-  do {                                                                                                   \
-    if (h->profile) CU(cudaEventRecord(h->prof_events[(size_t)e * 7 + (k)], st));                        \
-    if (h->prm.flags & SVNICP_FLAG_DEBUG_SYNC) {                                                         \
-      fprintf(stderr, "[svnicp] iteration %d: before phase %d ...", e, (k));                             \
-      fflush(stderr);                                                                                    \
-      const cudaError_t e1__ = cudaStreamSynchronize(st), e2__ = cudaStreamSynchronize(hs);              \
-      fprintf(stderr, " main %s, head %s\n", cudaGetErrorString(e1__), cudaGetErrorString(e2__));        \
-      fflush(stderr);                                                                                    \
-    }                                                                                                    \
-  } while (0)
-    if (S.use_graph && e >= 1) {
-      const int par = e & 1;
-      if (!S.graph_ready[par]) {
-        // ping-pong buffers of this parity (as below); clist_prev is never null here
-        ia.clist = par ? h->clist2.p : h->clist.p;
-        ia.hdr = par ? h->hdr2.p : h->hdr.p;
-        if (h->filter_reuse) {
-          ia.cbase = h->cbase[par].p; ia.ball = h->ball[par].p;
-          ia.clist_prev = par ? h->clist.p : h->clist2.p;
-          ia.cbase_prev = h->cbase[par ^ 1].p; ia.ball_prev = h->ball[par ^ 1].p;
-          ia.kept_hist = h->kept_hist.p;
-        } else {
-          ia.clist = h->clist.p; ia.hdr = h->hdr.p;
-        }
-        cudaGraph_t g = nullptr;
-        int n = 0;
-        bool ok = cudaStreamBeginCapture(st, cudaStreamCaptureModeRelaxed) == cudaSuccess;
-        if (ok) {
-          ok = cudaEventRecord(h->ev_cfork, st) == cudaSuccess && cudaStreamWaitEvent(hs, h->ev_cfork, 0) == cudaSuccess;
-          const int nh = ok ? launch_head(sa, pt, 0u, 0, hs) : -1;
-          ok = ok && nh >= 0 && cudaEventRecord(h->ev_chead, hs) == cudaSuccess;
-          if (ok) {
-            n = nh + launch_filter(ia, st) + launch_gn(ia, st) + launch_finalize(ia, pt, 0u, st);
-            ok = cudaStreamWaitEvent(st, h->ev_chead, 0) == cudaSuccess;
-            n += launch_tail(sa, ia, pt, 0u, 0u, st);
-          }
-          ok = (cudaStreamEndCapture(st, &g) == cudaSuccess) && ok && g;  // always end the capture, also after a failure inside it
-        }
-        if (ok && h->gexec[par]) {  // same topology as the last scan's: patch the arguments in place
-          cudaGraphExecUpdateResultInfo info;
-          if (cudaGraphExecUpdate(h->gexec[par], g, &info) != cudaSuccess) {
-            cudaGraphExecDestroy(h->gexec[par]);
-            h->gexec[par] = nullptr;
-          }
-        }
-        if (ok && !h->gexec[par]) ok = cudaGraphInstantiate(&h->gexec[par], g, 0) == cudaSuccess;
-        if (g) cudaGraphDestroy(g);
-        cudaGetLastError();  // a failed capture / update / instantiation is not an error of the scan (see below)
-        h->glaunches[par] = n;
-        S.graph_ready[par] = ok;
-      }
-      if (S.graph_ready[par]) {
-        CU(cudaGraphLaunch(h->gexec[par], st));
-        h->launches += h->glaunches[par];
-        if (h->prm.check_early_stop) {
-          CU(cudaMemcpyAsync(&h->h_stop[e], &h->ctrl.p->stop, sizeof(int), cudaMemcpyDeviceToHost, st));
-          CU(cudaEventRecord(h->iter_events[e], st));
-        }
-        S.e = e + 1;
-        if (S.e >= I) S.enqueue_done = true;
-        return SVNICP_OK;
-      }
-      // The graph could not be built (e.g. a caller's stream that cannot be captured): this handle keeps the direct launches
-      // of the same kernels from here on.  Nothing captured was executed; the head chain below must wait for everything
-      // enqueued so far, hence a fresh ev_x.
+  cudaStream_t st = h->stream;
+  if (h->prm.check_early_stop && e >= LAG) {
+    // deterministic host cut: the stop flag as of the END of iteration e-LAG decides (identical on every rank)
+    CU(cudaEventSynchronize(h->iter_events[e - LAG]));
+    if (h->h_stop[e - LAG]) { S.enqueue_done = true; return SVNICP_OK; }
+  }
+  bool replayed = false;
+  if (S.use_graph && e >= 1) {
+    const int par = e & 1;
+    if (!S.graph_ready[par]) S.graph_ready[par] = capture_iteration(h, S, e);
+    if (S.graph_ready[par]) {
+      CU(cudaGraphLaunch(h->gexec[par], st));
+      h->launches += h->glaunches[par];
+      replayed = true;
+    } else {
+      // The graph could not be built: this handle keeps the direct launches of the same kernels from here on.  Nothing
+      // captured was executed; the head chain below must wait for everything enqueued so far, hence a fresh ev_x.
       S.use_graph = false;
       h->graph_off = true;
       if (h->gexec[par]) { cudaGraphExecDestroy(h->gexec[par]); h->gexec[par] = nullptr; }
       CU(cudaEventRecord(h->ev_x, st));
     }
-    PROF(0);
-    if (svgd) h->launches += launch_prep(ia, st, 0, nullptr);
-    else if (overlap) {
-      CU(cudaStreamWaitEvent(hs, h->ev_x, 0));
-      const int n = launch_head(sa, pt, (h->peer_mode && e > 0) ? seq0 + (unsigned)e : 0u, 0, hs);
-      if (n < 0) return fail(h, SVNICP_ERR_CUDA, "launch of k_head failed: %s", cudaGetErrorString(cudaGetLastError()));
-      h->launches += n;
-      CU(cudaEventRecord(h->ev_head, hs));
-    }
-    PROF(1);
-    if (h->filter_reuse) {  // ping-pong: iteration e prunes the lists of iteration e-1 wherever its ball still covers this one's
-      const int cur = e & 1;
-      ia.clist = cur ? h->clist2.p : h->clist.p;
-      ia.hdr = cur ? h->hdr2.p : h->hdr.p;
-      ia.cbase = h->cbase[cur].p;
-      ia.ball = h->ball[cur].p;
-      ia.clist_prev = e > 0 ? (cur ? h->clist.p : h->clist2.p) : nullptr;
-      ia.cbase_prev = h->cbase[cur ^ 1].p;
-      ia.ball_prev = h->ball[cur ^ 1].p;
-      ia.kept_hist = h->kept_hist.p;
-    }
-    h->launches += launch_filter(ia, st);
-    PROF(2);
-    h->launches += launch_gn(ia, st);
-    if (h->prm.debug_corr) {  // parity tap: the transforms this iteration's correspondences were computed with
-      CU(h->dbg_xf.ensure((size_t)(h->P_l > 0 ? h->P_l : 1) * 12));
-      CU(cudaMemcpyAsync(h->dbg_xf.p, h->xf.p, (size_t)h->P_l * 12 * sizeof(float), cudaMemcpyDeviceToDevice, st));
-    }
-    PROF(3);
-    if (svgd) {
-      h->launches += launch_finalize_first(ia, sv, st);
-      PROF(4);
-      int rc = do_allgather(h);
-      if (rc) return rc;
-      PROF(5);
-      const int n = launch_head(sa, pt, 0u, 0, st);
-      if (n < 0) return fail(h, SVNICP_ERR_CUDA, "launch of k_head failed: %s", cudaGetErrorString(cudaGetLastError()));
-      h->launches += n;
-      h->launches += launch_stein_first(sa, st);
-      h->launches += launch_update_opt(sa, sv, e + 1, st);
-    } else {
-      // k_finalize does not wait for the head chain: it needs neither the bandwidth nor (for correctness) the stop flag -- if
-      // the stop fires concurrently it writes one more (b, H) into the record buffer of the NEXT parity, which nobody reads
-      h->launches += launch_finalize(ia, pt, seq0 + (unsigned)e + 1u, st);
-      PROF(4);
-      if (!overlap) {
-        int rc = do_allgather(h, e & 1);  // NCCL fallback: whole records (x of this iteration + b, H, g)
-        if (rc) return rc;
-        const int n = launch_head(sa, pt, 0u, 0, st);
-        if (n < 0) return fail(h, SVNICP_ERR_CUDA, "launch of k_head failed: %s", cudaGetErrorString(cudaGetLastError()));
-        h->launches += n;
-      }
-      PROF(5);
-      if (overlap) CU(cudaStreamWaitEvent(st, h->ev_head, 0));  // stop flag and bandwidth of this iteration
-      h->launches += launch_tail(sa, ia, pt, seq0 + (unsigned)e + 1u, seq0 + (unsigned)e + 1u, st);
-    }
-    PROF(6);
-#undef PROF
-    CU(cudaGetLastError());
-    // Sharded handles: the stop flag as of the END of iteration e must be copied BEFORE ev_x lets the head chain of iteration
-    // e+1 (which may set it) start on the side stream -- every rank then reads the same value, enqueues the same number of
-    // iterations and keeps the same sequence numbers.  Unsharded handles release the head chain first: one no-op iteration more
-    // or less behind the stop is harmless there, and the 4-byte copy in front of the head chain cost 10 us per iteration on
-    // small scans (3.47 -> 4.03 ms in the shipped regime).
-    const bool strict_cut = h->n_ranks > 1;
-    if (!svgd && overlap && !strict_cut) CU(cudaEventRecord(h->ev_x, st));
-    if (h->prm.check_early_stop) {
-      CU(cudaMemcpyAsync(&h->h_stop[e], &h->ctrl.p->stop, sizeof(int), cudaMemcpyDeviceToHost, st));
-      CU(cudaEventRecord(h->iter_events[e], st));
-    }
-    if (!svgd && overlap && strict_cut) CU(cudaEventRecord(h->ev_x, st));
-    S.e = e + 1;
-  if (S.e >= I) S.enqueue_done = true;
+  }
+  if (!replayed) {
+    const int n = enqueue_iteration(h, S, e, h->ev_x, h->ev_head);
+    if (n < 0) return n;
+    h->launches += n;
+  }
+  // Sharded handles: the stop flag as of the END of iteration e must be copied BEFORE ev_x lets the head chain of iteration
+  // e+1 (which may set it) start on the side stream -- every rank then reads the same value, enqueues the same number of
+  // iterations and keeps the same sequence numbers.  Unsharded handles release the head chain first: one no-op iteration more
+  // or less behind the stop is harmless there, and the 4-byte copy in front of the head chain cost 10 us per iteration on
+  // small scans (3.47 -> 4.03 ms in the shipped regime).  A replayed iteration records no ev_x: nothing that follows waits on it.
+  const bool release_head = S.overlap && !replayed, strict_cut = h->n_ranks > 1;
+  if (release_head && !strict_cut) CU(cudaEventRecord(h->ev_x, st));
+  if (h->prm.check_early_stop) {
+    CU(cudaMemcpyAsync(&h->h_stop[e], &h->ctrl.p->stop, sizeof(int), cudaMemcpyDeviceToHost, st));
+    CU(cudaEventRecord(h->iter_events[e], st));
+  }
+  if (release_head && strict_cut) CU(cudaEventRecord(h->ev_x, st));
+  S.e = e + 1;
+  if (S.e >= S.I) S.enqueue_done = true;
   return SVNICP_OK;
 }
 
 static int align_epilogue(svnicp_handle h, AlignState &S) {
-  ALIGN_LOCALS
+  cudaStream_t st = h->stream;
   const int e = S.e;
   h->enqueued_iters = e;
-  h->seq = seq0 + (unsigned)e + 1u;
+  h->seq = S.seq0 + (unsigned)e + 1u;
   CU(cudaEventRecord(h->ev[2], st));
   // ---- epilogue: last stop decision / history row, getters (SVNICP.cpp:111, :281-308) ----
-  if (svgd) {
-    h->launches += launch_svgd_rec(h->rec, h->pose6.p, h->dnorm.p, h->p_lo, h->P_l, h->p_lo, st);
-    int rc = do_allgather(h);
-    if (rc) return rc;
-    const int n = launch_head(sa, pt, 0u, 1, st);
-    if (n < 0) return fail(h, SVNICP_ERR_CUDA, "launch of k_head failed: %s", cudaGetErrorString(cudaGetLastError()));
-    h->launches += n + launch_stats_svgd(sa, h->prev.p, st);
-  } else {
-    // the final x of every particle already sits in the record buffer of parity (updates applied & 1) on every rank
-    if (!overlap && h->n_ranks > 1)
-      for (int b2 = 0; b2 < 2; b2++) {  // NCCL fallback: the device knows which buffer is final (early stop), so gather both
-        int rc = do_allgather(h, b2);
-        if (rc) return rc;
-      }
-    const int n = launch_head(sa, pt, (h->peer_mode && e > 0) ? seq0 + (unsigned)e : 0u, 1, st);
-    if (n < 0) return fail(h, SVNICP_ERR_CUDA, "launch of k_head failed: %s", cudaGetErrorString(cudaGetLastError()));
-    h->launches += n + launch_stats(sa, 1, st);
+  int n = 0;
+  if (S.svgd) {
+    n += launch_svgd_rec(h->rec, h->pose6.p, h->dnorm.p, h->p_lo, h->P_l, h->p_lo, st);
+    if (int rc = do_allgather(h)) return rc;
+  } else if (!S.overlap && h->n_ranks > 1) {
+    // the final x of every particle already sits in the record buffer of parity (updates applied & 1) on every rank; NCCL
+    // fallback: the device knows which buffer is final (early stop), so gather both
+    for (int b2 = 0; b2 < 2; b2++)
+      if (int rc = do_allgather(h, b2)) return rc;
   }
+  if (int rc = head_chain(h, S, e, 1, st, n)) return rc;
+  n += S.svgd ? launch_stats_svgd(S.sa, h->prev.p, st) : launch_stats(S.sa, 1, st);
+  h->launches += n;
   CU(cudaGetLastError());
   CU(cudaMemcpyAsync(h->h_stats, h->stats.p, 48 * sizeof(double), cudaMemcpyDeviceToHost, st));
   CU(cudaMemcpyAsync(h->h_particles, h->particles.p, (size_t)6 * h->P * sizeof(double), cudaMemcpyDeviceToHost, st));
   CU(cudaMemcpyAsync(h->h_ctrl, h->ctrl.p, sizeof(Ctrl), cudaMemcpyDeviceToHost, st));
-  CU(cudaMemcpyAsync(h->h_kept, h->kept_hist.p, ((size_t)I + 2) * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+  CU(cudaMemcpyAsync(h->h_kept, h->kept_hist.p, ((size_t)S.I + 2) * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
   CU(cudaEventRecord(h->ev[3], st));
   return SVNICP_OK;
 }
 
 static int align_finish(svnicp_handle h, AlignState &S) {
-  ALIGN_LOCALS
+  cudaStream_t st = h->stream, hs = h->head_stream;
   if (h->prm.flags & SVNICP_FLAG_WATCHDOG) {  // diagnostic watchdog: poll instead of blocking, report which stream is stuck and the device-side state
     const double t0 = (double)clock() / CLOCKS_PER_SEC;
     bool done = false;

@@ -9,9 +9,11 @@ from svn_icp_b200 import synth
 pytestmark = pytest.mark.gpu
 
 
-@pytest.mark.parametrize("full,es", [(True, False), (False, True)])
-def test_batched_streams_equal_single_handles(full, es):
-    S, P, I = 5, 96, 9
+# 20 iterations without early stop: every stream captures and replays its CUDA graphs while the scans are interleaved
+@pytest.mark.parametrize("full,es,I", [(True, False, 9), (False, True, 9), (True, False, 20)],
+                         ids=["True-False", "False-True", "True-False-20"])
+def test_batched_streams_equal_single_handles(full, es, I):
+    S, P = 5, 96
     rng = np.random.default_rng(11)
     pbs = [synth.make_problem(P, sensor="32", scan_index=5 + (s % 2), n_map_scans=5, seed=0xC0FFEE + (s % 2)) for s in range(2)]
     inits = np.stack([synth.init_particles(P, rng) for _ in range(S)])
