@@ -265,6 +265,27 @@ int svnicp_map_size(svnicp_map m, int64_t *voxels, int64_t *points);
 int svnicp_map_evaluate(svnicp_map m, const void *source, int64_t n, int dtype_f64, int on_device, const double R0[9],
                         const double t0[3], int n_poses, const double *poses_6xM, double max_dist, double *out_stats,
                         double *out_H, double *out_b, uint8_t *out_mask, float *out_nearest);
+/* Snapshot of the map's content (no reference counterpart), to save a map and restore it bit for bit with svnicp_map_import:
+ *   voxels [V][3] int32  voxel indices (vx, vy, vz) in ascending lexicographic order
+ *   counts [V]    int32  points per voxel, 1 <= count <= max_pointscount
+ *   xyz [Npts][3] float  each voxel's points one after another, in the voxel order, and inside a voxel in stored order
+ *                        (arrival order: the first point is the one GetMap(pose, r) and RemoveFarPointCloud test)
+ * n_voxels / n_points must equal svnicp_map_size (V, Npts).  The snapshot depends on the content only, not on the slot layout,
+ * the table capacity or the map's history: two maps that hold the same content give the same bytes.  Outputs are host memory,
+ * or device memory on the map's GPU with on_device = 1.  Blocking, on the map's stream.  Changes no state of the map (the table,
+ * Size(), the last svnicp_map_get result and its device pointer stay valid). */
+int svnicp_map_export(svnicp_map m, int32_t *voxels, int32_t *counts, float *xyz, int64_t n_voxels, int64_t n_points, int on_device);
+/* Replace the map's content by a snapshot in the layout of svnicp_map_export (any earlier content is discarded; no transform, no
+ * RemoveFarPointCloud).  The voxels may come in any order; each voxel's points are stored in the order given.  Inputs are host
+ * memory, or device memory on the map's GPU with on_device = 1.  Blocking.  All or nothing: on any error the map is exactly as
+ * before.  SVNICP_ERR_INVALID for null pointers with a size > 0, negative sizes, n_points != sum of counts, and -- naming the
+ * lowest offending voxel index in svnicp_map_last_error -- a count outside [1, max_pointscount], a voxel index outside
+ * [-2^20, 2^20), a duplicate voxel (the later one is named), or a point that does not belong to its voxel: (int)(p /
+ * float(voxel_size)) per axis, the arithmetic of AddPointCloud, so anything the map can hold round-trips (NaN points sit in
+ * voxel 0).  SVNICP_ERR_OOM when n_voxels exceeds the table (2x capacity_voxels slots hold at least capacity_voxels voxels).
+ * n_voxels = 0 has the effect of svnicp_map_clear. */
+int svnicp_map_import(svnicp_map m, const int32_t *voxels, const int32_t *counts, const float *xyz, int64_t n_voxels, int64_t n_points,
+                      int on_device);
 
 /* ---------------------------------------------------------------------------------------------
  * Scan pre-processing on the device, the step right before add_cloud in the reference's node

@@ -91,7 +91,7 @@ EXPORTS = [
     "svnicp_get_timing", "svnicp_get_slice", "svnicp_get_launch_count", "svnicp_set_profiling", "svnicp_get_phase_times",
     "svnicp_get_scan_info", "svnicp_get_tail_stamps", "svnicp_evaluate",
     "svnicp_map_create", "svnicp_map_destroy", "svnicp_map_last_error", "svnicp_map_clear", "svnicp_map_add_cloud", "svnicp_map_get",
-    "svnicp_map_download", "svnicp_map_size", "svnicp_map_evaluate",
+    "svnicp_map_download", "svnicp_map_size", "svnicp_map_evaluate", "svnicp_map_export", "svnicp_map_import",
     "svnicp_pre_create", "svnicp_pre_destroy", "svnicp_pre_last_error", "svnicp_pre_crop", "svnicp_pre_downsample_uniform",
     "svnicp_pre_to_f64", "svnicp_pre_download", "svnicp_pre_deskew", "svnicp_pose_compose",
     "svnicp_batch_create", "svnicp_batch_destroy", "svnicp_batch_last_error", "svnicp_batch_size", "svnicp_batch_stream", "svnicp_batch_align",
@@ -152,7 +152,8 @@ def _ARGTYPES(V, I, L, D):
         "svnicp_evaluate": [V, I, V, V, V, V, V, V],
         "svnicp_map_create": [V, D, D, I, L, I], "svnicp_map_clear": [V], "svnicp_map_add_cloud": [V, V, L, I, I, V, V],
         "svnicp_map_get": [V, V, D, V, V], "svnicp_map_download": [V, V, L], "svnicp_map_size": [V, V, V],
-        "svnicp_map_evaluate": [V, V, L, I, I, V, V, I, V, D, V, V, V, V, V],
+        "svnicp_map_evaluate": [V, V, L, I, I, V, V, I, V, D, V, V, V, V, V], "svnicp_map_export": [V, V, V, V, L, L, I],
+        "svnicp_map_import": [V, V, V, V, L, L, I],
         "svnicp_pre_create": [V, L, I], "svnicp_pre_crop": [V, V, L, I, D, D, V, V, V],
         "svnicp_pre_downsample_uniform": [V, V, L, I, D, V, V], "svnicp_pre_to_f64": [V, V, L, V], "svnicp_pre_download": [V, V, L, V],
         "svnicp_pre_deskew": [V, V, L, I, V, I, I, V, V, V, V, V, V], "svnicp_pose_compose": [V, V, V, V, V],
@@ -516,6 +517,61 @@ class SVNICPBatch:
             pass
 
 
+MAP_SNAPSHOT_MAGIC = b"SVNMAP01"
+MAP_SNAPSHOT_VERSION = 1
+_SNAP_HEADER = np.dtype([("magic", "S8"), ("version", "<u4"), ("max_pointscount", "<u4"), ("voxel_size", "<f8"), ("max_range", "<f8"),
+                         ("n_voxels", "<i8"), ("n_points", "<i8")])  # 48 bytes, then voxels, counts and xyz, raw
+
+
+@dataclasses.dataclass
+class MapSnapshot:
+    """A local map's content in canonical form (svnicp_map_export): voxels [V, 3] int32 in ascending (vx, vy, vz), counts [V]
+    int32, points [sum(counts), 3] float32 (each voxel's points in stored order, the voxels in order), and the map parameters."""
+    voxel_size: float
+    max_range: float
+    max_pointscount: int
+    voxels: np.ndarray
+    counts: np.ndarray
+    points: np.ndarray
+
+
+def write_map_snapshot(path: str, snap: MapSnapshot) -> None:
+    """The snapshot file shared with the C++ mirror (svnicp::write_map_snapshot): little-endian header `SVNMAP01`, u32 version 1,
+    u32 max_pointscount, f64 voxel_size, f64 max_range, i64 V, i64 Npts; then voxels int32 [V][3], counts int32 [V], xyz float32
+    [Npts][3]."""
+    vox = np.ascontiguousarray(snap.voxels, dtype="<i4").reshape(-1, 3)
+    cnt = np.ascontiguousarray(snap.counts, dtype="<i4").reshape(-1)
+    pts = np.ascontiguousarray(snap.points, dtype="<f4").reshape(-1, 3)
+    if len(cnt) != len(vox):
+        raise SvnIcpError("write_map_snapshot: voxels and counts differ in length")
+    h = np.array([(MAP_SNAPSHOT_MAGIC, MAP_SNAPSHOT_VERSION, snap.max_pointscount, snap.voxel_size, snap.max_range, len(vox), len(pts))],
+                 dtype=_SNAP_HEADER)
+    with open(path, "wb") as f:
+        for a in (h, vox, cnt, pts):
+            f.write(a.tobytes())
+
+
+def read_map_snapshot(path: str) -> MapSnapshot:
+    """Read a snapshot file; rejects a wrong magic or version and a length that does not match the sizes."""
+    with open(path, "rb") as f:
+        data = f.read()
+    if len(data) < _SNAP_HEADER.itemsize:
+        raise SvnIcpError(f"{path}: not a map snapshot (shorter than its header)")
+    h = np.frombuffer(data, dtype=_SNAP_HEADER, count=1)[0]
+    if h["magic"] != MAP_SNAPSHOT_MAGIC:
+        raise SvnIcpError(f"{path}: not a map snapshot (magic)")
+    if h["version"] != MAP_SNAPSHOT_VERSION:
+        raise SvnIcpError(f"{path}: map snapshot version {h['version']}, this reader knows {MAP_SNAPSHOT_VERSION}")
+    V, N = int(h["n_voxels"]), int(h["n_points"])
+    if V < 0 or N < 0 or len(data) != _SNAP_HEADER.itemsize + 16 * V + 12 * N:
+        raise SvnIcpError(f"{path}: map snapshot length {len(data)} does not match V = {V}, Npts = {N}")
+    o = _SNAP_HEADER.itemsize
+    vox = np.frombuffer(data, dtype="<i4", count=3 * V, offset=o).reshape(V, 3).astype(np.int32)
+    cnt = np.frombuffer(data, dtype="<i4", count=V, offset=o + 12 * V).astype(np.int32)
+    pts = np.frombuffer(data, dtype="<f4", count=3 * N, offset=o + 16 * V).reshape(N, 3).astype(np.float32)
+    return MapSnapshot(float(h["voxel_size"]), float(h["max_range"]), int(h["max_pointscount"]), vox, cnt, pts)
+
+
 class VoxelHashMap:
     """Drop-in for svnicp::VoxelHashMap (VoxelHashMap.h:28-72, VoxelHashMap.cpp:22-101), device resident: the local map the
     node keeps between scans (OdometryPipeline.cpp:577-581, :630).  Same method names; poses are (R [3,3], t [3])."""
@@ -628,6 +684,51 @@ class VoxelHashMap:
             if v is not None:
                 out[k] = v
         return {k: v[0] for k, v in out.items()} if single else out
+
+    # -- snapshots (svnicp_map_export / svnicp_map_import; no reference counterpart) --------------
+    def Export(self) -> MapSnapshot:
+        """The map's content in canonical form: the same bytes for the same content, whatever the slot layout or history."""
+        V, N = self.Size(), self.PointCount()
+        vox, cnt, pts = np.zeros((V, 3), dtype=np.int32), np.zeros(V, dtype=np.int32), np.zeros((N, 3), dtype=np.float32)
+        self._check(self._lib.svnicp_map_export(self._m, _p(vox), _p(cnt), _p(pts), C.c_int64(V), C.c_int64(N), C.c_int(0)), "Export")
+        return MapSnapshot(self.voxel_size_, self.max_range_, self.max_pointscount_, vox, cnt, pts)
+
+    def ExportDevice(self, voxels_ptr: int, counts_ptr: int, xyz_ptr: int):
+        """Export into device memory on the map's GPU: int32 [Size(), 3], int32 [Size()], float32 [PointCount(), 3]."""
+        self._check(self._lib.svnicp_map_export(self._m, C.c_void_p(voxels_ptr), C.c_void_p(counts_ptr), C.c_void_p(xyz_ptr),
+                                                C.c_int64(self.Size()), C.c_int64(self.PointCount()), C.c_int(1)), "Export")
+
+    def Import(self, snapshot: MapSnapshot):
+        """Replace the content by a snapshot (no transform, no RemoveFarPointCloud).  The snapshot's voxel_size, max_range and
+        max_pointscount must be the map's.  All or nothing: on an error the map is unchanged."""
+        mine = (self.voxel_size_, self.max_range_, self.max_pointscount_)
+        theirs = (snapshot.voxel_size, snapshot.max_range, snapshot.max_pointscount)
+        if tuple(map(float, mine)) != tuple(map(float, theirs)):
+            raise SvnIcpError(f"Import: snapshot of a map with (voxel_size, max_range, max_pointscount) = {theirs}, this map has {mine}")
+        vox = np.ascontiguousarray(snapshot.voxels, dtype=np.int32).reshape(-1, 3)
+        cnt = np.ascontiguousarray(snapshot.counts, dtype=np.int32).reshape(-1)
+        pts = np.ascontiguousarray(snapshot.points, dtype=np.float32).reshape(-1, 3)
+        if len(cnt) != len(vox):
+            raise SvnIcpError("Import: voxels and counts differ in length")
+        self._check(self._lib.svnicp_map_import(self._m, _p(vox), _p(cnt), _p(pts), C.c_int64(len(vox)), C.c_int64(len(pts)), C.c_int(0)),
+                    "Import")
+
+    def ImportDevice(self, voxels_ptr: int, counts_ptr: int, xyz_ptr: int, n_voxels: int, n_points: int):
+        """Import from device memory on the map's GPU (layout of ExportDevice).  Only the ABI's checks apply: counts and membership."""
+        self._check(self._lib.svnicp_map_import(self._m, C.c_void_p(voxels_ptr), C.c_void_p(counts_ptr), C.c_void_p(xyz_ptr),
+                                                C.c_int64(n_voxels), C.c_int64(n_points), C.c_int(1)), "Import")
+
+    def Save(self, path: str):
+        write_map_snapshot(path, self.Export())
+
+    @classmethod
+    def Load(cls, path: str, capacity_voxels: int | None = None, device: int = -1) -> "VoxelHashMap":
+        """A new map with the file's parameters, a capacity of at least its voxel count, and its content."""
+        snap = read_map_snapshot(path)
+        cap = max(capacity_voxels if capacity_voxels is not None else 1 << 19, len(snap.counts), 1)
+        m = cls(snap.voxel_size, snap.max_range, snap.max_pointscount, capacity_voxels=cap, device=device)
+        m.Import(snap)
+        return m
 
 
 class ScanPreprocessor:

@@ -17,6 +17,10 @@
 // svnicp_map_evaluate (DESIGN.md section 10b) scores a scan at caller-given poses against the table itself: an exact
 // nearest-map-point search per (source point, pose) by read-only probes of the same hash (k_map_eval), then the fixed-order
 // reduction of svnicp_evaluate (k_eval_fin, eval_kernels.cu).
+//
+// svnicp_map_export / svnicp_map_import (DESIGN.md section 10c) save and restore the content in canonical form -- voxels in
+// ascending (vx, vy, vz), each voxel's points in stored order -- independent of the slot layout: a radix sort of the live keys
+// on the way out, a rebuild into the twin table with full validation on the way in.
 #include <cuda_runtime.h>
 #include <limits.h>
 #include <math.h>
@@ -61,6 +65,13 @@ __device__ __forceinline__ unsigned hash_key(unsigned long long k) {
   return (unsigned)k;
 }
 
+// The voxel a stored point belongs to (VoxelHashMap.cpp:30): (int)(p / float(voxel_size)) per axis -- truncation toward zero,
+// so (-v, v) is voxel 0, and NaN converts to 0 -- packed.  k_map_insert_link files points with it and svnicp_map_import checks
+// membership with it, so the two cannot drift.
+__device__ __forceinline__ unsigned long long voxel_key(const float q[3], float voxel_size_f) {
+  return pack_key((int)(q[0] / voxel_size_f), (int)(q[1] / voxel_size_f), (int)(q[2] / voxel_size_f));
+}
+
 // find-or-create; returns the slot or -1 when the table is full
 __device__ int find_or_create(const MapDev &m, unsigned long long key, bool *created) {
   unsigned slot = hash_key(key) & (unsigned)m.slots_mask;
@@ -89,9 +100,8 @@ __global__ void k_map_insert_link(MapDev m, const T *xyz, int n, const double *R
   for (int r = 0; r < 3; r++) q[r] = (float)(Rt[3 * r] * p[0] + Rt[3 * r + 1] * p[1] + Rt[3 * r + 2] * p[2] + Rt[9 + r]);
 #pragma unroll
   for (int r = 0; r < 3; r++) wxyz[3 * (size_t)i + r] = q[r];
-  const int vx = (int)(q[0] / m.voxel_size_f), vy = (int)(q[1] / m.voxel_size_f), vz = (int)(q[2] / m.voxel_size_f);
   bool created;
-  const int slot = find_or_create(m, pack_key(vx, vy, vz), &created);
+  const int slot = find_or_create(m, voxel_key(q, m.voxel_size_f), &created);
   pt_slot[i] = slot;
   if (slot < 0) { atomicAdd((unsigned long long *)&m.counters[3], 1ull); return; }
   if (created) atomicAdd((unsigned long long *)&m.counters[0], 1ull);
@@ -193,41 +203,43 @@ __global__ void __launch_bounds__(SCAN_BLOCK) k_getmap_count(MapDev m, const dou
   }
 }
 
-__device__ int block_exclusive_scan(int v, int *total) {  // SCAN_BLOCK threads
-  __shared__ int s_w[32];
-  __shared__ int s_tot;
+template <typename T>
+__device__ T block_exclusive_scan(T v, T *total) {  // SCAN_BLOCK threads; int, or long long for point offsets
+  __shared__ T s_w[32];
+  __shared__ T s_tot;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  int incl = v;
+  T incl = v;
   for (int o = 1; o < 32; o <<= 1) {
-    const int u = __shfl_up_sync(0xffffffffu, incl, o);
+    const T u = __shfl_up_sync(0xffffffffu, incl, o);
     if (lane >= o) incl += u;
   }
   if (lane == 31) s_w[warp] = incl;
   __syncthreads();
   if (warp == 0) {
-    int x = s_w[lane], xi = x;
+    T x = s_w[lane], xi = x;
     for (int o = 1; o < 32; o <<= 1) {
-      const int u = __shfl_up_sync(0xffffffffu, xi, o);
+      const T u = __shfl_up_sync(0xffffffffu, xi, o);
       if (lane >= o) xi += u;
     }
     s_w[lane] = xi - x;
     if (lane == 31) s_tot = xi;
   }
   __syncthreads();
-  const int r = s_w[warp] + incl - v;
+  const T r = s_w[warp] + incl - v;
   if (total) *total = s_tot;
   __syncthreads();
   return r;
 }
 
-__global__ void __launch_bounds__(SCAN_BLOCK) k_getmap_scan(int *block_sums, int n_blocks, long long *total_out) {
-  // one block; n_blocks <= SCAN_BLOCK * 8
-  int carry = 0;
+template <typename T>
+__global__ void __launch_bounds__(SCAN_BLOCK) k_getmap_scan(T *block_sums, int n_blocks, long long *total_out) {
+  // one block, looping over the sums SCAN_BLOCK at a time (GetMap: n_blocks <= SCAN_BLOCK * 8)
+  T carry = 0;
   for (int base = 0; base < n_blocks; base += SCAN_BLOCK) {
     const int i = base + threadIdx.x;
-    const int v = i < n_blocks ? block_sums[i] : 0;
-    int tot;
-    const int ex = block_exclusive_scan(v, &tot);
+    const T v = i < n_blocks ? block_sums[i] : 0;
+    T tot;
+    const T ex = block_exclusive_scan(v, &tot);
     if (i < n_blocks) block_sums[i] = carry + ex;
     carry += tot;
   }
@@ -237,7 +249,7 @@ __global__ void __launch_bounds__(SCAN_BLOCK) k_getmap_scan(int *block_sums, int
 __global__ void __launch_bounds__(SCAN_BLOCK) k_getmap_emit(MapDev m, const double *pos, double r2, int all, const int *block_offs, double *out) {
   const int s = blockIdx.x * SCAN_BLOCK + threadIdx.x;
   const int c = slot_emit_count(m, s, pos, r2, all);
-  const int off = block_offs[blockIdx.x] + block_exclusive_scan(c, nullptr);
+  const int off = block_offs[blockIdx.x] + block_exclusive_scan<int>(c, nullptr);
   if (c == 0) return;
   const float *src = m.tab.pts + (size_t)s * m.cap * 3;
   double *dst = out + (size_t)off * 3;
@@ -247,6 +259,206 @@ __global__ void __launch_bounds__(SCAN_BLOCK) k_getmap_emit(MapDev m, const doub
 __global__ void k_fill_i32(int *p, int v, size_t n) {
   const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) p[i] = v;
+}
+
+// ---- svnicp_map_export / svnicp_map_import (DESIGN.md section 10c) ----------------------------------------------------------
+// Export: live slots -> (canonical key, slot) pairs (count -> single-block scan -> emit, as GetMap) -> stable LSD radix sort
+// by canonical key -> int64 point offsets in that order -> one warp per voxel gathers index, count and points.
+// Import: int64 point offsets of the snapshot -> one warp per voxel builds into the twin table and checks it -> duplicates.
+constexpr int RADIX_BITS = 8;
+constexpr int RADIX_DIGITS = 1 << RADIX_BITS;
+constexpr int RADIX_THREADS = 256;  // == RADIX_DIGITS: one thread per digit in the histogram and offset steps
+constexpr int RADIX_IPT = 16;       // keys per thread
+constexpr int RADIX_TILE = RADIX_THREADS * RADIX_IPT;
+constexpr int CANON_BITS = 63;      // three 21-bit fields
+static_assert(((CANON_BITS + RADIX_BITS - 1) / RADIX_BITS) % 2 == 0, "an even pass count leaves the sorted pairs in buffer 0");
+constexpr unsigned long long SNAP_NO_ERROR = ~0ull;
+enum { SNAP_BAD_COUNT = 1, SNAP_BAD_INDEX = 2, SNAP_DUPLICATE = 3, SNAP_NOT_MEMBER = 4 };  // the reason in the low 3 bits
+
+// The packed key with the x and z fields swapped: each field holds index + 2^20, so ascending canonical keys are ascending
+// lexicographic (vx, vy, vz).  The swap is its own inverse.
+__device__ __forceinline__ unsigned long long canon_key(unsigned long long k) {
+  const unsigned long long F = 0x1FFFFFull;
+  return ((k & F) << 42) | (k & (F << 21)) | ((k >> 42) & F);
+}
+
+__device__ __forceinline__ bool slot_live(const MapDev &m, int s) {
+  return s <= m.slots_mask && m.tab.keys[s] != EMPTY_KEY && m.tab.count[s] > 0;
+}
+
+__global__ void __launch_bounds__(SCAN_BLOCK) k_snap_count(MapDev m, int *block_sums) {
+  const int c = __syncthreads_count(slot_live(m, blockIdx.x * SCAN_BLOCK + threadIdx.x));
+  if (threadIdx.x == 0) block_sums[blockIdx.x] = c;
+}
+
+// (canonical key, slot) of every live slot, in slot order; at most V are written
+__global__ void __launch_bounds__(SCAN_BLOCK) k_snap_emit(MapDev m, const int *block_offs, long long V, unsigned long long *keys, int *slots) {
+  const int s = blockIdx.x * SCAN_BLOCK + threadIdx.x;
+  const int live = slot_live(m, s) ? 1 : 0;
+  const int off = block_offs[blockIdx.x] + block_exclusive_scan<int>(live, nullptr);
+  if (!live || off >= V) return;
+  keys[off] = canon_key(m.tab.keys[s]);
+  slots[off] = s;
+}
+
+// Radix pass, step 1: digit histogram of each tile of RADIX_TILE keys, digit-major ([digit][tile]) so that one exclusive scan
+// gives every (digit, tile) its output offset.
+__global__ void __launch_bounds__(RADIX_THREADS) k_radix_hist(const unsigned long long *keys, int n, int shift, int n_tiles, int *hist) {
+  __shared__ int s_h[RADIX_DIGITS];
+  s_h[threadIdx.x] = 0;
+  __syncthreads();
+  const int base = blockIdx.x * RADIX_TILE;
+  for (int k = threadIdx.x; k < RADIX_TILE && base + k < n; k += RADIX_THREADS)
+    atomicAdd(&s_h[(keys[base + k] >> shift) & (RADIX_DIGITS - 1)], 1);
+  __syncthreads();
+  hist[(size_t)threadIdx.x * n_tiles + blockIdx.x] = s_h[threadIdx.x];
+}
+
+// Radix pass, step 3: stable scatter.  Warp w of a tile owns keys [w * 32 * IPT, (w + 1) * 32 * IPT) of it, 32 consecutive keys
+// per round; a key's rank among the equal digits before it comes from __match_any_sync within the round plus the warp's running
+// per-digit count, and the lower warps' counts are added once the tile is counted.
+__global__ void __launch_bounds__(RADIX_THREADS) k_radix_scatter(const unsigned long long *keys_in, const int *vals_in, unsigned long long *keys_out,
+                                                                int *vals_out, int n, int shift, int n_tiles, const int *offs) {
+  __shared__ int s_cnt[RADIX_THREADS / 32][RADIX_DIGITS];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  for (int d = lane; d < RADIX_DIGITS; d += 32) s_cnt[warp][d] = 0;
+  __syncwarp();
+  const int base = blockIdx.x * RADIX_TILE + warp * 32 * RADIX_IPT + lane;
+  const unsigned below = (1u << lane) - 1u;
+  int dig[RADIX_IPT], rank[RADIX_IPT];
+#pragma unroll
+  for (int r = 0; r < RADIX_IPT; r++) {
+    const int i = base + 32 * r;
+    const int d = i < n ? (int)((keys_in[i] >> shift) & (RADIX_DIGITS - 1)) : RADIX_DIGITS;  // RADIX_DIGITS: no key
+    const unsigned peers = __match_any_sync(0xffffffffu, d);
+    rank[r] = s_cnt[warp][d & (RADIX_DIGITS - 1)] + __popc(peers & below);
+    __syncwarp();
+    if (d < RADIX_DIGITS && (peers & below) == 0) s_cnt[warp][d] += __popc(peers);
+    __syncwarp();
+    dig[r] = d;
+  }
+  __syncthreads();
+  {
+    const int d = threadIdx.x;
+    int run = offs[(size_t)d * n_tiles + blockIdx.x];
+    for (int w = 0; w < RADIX_THREADS / 32; w++) {
+      const int c = s_cnt[w][d];
+      s_cnt[w][d] = run;
+      run += c;
+    }
+  }
+  __syncthreads();
+#pragma unroll
+  for (int r = 0; r < RADIX_IPT; r++) {
+    if (dig[r] == RADIX_DIGITS) continue;
+    const int i = base + 32 * r, dst = s_cnt[warp][dig[r]] + rank[r];
+    keys_out[dst] = keys_in[i];
+    vals_out[dst] = vals_in[i];
+  }
+}
+
+// Point count of voxel i: the table's through the sorted slots (export), or the snapshot's, taken as 0 outside [1, cap] so that
+// the offsets stay in bounds (import; k_map_import reports such a count).
+__device__ __forceinline__ int snap_count(const int32_t *counts, const int *slots, const int *tab_count, int cap, long long i, long long V) {
+  if (i >= V) return 0;
+  if (slots) return tab_count[slots[i]];
+  const int c = counts[i];
+  return c >= 1 && c <= cap ? c : 0;
+}
+
+__global__ void __launch_bounds__(SCAN_BLOCK) k_snap_pts_count(const int32_t *counts, const int *slots, const int *tab_count, int cap, long long V,
+                                                             long long *block_sums) {
+  const long long c = snap_count(counts, slots, tab_count, cap, (long long)blockIdx.x * SCAN_BLOCK + threadIdx.x, V);
+  long long tot;
+  block_exclusive_scan<long long>(c, &tot);
+  if (threadIdx.x == 0) block_sums[blockIdx.x] = tot;
+}
+
+__global__ void __launch_bounds__(SCAN_BLOCK) k_snap_pts_offsets(const int32_t *counts, const int *slots, const int *tab_count, int cap, long long V,
+                                                               const long long *block_offs, long long *off) {
+  const long long i = (long long)blockIdx.x * SCAN_BLOCK + threadIdx.x;
+  const long long c = snap_count(counts, slots, tab_count, cap, i, V);
+  const long long o = block_offs[blockIdx.x] + block_exclusive_scan<long long>(c, nullptr);
+  if (i < V) off[i] = o;
+}
+
+// one warp per sorted voxel: index, count, and the points in stored order (the coalesced copy of k_map_rebuild)
+__global__ void k_snap_gather(MapTable t, int cap, const unsigned long long *keys, const int *slots, const long long *off, long long V, long long N,
+                              int32_t *voxels, int32_t *counts, float *xyz) {
+  const long long i = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (i >= V) return;
+  const int s = slots[i], c = t.count[s];
+  if (lane < 3) voxels[3 * i + lane] = (int)((keys[i] >> (42 - 21 * lane)) & 0x1FFFFFull) - (1 << 20);
+  if (lane == 3) counts[i] = c;
+  const long long o = off[i];
+  if (o + c > N) return;  // the table disagrees with the counters: reported by the caller, nothing written out of bounds
+  const float *src = t.pts + (size_t)s * cap * 3;
+  float *dst = xyz + o * 3;
+  for (int e = lane; e < 3 * c; e += 32) dst[e] = src[e];
+}
+
+__device__ __forceinline__ void snap_flag(unsigned long long *err, long long i, int reason) {
+  atomicMin(err, ((unsigned long long)i << 3) | (unsigned long long)reason);
+}
+
+// One warp per snapshot voxel into the (cleared) twin table: find_or_create, count, points; every point's membership is
+// checked with voxel_key.  words: [0] lowest (voxel << 3 | reason) of the count and index errors, [2] voxels refused by a full
+// table, [3] lowest of the duplicate and membership errors (meaningful only when the counts are valid and sum to N, since the
+// point offsets come from them).  Each voxel's slot goes to slot_of (-1 when not inserted) and the lowest voxel index per slot
+// to walker, for k_map_import_dups.
+__global__ void k_map_import(MapDev neu, const int32_t *voxels, const int32_t *counts, const float *xyz, long long V, long long N,
+                             const long long *off, int *slot_of, unsigned long long *words) {
+  const long long i = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (i >= V) return;
+  const int vx = voxels[3 * i], vy = voxels[3 * i + 1], vz = voxels[3 * i + 2], c = counts[i];
+  const int lim = 1 << 20;
+  const bool count_ok = c >= 1 && c <= neu.cap;
+  const bool index_ok = vx >= -lim && vx < lim && vy >= -lim && vy < lim && vz >= -lim && vz < lim;
+  const unsigned long long key = pack_key(vx, vy, vz);
+  int slot = -1;
+  if (lane == 0) {
+    if (!count_ok) snap_flag(words, i, SNAP_BAD_COUNT);
+    else if (!index_ok) snap_flag(words, i, SNAP_BAD_INDEX);
+    else {
+      bool created;
+      slot = find_or_create(neu, key, &created);
+      if (slot < 0) atomicAdd(&words[2], 1ull);
+      else {
+        atomicMin(&neu.walker[slot], (int)i);
+        neu.tab.count[slot] = c;
+      }
+    }
+    slot_of[i] = slot;
+  }
+  slot = __shfl_sync(0xffffffffu, slot, 0);
+  if (!count_ok || !index_ok) return;
+  const long long o = off[i];
+  if (o + c > N) return;  // the counts sum past n_points: reported from the sum
+  const float *src = xyz + o * 3;
+  for (int k = lane; k < c; k += 32) {
+    const float q[3] = {src[3 * k], src[3 * k + 1], src[3 * k + 2]};
+    if (voxel_key(q, neu.voxel_size_f) != key) snap_flag(words + 3, i, SNAP_NOT_MEMBER);
+  }
+  if (slot < 0) return;
+  float *dst = neu.tab.pts + (size_t)slot * neu.cap * 3;
+  for (int e = lane; e < 3 * c; e += 32) dst[e] = src[e];
+}
+
+// A voxel whose slot was claimed by a lower index repeats that voxel; the lowest index of each slot is not a duplicate.
+__global__ void k_map_import_dups(const int *walker, const int *slot_of, long long V, unsigned long long *words) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= V) return;
+  const int s = slot_of[i];
+  if (s >= 0 && walker[s] != (int)i) snap_flag(words + 3, i, SNAP_DUPLICATE);
+}
+
+__global__ void k_map_import_reset(int *walker, const int *slot_of, long long V) {  // walker back to INT_MAX, as after a batch
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= V) return;
+  const int s = slot_of[i];
+  if (s >= 0) walker[s] = INT_MAX;
 }
 
 // ---- svnicp_map_evaluate ----------------------------------------------------------------------------------------------------
@@ -466,6 +678,9 @@ struct svnicp_map_t {
   uint8_t *ev_mask = nullptr;
   float *ev_near = nullptr;
   size_t ev_src_cap = 0, ev_part_cap = 0, ev_mask_cap = 0, ev_near_cap = 0;
+  // svnicp_map_export / svnicp_map_import scratch (grown on demand; nothing above is touched by it), indexed by SN_*
+  void *sn[11] = {};
+  size_t sn_cap[11] = {};
   int sm_count = 148;
   cudaStream_t stream = nullptr;
   std::string err;
@@ -557,6 +772,7 @@ void svnicp_map_destroy(svnicp_map m) {
   cudaFree(m->head); cudaFree(m->walker); cudaFree(m->counters); cudaFree(m->d_pose); cudaFree(m->block_sums);
   cudaFree(m->batch_in); cudaFree(m->wxyz); cudaFree(m->pt_slot); cudaFree(m->next); cudaFree(m->out);
   cudaFree(m->ev_src); cudaFree(m->ev_pose); cudaFree(m->ev_part); cudaFree(m->ev_out); cudaFree(m->ev_mask); cudaFree(m->ev_near);
+  for (void *p : m->sn) cudaFree(p);
   if (m->h_counters) cudaFreeHost(m->h_counters);
   if (m->stream) cudaStreamDestroy(m->stream);
   delete m;
@@ -665,7 +881,7 @@ int svnicp_map_get(svnicp_map m, const double position[3], double max_range, con
   const int n_blocks = (int)((m->slots + SCAN_BLOCK - 1) / SCAN_BLOCK);
   const double r2 = max_range * max_range;
   k_getmap_count<<<n_blocks, SCAN_BLOCK, 0, m->stream>>>(d, m->d_pose + 12, r2, all, m->block_sums);
-  k_getmap_scan<<<1, SCAN_BLOCK, 0, m->stream>>>(m->block_sums, n_blocks, m->counters + 2);
+  k_getmap_scan<int><<<1, SCAN_BLOCK, 0, m->stream>>>(m->block_sums, n_blocks, m->counters + 2);
   k_getmap_emit<<<n_blocks, SCAN_BLOCK, 0, m->stream>>>(d, m->d_pose + 12, r2, all, m->block_sums, m->out);
   MCU(cudaGetLastError());
   int rc = sync_counters(m);
@@ -784,5 +1000,153 @@ extern "C" int svnicp_map_evaluate(svnicp_map m, const void *source, int64_t n, 
       if (out_b) memcpy(out_b + 6 * g, o + 39, 6 * sizeof(double));
     }
   }
+  return SVNICP_OK;
+}
+
+// ---- svnicp_map_export / svnicp_map_import -----------------------------------------------------------------------------------
+enum { SN_KEY0, SN_KEY1, SN_SLOT0, SN_SLOT1, SN_OFF, SN_PSUM, SN_HIST, SN_WORDS, SN_VOX, SN_CNT, SN_XYZ, SN_COUNT };
+static_assert(SN_COUNT == sizeof(svnicp_map_t::sn) / sizeof(void *), "one scratch buffer per SN_* index");
+
+static int sn_grow(svnicp_map m, int k, size_t bytes) { return ev_grow(m, &m->sn[k], &m->sn_cap[k], bytes > 0 ? bytes : 1); }
+
+// int64 exclusive scan of the V voxels' point counts into sn[SN_OFF] (the table's counts through slots, or a snapshot's counts);
+// the total goes to the device word *total
+static void launch_point_offsets(svnicp_map m, const int32_t *counts, const int *slots, const int *tab_count, long long V, long long *total) {
+  const int nb = (int)((V + SCAN_BLOCK - 1) / SCAN_BLOCK);
+  long long *psum = (long long *)m->sn[SN_PSUM], *off = (long long *)m->sn[SN_OFF];
+  k_snap_pts_count<<<nb, SCAN_BLOCK, 0, m->stream>>>(counts, slots, tab_count, m->cap, V, psum);
+  k_getmap_scan<long long><<<1, SCAN_BLOCK, 0, m->stream>>>(psum, nb, total);
+  k_snap_pts_offsets<<<nb, SCAN_BLOCK, 0, m->stream>>>(counts, slots, tab_count, m->cap, V, psum, off);
+}
+
+extern "C" int svnicp_map_export(svnicp_map m, int32_t *voxels, int32_t *counts, float *xyz, int64_t n_voxels, int64_t n_points, int on_device) {
+  if (!m) return SVNICP_ERR_INVALID;
+  const long long V = m->h_counters[0], N = m->h_counters[1];
+  if (n_voxels != V || n_points != N) {
+    char buf[256];
+    snprintf(buf, sizeof(buf), "svnicp_map_export: n_voxels = %lld and n_points = %lld, but the map holds %lld voxels and %lld points",
+             (long long)n_voxels, (long long)n_points, V, N);
+    return mfail(m, SVNICP_ERR_INVALID, buf);
+  }
+  if ((V > 0 && (!voxels || !counts)) || (N > 0 && !xyz)) return mfail(m, SVNICP_ERR_INVALID, "svnicp_map_export: null output");
+  if (V == 0) return SVNICP_OK;
+  MCU(cudaSetDevice(m->device));
+  cudaStream_t st = m->stream;
+  const int n_tiles = (int)((V + RADIX_TILE - 1) / RADIX_TILE);
+  const int slot_blocks = (int)((m->slots + SCAN_BLOCK - 1) / SCAN_BLOCK);
+  const size_t hist_n = (size_t)RADIX_DIGITS * n_tiles > (size_t)slot_blocks ? (size_t)RADIX_DIGITS * n_tiles : (size_t)slot_blocks;
+  int rc;
+  if ((rc = sn_grow(m, SN_KEY0, V * 8)) || (rc = sn_grow(m, SN_KEY1, V * 8)) || (rc = sn_grow(m, SN_SLOT0, V * 4)) ||
+      (rc = sn_grow(m, SN_SLOT1, V * 4)) || (rc = sn_grow(m, SN_OFF, V * 8)) || (rc = sn_grow(m, SN_PSUM, (V / SCAN_BLOCK + 2) * 8)) ||
+      (rc = sn_grow(m, SN_HIST, hist_n * 4)) || (rc = sn_grow(m, SN_WORDS, 4 * 8)) ||
+      (!on_device && ((rc = sn_grow(m, SN_VOX, V * 12)) || (rc = sn_grow(m, SN_CNT, V * 4)) || (rc = sn_grow(m, SN_XYZ, N * 12)))))
+    return rc;
+  unsigned long long *key[2] = {(unsigned long long *)m->sn[SN_KEY0], (unsigned long long *)m->sn[SN_KEY1]};
+  int *slot[2] = {(int *)m->sn[SN_SLOT0], (int *)m->sn[SN_SLOT1]};
+  int *hist = (int *)m->sn[SN_HIST];
+  long long *words = (long long *)m->sn[SN_WORDS];  // [0] live slots, [1] their points, [3] sink of the radix scans
+  MCU(cudaMemsetAsync(words, 0, 4 * sizeof(long long), st));
+  const MapDev d = dev_view(m, m->cur);
+  k_snap_count<<<slot_blocks, SCAN_BLOCK, 0, st>>>(d, hist);
+  k_getmap_scan<int><<<1, SCAN_BLOCK, 0, st>>>(hist, slot_blocks, words);
+  k_snap_emit<<<slot_blocks, SCAN_BLOCK, 0, st>>>(d, hist, V, key[0], slot[0]);
+  for (int shift = 0, a = 0; shift < CANON_BITS; shift += RADIX_BITS, a ^= 1) {
+    k_radix_hist<<<n_tiles, RADIX_THREADS, 0, st>>>(key[a], (int)V, shift, n_tiles, hist);
+    k_getmap_scan<int><<<1, SCAN_BLOCK, 0, st>>>(hist, RADIX_DIGITS * n_tiles, words + 3);
+    k_radix_scatter<<<n_tiles, RADIX_THREADS, 0, st>>>(key[a], slot[a], key[a ^ 1], slot[a ^ 1], (int)V, shift, n_tiles, hist);
+  }
+  launch_point_offsets(m, nullptr, slot[0], d.tab.count, V, words + 1);
+  int32_t *ov = on_device ? voxels : (int32_t *)m->sn[SN_VOX], *oc = on_device ? counts : (int32_t *)m->sn[SN_CNT];
+  float *ox = on_device ? xyz : (float *)m->sn[SN_XYZ];
+  k_snap_gather<<<(unsigned)((V * 32 + 255) / 256), 256, 0, st>>>(d.tab, m->cap, key[0], slot[0], (const long long *)m->sn[SN_OFF], V, N, ov, oc, ox);
+  MCU(cudaGetLastError());
+  if (!on_device) {
+    MCU(cudaMemcpyAsync(voxels, ov, (size_t)V * 3 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    MCU(cudaMemcpyAsync(counts, oc, (size_t)V * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    if (N > 0) MCU(cudaMemcpyAsync(xyz, ox, (size_t)N * 3 * sizeof(float), cudaMemcpyDeviceToHost, st));
+  }
+  long long h[2];
+  MCU(cudaMemcpyAsync(h, words, sizeof(h), cudaMemcpyDeviceToHost, st));
+  MCU(cudaStreamSynchronize(st));
+  if (h[0] != V || h[1] != N) {
+    char buf[256];
+    snprintf(buf, sizeof(buf), "svnicp_map_export: the table holds %lld voxels and %lld points, the counters %lld and %lld", h[0], h[1], V, N);
+    return mfail(m, SVNICP_ERR_CUDA, buf);
+  }
+  return SVNICP_OK;
+}
+
+extern "C" int svnicp_map_import(svnicp_map m, const int32_t *voxels, const int32_t *counts, const float *xyz, int64_t n_voxels,
+                                 int64_t n_points, int on_device) {
+  if (!m) return SVNICP_ERR_INVALID;
+  char buf[256];
+  if (n_voxels < 0 || n_points < 0) return mfail(m, SVNICP_ERR_INVALID, "svnicp_map_import: negative n_voxels or n_points");
+  if ((n_voxels > 0 && (!voxels || !counts)) || (n_points > 0 && !xyz)) return mfail(m, SVNICP_ERR_INVALID, "svnicp_map_import: null input");
+  const long long V = n_voxels, N = n_points;
+  if ((size_t)V > m->slots / 2) {
+    snprintf(buf, sizeof(buf), "svnicp_map_import: %lld voxels do not fit a table of %zu voxels; create the map with a larger capacity_voxels",
+             V, m->slots / 2);
+    return mfail(m, SVNICP_ERR_OOM, buf);
+  }
+  if (N > V * m->cap) {
+    snprintf(buf, sizeof(buf), "svnicp_map_import: n_points = %lld exceeds n_voxels * max_pointscount = %lld, so it is not the sum of the counts",
+             N, V * m->cap);
+    return mfail(m, SVNICP_ERR_INVALID, buf);
+  }
+  if (V == 0) return svnicp_map_clear(m);  // N == 0 here
+  MCU(cudaSetDevice(m->device));
+  cudaStream_t st = m->stream;
+  int rc;
+  if ((rc = sn_grow(m, SN_SLOT0, V * 4)) || (rc = sn_grow(m, SN_OFF, V * 8)) || (rc = sn_grow(m, SN_PSUM, (V / SCAN_BLOCK + 2) * 8)) ||
+      (rc = sn_grow(m, SN_WORDS, 4 * 8)) ||
+      (!on_device && ((rc = sn_grow(m, SN_VOX, V * 12)) || (rc = sn_grow(m, SN_CNT, V * 4)) || (rc = sn_grow(m, SN_XYZ, N * 12)))))
+    return rc;
+  if (!on_device) {
+    MCU(cudaMemcpyAsync(m->sn[SN_VOX], voxels, (size_t)V * 3 * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    MCU(cudaMemcpyAsync(m->sn[SN_CNT], counts, (size_t)V * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    if (N > 0) MCU(cudaMemcpyAsync(m->sn[SN_XYZ], xyz, (size_t)N * 3 * sizeof(float), cudaMemcpyHostToDevice, st));
+    voxels = (const int32_t *)m->sn[SN_VOX];
+    counts = (const int32_t *)m->sn[SN_CNT];
+    xyz = (const float *)m->sn[SN_XYZ];
+  }
+  // build into the twin table (the one RemoveFar rebuilds into); the map's own table, cur and counters stay as they are
+  const int nxt = m->cur ^ 1;
+  if ((rc = clear_table(m, nxt))) return rc;
+  // [0] lowest count / index error, [1] sum of the valid counts, [2] voxels refused, [3] lowest duplicate / membership error
+  long long *words = (long long *)m->sn[SN_WORDS];
+  MCU(cudaMemsetAsync(words, 0xFF, 4 * sizeof(long long), st));
+  MCU(cudaMemsetAsync(words + 1, 0, 2 * sizeof(long long), st));
+  launch_point_offsets(m, counts, nullptr, nullptr, V, words + 1);
+  const MapDev dn = dev_view(m, nxt);
+  int *slot_of = (int *)m->sn[SN_SLOT0];
+  k_map_import<<<(unsigned)((V * 32 + 255) / 256), 256, 0, st>>>(dn, voxels, counts, xyz, V, N, (const long long *)m->sn[SN_OFF], slot_of,
+                                                                 (unsigned long long *)words);
+  const unsigned grid = (unsigned)((V + 255) / 256);
+  k_map_import_dups<<<grid, 256, 0, st>>>(m->walker, slot_of, V, (unsigned long long *)words);
+  k_map_import_reset<<<grid, 256, 0, st>>>(m->walker, slot_of, V);
+  MCU(cudaGetLastError());
+  unsigned long long h[4];
+  MCU(cudaMemcpyAsync(h, words, sizeof(h), cudaMemcpyDeviceToHost, st));
+  MCU(cudaStreamSynchronize(st));
+  // the counts and indices first, then their sum (which places the points), then what the points say: each names its lowest voxel
+  static const char *why[] = {"", "its count is outside [1, max_pointscount]", "its index is outside [-2^20, 2^20)",
+                              "it repeats an earlier voxel", "a point does not belong to it"};
+  const bool sum_ok = (long long)h[1] == N;
+  const unsigned long long e = h[0] != SNAP_NO_ERROR ? h[0] : sum_ok ? h[3] : SNAP_NO_ERROR;
+  if (e != SNAP_NO_ERROR) {
+    snprintf(buf, sizeof(buf), "svnicp_map_import: voxel %llu: %s", e >> 3, why[e & 7]);
+    return mfail(m, SVNICP_ERR_INVALID, buf);
+  }
+  if (!sum_ok) {
+    snprintf(buf, sizeof(buf), "svnicp_map_import: n_points = %lld, but the counts sum to %lld", N, (long long)h[1]);
+    return mfail(m, SVNICP_ERR_INVALID, buf);
+  }
+  if (h[2] > 0) return mfail(m, SVNICP_ERR_OOM, "svnicp_map_import: the voxel table is full");
+  long long size[2] = {V, N};
+  MCU(cudaMemcpyAsync(m->counters, size, sizeof(size), cudaMemcpyHostToDevice, st));
+  MCU(cudaStreamSynchronize(st));
+  m->h_counters[0] = V;
+  m->h_counters[1] = N;
+  m->cur = nxt;
   return SVNICP_OK;
 }

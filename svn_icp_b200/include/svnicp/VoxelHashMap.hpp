@@ -4,12 +4,90 @@
 // map every scan: OdometryPipeline.cpp:577-581).  Poses are passed as svnicp::InitialMean (row-major R, t).
 #pragma once
 #include <cstdint>
+#include <cstdio>
+#include <cstring>
+#include <memory>
 #include <string>
 #include <vector>
 
 #include "svnicp/SVNICP.hpp"
 
 namespace svnicp {
+
+/** A local map's content in canonical form (svnicp_map_export): voxels [V][3] ascending (vx, vy, vz), counts [V], xyz [Npts][3]
+ *  with each voxel's points in stored order, and the parameters of the map it came from. */
+struct MapSnapshot {
+  double voxel_size = 1.0;
+  double max_range = 80;
+  int max_pointscount = 20;
+  std::vector<int32_t> voxels;
+  std::vector<int32_t> counts;
+  std::vector<float> xyz;
+};
+
+/** The snapshot file, shared with the Python mirror: little-endian header "SVNMAP01", u32 version 1, u32 max_pointscount,
+ *  f64 voxel_size, f64 max_range, i64 V, i64 Npts; then voxels int32 [V][3], counts int32 [V], xyz float [Npts][3].  No GPU. */
+constexpr uint32_t kMapSnapshotVersion = 1;
+
+namespace detail {
+inline bool host_is_little_endian() {
+  const uint16_t one = 1;
+  unsigned char b;
+  std::memcpy(&b, &one, 1);
+  return b == 1;
+}
+}  // namespace detail
+
+inline void write_map_snapshot(const std::string &path, const MapSnapshot &s) {
+  if (!detail::host_is_little_endian()) throw Error("write_map_snapshot: the file format is little-endian, this host is not");
+  if (s.voxels.size() != 3 * s.counts.size() || s.xyz.size() % 3 != 0) throw Error("write_map_snapshot: voxels, counts and xyz disagree");
+  std::unique_ptr<FILE, int (*)(FILE *)> f(std::fopen(path.c_str(), "wb"), &std::fclose);
+  if (!f) throw Error("write_map_snapshot: cannot open " + path);
+  const uint32_t head32[2] = {kMapSnapshotVersion, (uint32_t)s.max_pointscount};
+  const double headf[2] = {s.voxel_size, s.max_range};
+  const int64_t sizes[2] = {(int64_t)s.counts.size(), (int64_t)(s.xyz.size() / 3)};
+  bool ok = std::fwrite("SVNMAP01", 1, 8, f.get()) == 8 && std::fwrite(head32, sizeof(head32), 1, f.get()) == 1 &&
+            std::fwrite(headf, sizeof(headf), 1, f.get()) == 1 && std::fwrite(sizes, sizeof(sizes), 1, f.get()) == 1;
+  ok = ok && std::fwrite(s.voxels.data(), sizeof(int32_t), s.voxels.size(), f.get()) == s.voxels.size();
+  ok = ok && std::fwrite(s.counts.data(), sizeof(int32_t), s.counts.size(), f.get()) == s.counts.size();
+  ok = ok && std::fwrite(s.xyz.data(), sizeof(float), s.xyz.size(), f.get()) == s.xyz.size();
+  if (!ok || std::fflush(f.get()) != 0) throw Error("write_map_snapshot: cannot write " + path);
+}
+
+/** Rejects a wrong magic or version and a file whose length does not match the sizes. */
+inline MapSnapshot read_map_snapshot(const std::string &path) {
+  if (!detail::host_is_little_endian()) throw Error("read_map_snapshot: the file format is little-endian, this host is not");
+  std::unique_ptr<FILE, int (*)(FILE *)> f(std::fopen(path.c_str(), "rb"), &std::fclose);
+  if (!f) throw Error("read_map_snapshot: cannot open " + path);
+  char magic[8];
+  uint32_t head32[2];
+  double headf[2];
+  int64_t sizes[2];
+  if (std::fread(magic, 1, 8, f.get()) != 8 || std::memcmp(magic, "SVNMAP01", 8) != 0) throw Error(path + ": not a map snapshot (magic)");
+  if (std::fread(head32, sizeof(head32), 1, f.get()) != 1 || std::fread(headf, sizeof(headf), 1, f.get()) != 1 ||
+      std::fread(sizes, sizeof(sizes), 1, f.get()) != 1)
+    throw Error(path + ": not a map snapshot (shorter than its header)");
+  if (head32[0] != kMapSnapshotVersion) throw Error(path + ": map snapshot version " + std::to_string(head32[0]) + ", this reader knows 1");
+  const int64_t V = sizes[0], N = sizes[1];
+  if (std::fseek(f.get(), 0, SEEK_END) != 0) throw Error("read_map_snapshot: cannot seek in " + path);
+  const long long len = std::ftell(f.get());
+  // sizes bounded before they are multiplied: 2^40 points are far beyond any file this could be
+  if (V < 0 || N < 0 || V > (1ll << 40) || N > (1ll << 40) || len != 48 + 16 * V + 12 * N)
+    throw Error(path + ": map snapshot length does not match V = " + std::to_string(V) + ", Npts = " + std::to_string(N));
+  std::fseek(f.get(), 48, SEEK_SET);
+  MapSnapshot s;
+  s.max_pointscount = (int)head32[1];
+  s.voxel_size = headf[0];
+  s.max_range = headf[1];
+  s.voxels.resize((size_t)V * 3);
+  s.counts.resize((size_t)V);
+  s.xyz.resize((size_t)N * 3);
+  if (std::fread(s.voxels.data(), sizeof(int32_t), s.voxels.size(), f.get()) != s.voxels.size() ||
+      std::fread(s.counts.data(), sizeof(int32_t), s.counts.size(), f.get()) != s.counts.size() ||
+      std::fread(s.xyz.data(), sizeof(float), s.xyz.size(), f.get()) != s.xyz.size())
+    throw Error("read_map_snapshot: cannot read " + path);
+  return s;
+}
 
 struct VoxelHashMap {
   double voxel_size_ = 1.0;   // VoxelHashMap.h:32-34
@@ -86,6 +164,39 @@ struct VoxelHashMap {
       r.rmse.push_back(stats[3 * m + 2]);
     }
     return r;
+  }
+
+  using Snapshot = MapSnapshot;
+  /** The content in canonical form (svnicp_map_export; no reference counterpart) */
+  Snapshot Export() const {
+    int64_t V = 0, N = 0;
+    check(svnicp_map_size(m_, &V, &N), "Export");
+    Snapshot s;
+    s.voxel_size = voxel_size_;
+    s.max_range = max_range_;
+    s.max_pointscount = max_pointscount_;
+    s.voxels.resize((size_t)V * 3);
+    s.counts.resize((size_t)V);
+    s.xyz.resize((size_t)N * 3);
+    check(svnicp_map_export(m_, s.voxels.data(), s.counts.data(), s.xyz.data(), V, N, 0), "Export");
+    return s;
+  }
+  /** Replace the content by a snapshot of a map with the same parameters (svnicp_map_import; all or nothing) */
+  void Import(const Snapshot &s) {
+    if (s.voxel_size != voxel_size_ || s.max_range != max_range_ || s.max_pointscount != max_pointscount_)
+      throw Error("Import: the snapshot's voxel_size, max_range or max_pointscount differ from this map's");
+    if (s.voxels.size() != 3 * s.counts.size() || s.xyz.size() % 3 != 0) throw Error("Import: voxels, counts and xyz disagree");
+    check(svnicp_map_import(m_, s.voxels.data(), s.counts.data(), s.xyz.data(), (int64_t)s.counts.size(), (int64_t)(s.xyz.size() / 3), 0),
+          "Import");
+  }
+  void Save(const std::string &path) const { write_map_snapshot(path, Export()); }
+  /** A new map with the file's parameters, a capacity of at least its voxel count, and its content */
+  static std::unique_ptr<VoxelHashMap> Load(const std::string &path, int64_t capacity_voxels = 1 << 19, int device = -1) {
+    const Snapshot s = read_map_snapshot(path);
+    const int64_t V = (int64_t)s.counts.size();
+    std::unique_ptr<VoxelHashMap> m(new VoxelHashMap(s.voxel_size, s.max_range, s.max_pointscount, capacity_voxels > V ? capacity_voxels : V, device));
+    m->Import(s);
+    return m;
   }
 
  private:
