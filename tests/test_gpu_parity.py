@@ -73,12 +73,16 @@ def test_candidate_table_tiny_map(oracle):
     assert np.all(idx[:, 10:] == 0)
 
 
-@pytest.mark.parametrize("which", ["small", "lidar"])
+@pytest.mark.parametrize("which", ["small", "lidar", "lidar_p30"])
 def test_correspondence_indices_bit_exact(oracle, request, which):
     """Indices chosen by the fused kernel == oracle restatement of the same fp32 arithmetic on the same inputs; the
-    exact pruning pass must not change a single index."""
-    pb = request.getfixturevalue(which)
-    icp = make_icp(pb, iterations=1, KNN_count=100, max_dist=3.0, debug_corr=True)
+    exact pruning pass must not change a single index.  lidar_p30: 30 particles (the reference's shipped regime), k_gn without
+    the warp-uniform early exit (fewer than 32 particle pairs per row group)."""
+    pb = request.getfixturevalue(which.split("_")[0])
+    init = pb.init_pose[:, :30] if which.endswith("_p30") else pb.init_pose
+    icp = sv.SVNICP(sv.SteinICPParam(iterations=1, KNN_count=100, max_dist=3.0, debug_corr=True), init)
+    icp.add_cloud(pb.source, pb.target, init)
+    icp.set_initial_mean(pb.R0, pb.t0)
     icp.stein_align()
     xf, idx, mask = icp.get_correspondences()
     cidx, rel = icp.get_candidates(want_rel=True)
@@ -87,7 +91,7 @@ def test_correspondence_indices_bit_exact(oracle, request, which):
     np.testing.assert_array_equal(idx, oidx)
     np.testing.assert_array_equal(mask, omask)
     # transforms from the fp64 state
-    R, t = initial_state(oracle, pb.init_pose)
+    R, t = initial_state(oracle, init)
     np.testing.assert_allclose(xf, oracle.transforms_f32(R, t, pb.R0), rtol=0, atol=2e-7)
     # against the reference semantics in fp64 (different arithmetic): only near-ties may differ
     q0 = oracle.transform_q0(pb.source, pb.R0, pb.t0)
