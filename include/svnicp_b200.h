@@ -52,6 +52,9 @@ typedef enum {
 #define SVNICP_CLASS_SVNICP 0
 #define SVNICP_CLASS_SVGDICP 1
 
+/* largest particle_count svnicp_create accepts: the bandwidth median counts the P^2 pairwise distances in 32-bit bins */
+#define SVNICP_MAX_PARTICLES 65535
+
 /* SteinICPParam (SVGDICP.h:41-57) + ParticleWeightOpt (SVNICP.h:25-27); same defaults. */
 typedef struct {
   int32_t iterations;            /* 50   */
@@ -101,7 +104,7 @@ int svnicp_abi_version(void);
  *   gradient (:398-455), RBF SVGD step (:457-474), params->optimizer update (:142-170, :476-494); svnicp_align returns
  *   SVNICP_NO_OPTIMIZER for an unknown optimizer name.  The constructor's init_pose seeds pose_particles_, which
  *   add_cloud does not refresh (:46-62): iteration 0 of a scan evaluates the kernel on the previous result.
- * use_minibatch != 0 is rejected (the reference never enables it, :178-185). */
+ * use_minibatch != 0 is rejected (the reference never enables it, :178-185); so is particle_count > SVNICP_MAX_PARTICLES. */
 int svnicp_create(svnicp_handle *out, const svnicp_params *params, int particle_count, const double *init_pose,
                   int class_type, int device);
 void svnicp_destroy(svnicp_handle h);
@@ -165,6 +168,10 @@ int svnicp_get_stein(svnicp_handle h, double *out_delta, double *out_bandwidth);
 /* mean candidates per (point) kept by the exact pruning pass, per iteration [iterations]
  * (handle created with SVNICP_FLAG_REUSE_STATS: the fraction of rows pruned from the previous iteration's list) */
 int svnicp_get_prune_stats(svnicp_handle h, double *out_mean_kept, int32_t *rows);
+/* how each iteration's bandwidth median was found, per iteration [iterations]: 0 sort of all pairs (P <= 64), 1 linear
+ * histogram around the previous median, 2 radix select (iteration 0, or the median left that histogram's window), 3 radix
+ * select after the histogram bin held too many values to pick from; -1 none (P == 1, iterations that did not run) */
+int svnicp_get_median_paths(svnicp_handle h, int32_t *out, int32_t *rows);
 /* device time of the phases of the last scan in ms: {setup, iterations, epilogue, total} */
 int svnicp_get_timing(svnicp_handle h, double out4[4]);
 /* local particle slice [lo, hi) */

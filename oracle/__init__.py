@@ -108,6 +108,14 @@ class Oracle:
         self.lib.oracle_stein_step(_ptr(x), _ptr(H), _ptr(b), C.c_int(P), C.c_int(int(full)), C.c_double(lr), _ptr(d), C.byref(h))
         return d, h.value
 
+    def pair_median_kernel_order(self, x):
+        """(median, nearest distinct entry below, nearest above) of the P^2 pairwise squared distances of x [P, 6], rounded
+        as the k_head_* kernels round them (oracle_pair_median_kernel_order)."""
+        x = _f64(x)
+        out = np.zeros(3)
+        self.lib.oracle_pair_median_kernel_order(_ptr(x), C.c_int(len(x)), _ptr(out))
+        return tuple(out.tolist())
+
     def pose_update(self, R, t, delta):
         R, t, delta = _f64(R).copy(), _f64(t).copy(), _f64(delta)
         with np.errstate(all="ignore"):

@@ -282,10 +282,9 @@ static void particle_gn(const double *Rt /*R_total 3x3*/, const double *tt /*t_t
   for (int k = 0; k < 6; k++) H[7 * k] += 1e-6; /* :153 (Q3) */
 }
 
-/* lower median of n doubles (torch::median over the flattened tensor, SVNICP.cpp:262):
- * element (n-1)/2 of the sorted order.  Quickselect on a scratch copy. */
-static double lower_median(double *a, int64_t n) {
-  int64_t k = (n - 1) / 2, lo = 0, hi = n - 1;
+/* element k of the ascending order of n doubles (no NaN).  Quickselect, reorders a. */
+static double select_kth(double *a, int64_t n, int64_t k) {
+  int64_t lo = 0, hi = n - 1;
   while (lo < hi) {
     double pv = a[lo + (hi - lo) / 2];
     int64_t i = lo, j = hi;
@@ -299,6 +298,42 @@ static double lower_median(double *a, int64_t n) {
     else break;
   }
   return a[k];
+}
+
+/* lower median of n doubles (torch::median over the flattened tensor, SVNICP.cpp:262):
+ * element (n-1)/2 of the sorted order.  Quickselect on a scratch copy. */
+static double lower_median(double *a, int64_t n) { return select_kth(a, n, (n - 1) / 2); }
+
+/* The bandwidth median as the k_head_* kernels compute it (tail2.cu): pair distances rounded as in hd_sweep,
+ * s = fma(df0, df0, df1 * df1), then s = fma(df, df, s) for d = 2..5, once per unordered pair.  x: [P][6].
+ * out[0] = lower median of the P^2 entries (P diagonal zeros, every pair twice), out[1] / out[2] = the nearest distinct
+ * entry below / above it (-inf / +inf if there is none): a bandwidth check that rejects a neighbouring rank. */
+void oracle_pair_median_kernel_order(const double *x, int P, double out[3]) {
+  const int64_t n = (int64_t)P * (P - 1) / 2;
+  const int64_t rank = ((int64_t)P * P - 1) / 2;
+  out[0] = 0.0; out[1] = -INFINITY; out[2] = INFINITY;
+  if (n == 0) return;
+  double *a = (double *)malloc(sizeof(double) * (size_t)n);
+#pragma omp parallel for schedule(dynamic, 16)
+  for (int i = 0; i < P; i++) {
+    double *row = a + (int64_t)i * (2 * (int64_t)P - i - 1) / 2;  /* pairs (i, j > i) */
+    for (int j = i + 1; j < P; j++) {
+      double df[6];
+      for (int d = 0; d < 6; d++) df[d] = x[6 * i + d] - x[6 * j + d];
+      double s = fma(df[0], df[0], df[1] * df[1]);
+      for (int d = 2; d < 6; d++) s = fma(df[d], df[d], s);
+      row[j - i - 1] = s;
+    }
+  }
+  /* ascending: P zeros, then pair k at entries P + 2k and P + 2k + 1 */
+  const double m = rank < P ? 0.0 : select_kth(a, n, (rank - P) / 2);
+  double below = m > 0.0 ? 0.0 : -INFINITY, above = INFINITY;
+  for (int64_t k = 0; k < n; k++) {
+    if (a[k] < m && a[k] > below) below = a[k];
+    if (a[k] > m && a[k] < above) above = a[k];
+  }
+  out[0] = m; out[1] = below; out[2] = above;
+  free(a);
 }
 
 /* SVNICP::rbf_hessian_kernel, SVNICP.cpp:254-266.  x: [P][6].  Kmat: [P][P]. returns h. */

@@ -24,6 +24,10 @@ ALIGN_SUCCESS = 1  # SteinICPState, SVGDICP.h:59-62
 NO_OPTIMIZER = 2
 CLASS_SVNICP = 0
 CLASS_SVGDICP = 1
+MAX_PARTICLES = 65535  # SVNICP_MAX_PARTICLES
+
+# svnicp_get_median_paths: how an iteration's bandwidth median was found (include/svnicp_b200.h)
+MEDIAN_NONE, MEDIAN_SORT, MEDIAN_FAST, MEDIAN_RADIX, MEDIAN_OVERFLOW = -1, 0, 1, 2, 3
 
 
 class SvnIcpError(RuntimeError):
@@ -88,7 +92,7 @@ EXPORTS = [
     "svnicp_get_particle_weight", "svnicp_get_particle_history", "svnicp_get_runtime", "svnicp_set_k", "svnicp_set_threshold",
     "svnicp_initialize_particles", "svnicp_initialize_particles_gaussian", "svnicp_iterations_done", "svnicp_get_candidates",
     "svnicp_get_source_f32", "svnicp_get_correspondences", "svnicp_get_gn_system", "svnicp_get_stein", "svnicp_get_prune_stats",
-    "svnicp_get_timing", "svnicp_get_slice", "svnicp_get_launch_count", "svnicp_set_profiling", "svnicp_get_phase_times",
+    "svnicp_get_median_paths", "svnicp_get_timing", "svnicp_get_slice", "svnicp_get_launch_count", "svnicp_set_profiling", "svnicp_get_phase_times",
     "svnicp_get_scan_info", "svnicp_get_tail_stamps", "svnicp_evaluate",
     "svnicp_map_create", "svnicp_map_destroy", "svnicp_map_last_error", "svnicp_map_clear", "svnicp_map_add_cloud", "svnicp_map_get",
     "svnicp_map_download", "svnicp_map_size", "svnicp_map_evaluate", "svnicp_map_export", "svnicp_map_import",
@@ -147,6 +151,7 @@ def _ARGTYPES(V, I, L, D):
         "svnicp_initialize_particles_gaussian": [I, V, C.c_uint64, V], "svnicp_iterations_done": [V, V],
         "svnicp_get_candidates": [V, V, V], "svnicp_get_source_f32": [V, V], "svnicp_get_correspondences": [V, V, V, V],
         "svnicp_get_gn_system": [V, V, V, V], "svnicp_get_stein": [V, V, V], "svnicp_get_prune_stats": [V, V, V],
+        "svnicp_get_median_paths": [V, V, V],
         "svnicp_get_timing": [V, V], "svnicp_get_slice": [V, V, V], "svnicp_get_launch_count": [V, V],
         "svnicp_get_tail_stamps": [V, V], "svnicp_set_profiling": [V, I], "svnicp_get_phase_times": [V, V], "svnicp_get_scan_info": [V, V],
         "svnicp_evaluate": [V, I, V, V, V, V, V, V],
@@ -419,6 +424,13 @@ class SVNICP:
         out = np.zeros(max(self.param.iterations, 1))
         rows = C.c_int32(0)
         self._check(self._lib.svnicp_get_prune_stats(self._h, _p(out), C.byref(rows)), "get_prune_stats")
+        return out[:self.param.iterations]
+
+    def get_median_paths(self):
+        """[iterations] int32: how each iteration's bandwidth median was found (MEDIAN_* codes; -1 none)."""
+        out = np.full(max(self.param.iterations, 1), -1, dtype=np.int32)
+        rows = C.c_int32(0)
+        self._check(self._lib.svnicp_get_median_paths(self._h, _p(out), C.byref(rows)), "get_median_paths")
         return out[:self.param.iterations]
 
     def get_timing(self):

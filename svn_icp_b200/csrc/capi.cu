@@ -132,7 +132,7 @@ struct svnicp_handle_t {
   DevBuf<float> xf, history, dbg_xf;
   DevBuf<unsigned> hist;
   DevBuf<Ctrl> ctrl;
-  DevBuf<int32_t> dbg_idx;
+  DevBuf<int32_t> dbg_idx, med_path;
   DevBuf<uint8_t> dbg_mask;
   // pinned host mirrors
   double *h_stats = nullptr;      // 48
@@ -141,6 +141,7 @@ struct svnicp_handle_t {
   Ctrl *h_ctrl = nullptr;
   int *h_stop = nullptr;          // per-iteration stop snapshots
   unsigned long long *h_kept = nullptr;
+  int32_t *h_med = nullptr;       // per-iteration median path (svnicp_get_median_paths)
   size_t h_hist_cap = 0, h_stop_cap = 0;
   std::vector<cudaEvent_t> iter_events;
   cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
@@ -331,6 +332,7 @@ static int alloc_particle_state(svnicp_handle h) {
   const size_t I = (size_t)(h->prm.iterations > 0 ? h->prm.iterations : 1);
   CU(h->history.ensure(I * 6 * h->P));
   CU(h->kept_hist.ensure(I + 2, true));
+  CU(h->med_path.ensure(I + 2));
   if (h->class_type == SVNICP_CLASS_SVGDICP) {
     CU(h->pose6.ensure(6 * P, true));
     CU(h->prev.ensure(6 * P, true));
@@ -355,6 +357,10 @@ int svnicp_create(svnicp_handle *out, const svnicp_params *params, int particle_
   if (!out || !params) return fail(nullptr, SVNICP_ERR_INVALID, "null argument");
   *out = nullptr;
   if (particle_count < 1) return fail(nullptr, SVNICP_ERR_INVALID, "particle_count must be >= 1");
+  if (particle_count > SVNICP_MAX_PARTICLES)  // k_head_* count the P^2 pairwise distances in 32-bit histogram bins (tail2.cu)
+    return fail(nullptr, SVNICP_ERR_INVALID,
+                "particle_count %d exceeds %d: the bandwidth median counts the P^2 pairwise distances in 32-bit histograms",
+                particle_count, SVNICP_MAX_PARTICLES);
   if (class_type != SVNICP_CLASS_SVNICP && class_type != SVNICP_CLASS_SVGDICP)
     return fail(nullptr, SVNICP_ERR_INVALID, "class_type must be SVNICP_CLASS_SVNICP or SVNICP_CLASS_SVGDICP");
   if (params->use_minibatch)
@@ -451,7 +457,7 @@ void svnicp_destroy(svnicp_handle h) {
   for (int i = 0; i < 2; i++) { h->ball[i].release(); h->cbase[i].release(); }
   h->cand_idx.release();
   h->counts.release(); h->starts.release(); h->fill.release(); h->pt_slot.release(); h->sidx.release(); h->misc.release();
-  h->keys.release(); h->kept_hist.release(); h->xf.release(); h->dbg_xf.release(); h->history.release(); h->hist.release(); h->ctrl.release();
+  h->keys.release(); h->kept_hist.release(); h->med_path.release(); h->xf.release(); h->dbg_xf.release(); h->history.release(); h->hist.release(); h->ctrl.release();
   h->dbg_idx.release(); h->dbg_mask.release();
   h->ev_pose.release(); h->ev_R.release(); h->ev_part.release(); h->ev_out.release(); h->ev_xf.release(); h->ev_mask.release(); h->ev_idx.release();
   if (h->h_stats) cudaFreeHost(h->h_stats);
@@ -460,6 +466,7 @@ void svnicp_destroy(svnicp_handle h) {
   if (h->h_ctrl) cudaFreeHost(h->h_ctrl);
   if (h->h_stop) cudaFreeHost(h->h_stop);
   if (h->h_kept) cudaFreeHost(h->h_kept);
+  if (h->h_med) cudaFreeHost(h->h_med);
   for (auto e : h->iter_events) cudaEventDestroy(e);
   for (auto e : h->prof_events) cudaEventDestroy(e);
   for (int i = 0; i < 4; i++) if (h->ev[i]) cudaEventDestroy(h->ev[i]);
@@ -725,9 +732,11 @@ static int align_begin(svnicp_handle h, AlignState &S) {
   if (h->h_stop_cap < (size_t)I + 4) {
     if (h->h_stop) cudaFreeHost(h->h_stop);
     if (h->h_kept) cudaFreeHost(h->h_kept);
+    if (h->h_med) cudaFreeHost(h->h_med);
     h->h_stop_cap = (size_t)I + 4;
     CU(cudaMallocHost((void **)&h->h_stop, h->h_stop_cap * sizeof(int)));
     CU(cudaMallocHost((void **)&h->h_kept, h->h_stop_cap * sizeof(unsigned long long)));
+    CU(cudaMallocHost((void **)&h->h_med, h->h_stop_cap * sizeof(int32_t)));
   }
   while ((int)h->iter_events.size() < I + 1) {
     cudaEvent_t e;
@@ -736,8 +745,10 @@ static int align_begin(svnicp_handle h, AlignState &S) {
   }
   CU(h->history.ensure((size_t)(I > 0 ? I : 1) * 6 * h->P));
   CU(h->kept_hist.ensure((size_t)I + 2, true));
+  CU(h->med_path.ensure((size_t)I + 2));
   CU(cudaMemsetAsync(h->history.p, 0, (size_t)(I > 0 ? I : 1) * 6 * h->P * sizeof(float), st));  // SVGDICP.cpp:172-174
   CU(cudaMemsetAsync(h->kept_hist.p, 0, ((size_t)I + 2) * sizeof(unsigned long long), st));
+  CU(cudaMemsetAsync(h->med_path.p, 0xff, ((size_t)I + 2) * sizeof(int32_t), st));  // -1: no median computed
   CU(cudaMemsetAsync(h->misc.p, 0, 8 * sizeof(int), st));
   const bool svgd = S.svgd = h->class_type == SVNICP_CLASS_SVGDICP;
   // A scan may be run again without a fresh add_cloud (the reference keeps R_/t_ and rewrites history rows 0..I-1; SVGDICP
@@ -758,6 +769,7 @@ static int align_begin(svnicp_handle h, AlignState &S) {
     CU(cudaStreamSynchronize(st));
     memset(h->h_ctrl, 0, sizeof(Ctrl));
     memset(h->h_kept, 0, ((size_t)I + 2) * sizeof(unsigned long long));
+    memset(h->h_med, 0xff, ((size_t)I + 2) * sizeof(int32_t));
     h->iters_done = 0;
     h->enqueued_iters = 0;
     h->ms_setup = h->ms_iter = h->ms_epi = h->ms_total = 0;
@@ -820,6 +832,7 @@ static int align_begin(svnicp_handle h, AlignState &S) {
   sa.Hbar_inv = h->Hbar_inv.p; sa.hist = h->hist.p; sa.history = h->history.p; sa.ctrl = h->ctrl.p;
   sa.stats = h->stats.p; sa.particles = h->particles.p; sa.sm_count = h->sm_count;
   sa.kept_hist = h->kept_hist.p;
+  sa.med_path = h->med_path.p;
   if (svgd) sa.rec_stride = 0;  // one record buffer: k_head_* read buffer 0 whatever the iteration's parity
   sa.prep_scratch_d = h->prep_scratch_d.p;
   sa.prep_scratch_i = h->prep_scratch_i.p;
@@ -1053,6 +1066,7 @@ static int align_epilogue(svnicp_handle h, AlignState &S) {
   CU(cudaMemcpyAsync(h->h_particles, h->particles.p, (size_t)6 * h->P * sizeof(double), cudaMemcpyDeviceToHost, st));
   CU(cudaMemcpyAsync(h->h_ctrl, h->ctrl.p, sizeof(Ctrl), cudaMemcpyDeviceToHost, st));
   CU(cudaMemcpyAsync(h->h_kept, h->kept_hist.p, ((size_t)S.I + 2) * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+  CU(cudaMemcpyAsync(h->h_med, h->med_path.p, ((size_t)S.I + 2) * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
   CU(cudaEventRecord(h->ev[3], st));
   return SVNICP_OK;
 }
@@ -1323,6 +1337,14 @@ int svnicp_get_prune_stats(svnicp_handle h, double *out_mean_kept, int32_t *rows
       // SVNICP_FLAG_REUSE_STATS: fraction of rows pruned from the previous list instead of mean kept candidates (tuning aid)
       out_mean_kept[i] = (h->prm.flags & SVNICP_FLAG_REUSE_STATS) ? (double)(v >> 40) / den : (double)(v & ((1ull << 40) - 1ull)) / den;
     }
+  return SVNICP_OK;
+}
+
+int svnicp_get_median_paths(svnicp_handle h, int32_t *out, int32_t *rows) {
+  if (!h || !h->aligned) return fail(h, SVNICP_ERR_INVALID, "no scan yet");
+  const int I = h->prm.iterations;
+  if (rows) *rows = I;
+  if (out) memcpy(out, h->h_med, (size_t)I * sizeof(int32_t));
   return SVNICP_OK;
 }
 

@@ -135,6 +135,7 @@ struct SteinArgs {
   double *stats;     // [6 + 6 + 36] mean, var, cov
   double *particles; // [6][P]
   unsigned long long *kept_hist;  // [I] candidates kept by the prune pass per iteration (statistics)
+  int32_t *med_path;              // [I + 2] how k_head_* settled each iteration's median (MED_PATH_*; -1 = not computed)
   double *prep_scratch_d;         // [sm_count][12] per-CTA partial sums of the fused tail kernel
   int *prep_scratch_i;            // [PRUNE_BINS + 3] envelope / alpha / beta / NaN flag maxima (bit patterns)
   double *stamps;                 // [8] globaltimer stamps of k_tail's phases (tuning aid; null = off)

@@ -43,6 +43,11 @@ constexpr int HD_THREADS = 128;
 constexpr int HD_WARPS = HD_THREADS / 32;
 constexpr int HD_COLLECT_CAP = 4096;  // doubles staged in the 32 KB histogram buffer
 static_assert(HD_COLLECT_CAP * sizeof(double) <= MED_BINS * sizeof(unsigned), "collected values are staged in the histogram buffer");
+// how the median of an iteration was settled, recorded in SteinArgs::med_path[iter] (svnicp_get_median_paths)
+enum { MED_PATH_SORT = 0,      // k_head_small: sort of all pairs (P <= HD_SMALL_P)
+       MED_PATH_FAST = 1,      // k_head_fast1/2: linear histogram around the previous median, then the bin's values
+       MED_PATH_RADIX = 2,     // k_head_radix: no fast path this iteration (iteration 0, no usable previous median) or a window miss
+       MED_PATH_OVERFLOW = 3 };  // k_head_radix after the fast path found the bin but could not pick (more than HD_COLLECT_CAP values)
 
 __device__ __forceinline__ int hd_pass_bits(int s) { return s == 0 ? 11 : 13; }
 __device__ __forceinline__ int hd_bits_before(int s) { return s == 0 ? 0 : 11 + 13 * (s - 1); }
@@ -200,11 +205,15 @@ __device__ __forceinline__ void hd_sweep(const double *__restrict__ X, int P, in
         on[u] = j < P;
         double s = 0.0;
         if (on[u]) {
+          double df[6];
 #pragma unroll
-          for (int d = 0; d < 6; d++) {
-            const double df = xi[d] - X[d * P + j];
-            s += df * df;  // SVNICP.cpp:257-260
-          }
+          for (int d = 0; d < 6; d++) df[d] = xi[d] - X[d * P + j];
+          // SVNICP.cpp:257-260, rounding spelled out: this is what nvcc made of `s += df * df` from s = 0 (it fused the first
+          // square into the second), written as explicit fma so that the order cannot change with the compiler and the CPU
+          // oracle (oracle_pair_median_kernel_order) can restate the exact values the median is selected from
+          s = fma(df[0], df[0], df[1] * df[1]);
+#pragma unroll
+          for (int d = 2; d < 6; d++) s = fma(df[d], df[d], s);
         }
         d2[u] = s;
       }
@@ -304,6 +313,7 @@ __global__ void __launch_bounds__(HD_THREADS, 8) k_head_fast2(SteinArgs a) {
   if (hd_pick(s_list, n_c, (unsigned)(c->fast_rank >> 1), &s_val, &s_found, &median) && tid == 0) {
     c->bandwidth = median / log((double)(P + 1));  // SVNICP.cpp:262 (Q4)
     c->med_done = 1;
+    if (a.med_path) a.med_path[c->iter] = MED_PATH_FAST;
   }
 }
 
@@ -331,7 +341,11 @@ __global__ void __launch_bounds__(HD_THREADS, 8) k_head_radix(SteinArgs a, int s
   if (tid == 0) {
     c->sel_prefix[s + 1] = np;
     c->sel_rank[s + 1] = nr;
-    if (s == MED_PASSES - 1) c->bandwidth = __longlong_as_double((long long)np) / log((double)(P + 1));  // SVNICP.cpp:262 (Q4)
+    if (s == MED_PASSES - 1) {
+      c->bandwidth = __longlong_as_double((long long)np) / log((double)(P + 1));  // SVNICP.cpp:262 (Q4)
+      const bool miss = c->fast_bin == 0ull || c->fast_bin == (unsigned long long)(MED_BINS - 1);
+      if (a.med_path) a.med_path[c->iter] = miss ? MED_PATH_RADIX : MED_PATH_OVERFLOW;
+    }
   }
 }
 
@@ -405,6 +419,7 @@ __global__ void __launch_bounds__(HD_THREADS, 8) k_head_small(SteinArgs a, PeerT
     const unsigned long long rank0 = ((unsigned long long)P * (unsigned long long)P - 1ull) / 2ull;  // lower median of P^2 entries
     const unsigned long long key = rank0 < (unsigned long long)P ? 0ull : s_key[(rank0 - (unsigned long long)P) / 2ull];
     c->bandwidth = __longlong_as_double((long long)key) / log((double)(P + 1));  // SVNICP.cpp:262 (Q4)
+    if (a.med_path) a.med_path[it] = MED_PATH_SORT;
   }
 }
 

@@ -61,6 +61,23 @@ def test_no_cpu_fallback(lib):
         sv.SVNICP(sv.SteinICPParam(), np.zeros((6, 4)))
 
 
+def test_particle_count_limit(lib):
+    """P > 65535 is refused before any device work: the bandwidth median counts the P^2 pair distances in 32-bit histogram
+    bins, and 65536^2 = 2^32 wraps them.  65535 passes that check (it then fails only where there is no device)."""
+    hdr = open(os.path.join(ROOT, "include", "svnicp_b200.h")).read()
+    assert int(re.search(r"#define\s+SVNICP_MAX_PARTICLES\s+(\d+)", hdr).group(1)) == sv.MAX_PARTICLES == 65535
+    assert sv.MAX_PARTICLES ** 2 < 2 ** 32 <= (sv.MAX_PARTICLES + 1) ** 2
+    for cls in (sv.SVNICP, sv.SVGDICP):
+        with pytest.raises(sv.SvnIcpError, match="65536 exceeds 65535: the bandwidth median counts .* 32-bit histograms"):
+            cls(sv.SteinICPParam(iterations=1), np.zeros((6, 65536)))
+    with pytest.raises(sv.SvnIcpError, match="exceeds 65535"):
+        sv.SVNICPBatch(sv.SteinICPParam(iterations=1), np.zeros((1, 6, 70000)))
+    try:
+        sv.SVNICP(sv.SteinICPParam(iterations=1), np.zeros((6, 65535))).close()
+    except sv.SvnIcpError as err:
+        assert "exceeds" not in str(err) and "no CUDA device" in str(err)
+
+
 def test_particle_initialisers(lib):
     """initialize_particles / _gaussian (ICPUtils.cpp:45-75): bounds, clamping, P == 1 -> zeros, determinism."""
     ub = np.array([0.3, 0.2, 0.1, 0.004, 0.004, 0.012])
