@@ -11,7 +11,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "libsvnicp_b200.so")
 SOURCES = ["cand_build.cu", "iter_kernels.cu", "stein_kernels.cu", "tail2.cu", "svgd_class.cu", "eval_kernels.cu", "voxel_map.cu", "preprocess.cu", "capi.cu"]
-HEADERS = ["common.cuh", "kernels.h", "ptx.cuh", os.path.join("..", "..", "include", "svnicp_b200.h")]
+HEADERS = ["block_scan.cuh", "common.cuh", "kernels.h", "ptx.cuh", "voxel_hash.cuh", os.path.join("..", "..", "include", "svnicp_b200.h")]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 # extra -D switches for A/B builds (e.g. SVNICP_NVCC_DEFS="-DSVN_GN_ACC2_FP32 -DSVN_GN_MINBLOCKS=3")
 EXTRA = os.environ.get("SVNICP_NVCC_DEFS", "").split()

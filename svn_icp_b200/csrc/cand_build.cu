@@ -14,12 +14,13 @@
 // Documented difference to the reference: slot ORDER (the reference leaves MinK replacement order,
 // mink.cuh:62-83); parity is therefore stated on global map indices, ties between exactly equal
 // fp32 distances go to the earlier slot of OUR order (see DESIGN.md "tie-break").
+#include "block_scan.cuh"
 #include "common.cuh"
 #include "kernels.h"
+#include "voxel_hash.cuh"
 
 namespace svn {
 
-constexpr unsigned long long EMPTY_KEY = 0xffffffffffffffffull;
 constexpr int RING_MAX = 6;
 constexpr int KNN_WARPS = 4;
 #ifndef SVN_KNN_CAP
@@ -38,16 +39,6 @@ struct Ent {
 };
 
 __device__ __forceinline__ int cell_of(double x, double inv_cell) { return (int)floor(x * inv_cell); }
-__device__ __forceinline__ unsigned long long pack_key(int cx, int cy, int cz) {
-  return ((unsigned long long)(unsigned)(cx + (1 << 20)) & 0x1fffffull) << 42 |
-         ((unsigned long long)(unsigned)(cy + (1 << 20)) & 0x1fffffull) << 21 |
-         ((unsigned long long)(unsigned)(cz + (1 << 20)) & 0x1fffffull);
-}
-__device__ __forceinline__ unsigned hash_key(unsigned long long k) {
-  k ^= k >> 33; k *= 0xff51afd7ed558ccdull; k ^= k >> 33; k *= 0xc4ceb9fe1a85ec53ull; k ^= k >> 33;
-  return (unsigned)k;
-}
-
 // q0 = R0 s + t0 (SVGDICP.cpp:204) in the fma order shared with oracle_transform_q0; sp = fp32(R0 s).
 __global__ void k_q0(const double *__restrict__ src, int n_s, ScanConst sc, double *__restrict__ q0, float4 *__restrict__ sp,
                      int n_pad) {
@@ -76,15 +67,11 @@ __global__ void k_grid_count(const double *__restrict__ tgt, int n_t, double inv
                              int *pt_slot, unsigned mask) {
   const int j = blockIdx.x * blockDim.x + threadIdx.x;
   if (j >= n_t) return;
-  const unsigned long long key = pack_key(cell_of(tgt[3 * j], inv_cell), cell_of(tgt[3 * j + 1], inv_cell), cell_of(tgt[3 * j + 2], inv_cell));
-  unsigned slot = hash_key(key) & mask;
-  while (true) {
-    const unsigned long long prev = atomicCAS(&keys[slot], EMPTY_KEY, key);
-    if (prev == EMPTY_KEY || prev == key) break;
-    slot = (slot + 1) & mask;
-  }
+  const unsigned long long key = pack_voxel_key(cell_of(tgt[3 * j], inv_cell), cell_of(tgt[3 * j + 1], inv_cell), cell_of(tgt[3 * j + 2], inv_cell));
+  bool created;
+  const int slot = hash_insert(keys, mask, key, &created);  // never -1: table_size >= 2 n_t
   atomicAdd(&counts[slot], 1);
-  pt_slot[j] = (int)slot;
+  pt_slot[j] = slot;
 }
 
 __global__ void k_grid_alloc(const int *counts, int *starts, int table_size, int *cursor) {
@@ -104,16 +91,6 @@ __global__ void k_grid_scatter(const double *__restrict__ tgt, int n_t, const in
   sxyz[3 * pos + 1] = tgt[3 * j + 1];
   sxyz[3 * pos + 2] = tgt[3 * j + 2];
   sidx[pos] = j;
-}
-
-__device__ __forceinline__ int find_cell(unsigned long long key, const unsigned long long *__restrict__ keys, unsigned mask) {
-  unsigned slot = hash_key(key) & mask;
-  while (true) {
-    const unsigned long long k = keys[slot];
-    if (k == key) return (int)slot;
-    if (k == EMPTY_KEY) return -1;
-    slot = (slot + 1) & mask;
-  }
 }
 
 __device__ __forceinline__ bool ent_less(const Ent &a, const Ent &b) { return a.d < b.d || (a.d == b.d && a.idx < b.idx); }
@@ -230,12 +207,7 @@ __device__ int warp_cut(Ent *buf, int count, int K, double *cut_scale, int *cut_
   for (int i = lane; i < count; i += 32) atomicAdd(&hist[cut_bin_of(buf[i].d, scale)], 1);
   __syncwarp();
   const int h0 = hist[2 * lane], h1 = hist[2 * lane + 1];
-  int incl = h0 + h1;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1) {
-    const int v = __shfl_up_sync(0xffffffffu, incl, o);
-    if (lane >= o) incl += v;
-  }
+  const int incl = warp_inclusive_scan(h0 + h1);
   const int before = incl - h0 - h1;
   int tbin = KNN_BINS;
   if (before < K && before + h0 >= K) tbin = 2 * lane;
@@ -300,16 +272,11 @@ k_knn(const double *__restrict__ q0, int row_lo, int row_hi, const double *__res
           const int dz = ci / (side * side) - r, dy = (ci / side) % side - r, dx = ci % side - r;
           const int ch = max(abs(dx), max(abs(dy), abs(dz)));
           if (ch == r) {
-            const int slot = find_cell(pack_key(c0[0] + dx, c0[1] + dy, c0[2] + dz), keys, mask);
+            const int slot = hash_find(keys, mask, pack_voxel_key(c0[0] + dx, c0[1] + dy, c0[2] + dz));
             if (slot >= 0) { st = starts[slot]; cn = counts[slot]; }
           }
         }
-        int incl = cn;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-          const int v = __shfl_up_sync(0xffffffffu, incl, o);
-          if (lane >= o) incl += v;
-        }
+        const int incl = warp_inclusive_scan(cn);
         const int total = __shfl_sync(0xffffffffu, incl, 31);
         s_start[warp][lane] = st;
         s_excl[warp][lane] = incl - cn;
@@ -393,12 +360,7 @@ k_knn(const double *__restrict__ q0, int row_lo, int row_hi, const double *__res
       __syncwarp();
       // inclusive prefix over the 64 bins (2 per lane)
       const int h0 = hist[2 * lane], h1 = hist[2 * lane + 1];
-      int incl = h0 + h1;
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) {
-        const int v = __shfl_up_sync(0xffffffffu, incl, o);
-        if (lane >= o) incl += v;
-      }
+      const int incl = warp_inclusive_scan(h0 + h1);
       const int before = incl - h0 - h1;
       int tbin = KNN_BINS;  // first bin whose inclusive count reaches K
       if (before < K && before + h0 >= K) tbin = 2 * lane;

@@ -23,51 +23,12 @@
 #include <string>
 
 #include "../../include/svnicp_b200.h"
+#include "block_scan.cuh"
+#include "voxel_hash.cuh"
 
 namespace {
 
-constexpr int PB = 1024;  // scan block
-constexpr unsigned long long EMPTY = ~0ull;
-
-__device__ int pre_block_excl_scan(int v, int *total) {
-  __shared__ int s_w[32];
-  __shared__ int s_tot;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  int incl = v;
-  for (int o = 1; o < 32; o <<= 1) {
-    const int u = __shfl_up_sync(0xffffffffu, incl, o);
-    if (lane >= o) incl += u;
-  }
-  if (lane == 31) s_w[warp] = incl;
-  __syncthreads();
-  if (warp == 0) {
-    int x = s_w[lane], xi = x;
-    for (int o = 1; o < 32; o <<= 1) {
-      const int u = __shfl_up_sync(0xffffffffu, xi, o);
-      if (lane >= o) xi += u;
-    }
-    s_w[lane] = xi - x;
-    if (lane == 31) s_tot = xi;
-  }
-  __syncthreads();
-  const int r = s_w[warp] + incl - v;
-  if (total) *total = s_tot;
-  __syncthreads();
-  return r;
-}
-
-__global__ void __launch_bounds__(PB) k_pre_scan_sums(int *sums, int n_blocks, long long *total_out) {
-  int carry = 0;
-  for (int base = 0; base < n_blocks; base += PB) {
-    const int i = base + threadIdx.x;
-    const int v = i < n_blocks ? sums[i] : 0;
-    int tot;
-    const int ex = pre_block_excl_scan(v, &tot);
-    if (i < n_blocks) sums[i] = carry + ex;
-    carry += tot;
-  }
-  if (threadIdx.x == 0) *total_out = carry;
-}
+constexpr int PB = svn::SCAN_BLOCK;  // threads per block of every kernel here (the block scans need SCAN_BLOCK)
 
 __device__ __forceinline__ bool crop_keep(const float *p, double lo2, double hi2, float *norm_out) {
   // :697, evaluated as the host compiler does for a baseline x86-64 build: three products, two adds, no fused multiply-add
@@ -77,43 +38,24 @@ __device__ __forceinline__ bool crop_keep(const float *p, double lo2, double hi2
 }
 
 __global__ void __launch_bounds__(PB) k_crop_count(const float *xyz, int n, double lo2, double hi2, int *sums, unsigned *max_bits) {
-  __shared__ int s_w[32];
   const int i = blockIdx.x * PB + threadIdx.x;
   int c = 0;
   float norm = 0.f;
   if (i < n) c = crop_keep(xyz + 3 * (size_t)i, lo2, hi2, &norm) ? 1 : 0;
   // max of the (non-negative) float norms: their bit patterns order like the values; NaN (bits above +inf) propagates as in a max
   unsigned nb = (i < n) ? __float_as_uint(norm) : 0u;
-  for (int o = 16; o > 0; o >>= 1) {
-    c += __shfl_xor_sync(0xffffffffu, c, o);
-    nb = max(nb, __shfl_xor_sync(0xffffffffu, nb, o));
-  }
-  if ((threadIdx.x & 31) == 0) { s_w[threadIdx.x >> 5] = c; atomicMax(max_bits, nb); }
-  __syncthreads();
-  if (threadIdx.x < 32) {
-    int v = s_w[threadIdx.x];
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    if (threadIdx.x == 0) sums[blockIdx.x] = v;
-  }
+  for (int o = 16; o > 0; o >>= 1) nb = max(nb, __shfl_xor_sync(0xffffffffu, nb, o));
+  if ((threadIdx.x & 31) == 0) atomicMax(max_bits, nb);
+  svn::block_sum_int(c, &sums[blockIdx.x]);
 }
 
 __global__ void __launch_bounds__(PB) k_crop_emit(const float *xyz, int n, double lo2, double hi2, const int *offs, float *out) {
   const int i = blockIdx.x * PB + threadIdx.x;
   float norm;
   const int c = (i < n && crop_keep(xyz + 3 * (size_t)i, lo2, hi2, &norm)) ? 1 : 0;
-  const int off = offs[blockIdx.x] + pre_block_excl_scan(c, nullptr);
+  const int off = offs[blockIdx.x] + svn::block_exclusive_scan<int>(c, nullptr);
   if (c)
     for (int k = 0; k < 3; k++) out[3 * (size_t)off + k] = xyz[3 * (size_t)i + k];
-}
-
-__device__ __forceinline__ unsigned long long leaf_key(int i, int j, int k) {
-  const unsigned long long B = 1ull << 20;
-  return ((unsigned long long)(i + (long long)B) & 0x1FFFFFull) | (((unsigned long long)(j + (long long)B) & 0x1FFFFFull) << 21) |
-         (((unsigned long long)(k + (long long)B) & 0x1FFFFFull) << 42);
-}
-__device__ __forceinline__ unsigned leaf_hash(unsigned long long k) {
-  k ^= k >> 33; k *= 0xff51afd7ed558ccdull; k ^= k >> 33; k *= 0xc4ceb9fe1a85ec53ull; k ^= k >> 33;
-  return (unsigned)k;
 }
 
 // first pass of UniformSampling::applyFilter: every point votes for its leaf with (distance bits, index)
@@ -127,39 +69,21 @@ __global__ void k_us_vote(const float *xyz, int n, float inv_leaf, unsigned long
   // NaN points vote last
   const float diff = __fadd_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)), __fmul_rn(dz, dz));
   const unsigned long long vote = ((unsigned long long)__float_as_uint(diff) << 32) | (unsigned)p;
-  const unsigned long long key = leaf_key(i, j, k);
-  unsigned slot = leaf_hash(key) & mask;
-  for (;;) {
-    const unsigned long long cur = keys[slot];
-    if (cur == key) break;
-    if (cur == EMPTY) {
-      const unsigned long long old = atomicCAS(&keys[slot], EMPTY, key);
-      if (old == EMPTY || old == key) break;
-    }
-    slot = (slot + 1) & mask;
-  }
+  bool created;
+  const int slot = svn::hash_insert(keys, mask, svn::pack_voxel_key(i, j, k), &created);  // never -1: slots >= 2 n
   atomicMin(&best[slot], vote);  // smaller distance wins; equal distances: the earlier point (strict '<' in cloud order)
 }
 
 __global__ void __launch_bounds__(PB) k_us_count(const unsigned long long *keys, int slots, int *sums) {
-  __shared__ int s_w[32];
   const int s = blockIdx.x * PB + threadIdx.x;
-  int c = (s < slots && keys[s] != EMPTY) ? 1 : 0;
-  for (int o = 16; o > 0; o >>= 1) c += __shfl_xor_sync(0xffffffffu, c, o);
-  if ((threadIdx.x & 31) == 0) s_w[threadIdx.x >> 5] = c;
-  __syncthreads();
-  if (threadIdx.x < 32) {
-    int v = s_w[threadIdx.x];
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    if (threadIdx.x == 0) sums[blockIdx.x] = v;
-  }
+  svn::block_sum_int((s < slots && keys[s] != svn::EMPTY_KEY) ? 1 : 0, &sums[blockIdx.x]);
 }
 
 __global__ void __launch_bounds__(PB) k_us_emit(const float *xyz, const unsigned long long *keys, const unsigned long long *best, int slots,
                                                 const int *offs, float *out) {
   const int s = blockIdx.x * PB + threadIdx.x;
-  const int c = (s < slots && keys[s] != EMPTY) ? 1 : 0;
-  const int off = offs[blockIdx.x] + pre_block_excl_scan(c, nullptr);
+  const int c = (s < slots && keys[s] != svn::EMPTY_KEY) ? 1 : 0;
+  const int off = offs[blockIdx.x] + svn::block_exclusive_scan<int>(c, nullptr);
   if (c) {
     const unsigned p = (unsigned)(best[s] & 0xFFFFFFFFull);
     for (int k = 0; k < 3; k++) out[3 * (size_t)off + k] = xyz[3 * (size_t)p + k];
@@ -424,7 +348,7 @@ int svnicp_pre_crop(svnicp_pre p, const float *xyz, int64_t n, int on_device, do
   const double lo2 = min_range * min_range, hi2 = max_range * max_range;
   if (n > 0) {
     k_crop_count<<<nb, PB, 0, p->stream>>>(src, (int)n, lo2, hi2, p->sums, p->d_max);
-    k_pre_scan_sums<<<1, PB, 0, p->stream>>>(p->sums, nb, p->d_total);
+    svn::k_scan_block_sums<int><<<1, PB, 0, p->stream>>>(p->sums, nb, p->d_total);
     k_crop_emit<<<nb, PB, 0, p->stream>>>(src, (int)n, lo2, hi2, p->sums, p->buf[ob]);
     PCU(cudaGetLastError());
   }
@@ -459,7 +383,7 @@ int svnicp_pre_downsample_uniform(svnicp_pre p, const float *xyz, int64_t n, int
     const int nb = (int)((p->slots + PB - 1) / PB);
     k_us_vote<<<(unsigned)((n + 255) / 256), 256, 0, p->stream>>>(src, (int)n, inv_leaf, p->keys, p->best, (unsigned)(p->slots - 1));
     k_us_count<<<nb, PB, 0, p->stream>>>(p->keys, (int)p->slots, p->sums);
-    k_pre_scan_sums<<<1, PB, 0, p->stream>>>(p->sums, nb, p->d_total);
+    svn::k_scan_block_sums<int><<<1, PB, 0, p->stream>>>(p->sums, nb, p->d_total);
     k_us_emit<<<nb, PB, 0, p->stream>>>(src, p->keys, p->best, (int)p->slots, p->sums, p->buf[ob]);
     PCU(cudaGetLastError());
   }

@@ -16,6 +16,7 @@
 // rank's record buffer over NVLink (PeerTable, common.cuh), followed by a sequence number in the peer's flag block; k_tail /
 // k_head spin on their local flags.  Records are double buffered by iteration parity, which is what makes the exchange
 // safe without a second handshake (see DESIGN.md section 5).  No NCCL call on the per-iteration path.
+#include "block_scan.cuh"
 #include "common.cuh"
 #include "kernels.h"
 #include "ptx.cuh"
@@ -69,12 +70,7 @@ __device__ void hd_select(const unsigned *hist, unsigned long long prefix_in, un
 #pragma unroll
     for (int u = 0; u < 16; u++) loc += v[u];
   }
-  unsigned long long incl = loc;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1) {
-    const unsigned long long v = __shfl_up_sync(0xffffffffu, incl, o);
-    if (lane >= o) incl += v;
-  }
+  const unsigned long long incl = warp_inclusive_scan(loc);
   if (lane == 31) s_warp[warp] = incl;
   if (tid == 0) { s_res[0] = (prefix_in << bits) | (unsigned long long)(nbins - 1); s_res[1] = 0ull; }
   __syncthreads();

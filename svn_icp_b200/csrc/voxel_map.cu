@@ -11,8 +11,8 @@
 // "Arrival order" is made deterministic on the GPU by ranking the points of one AddPointCloud batch by their index in the
 // cloud (what the reference's sequential loop does): pass 1 links every point into its voxel's list and elects the lowest
 // index as the voxel's walker; pass 2 lets the walker keep the (cap - count) lowest indices, ascending.
-// The table is open addressing (linear probing) over packed 3x21-bit voxel indices; RemoveFar rebuilds into the twin table
-// (no tombstones).  Point output order of GetMap is slot order: arbitrary like the reference's robin_map iteration.
+// The table is the voxel hash of voxel_hash.cuh (open addressing over packed 3x21-bit voxel indices); RemoveFar rebuilds into
+// the twin table (no tombstones).  Point output order of GetMap is slot order: arbitrary like the reference's robin_map iteration.
 //
 // svnicp_map_evaluate (DESIGN.md section 10b) scores a scan at caller-given poses against the table itself: an exact
 // nearest-map-point search per (source point, pose) by read-only probes of the same hash (k_map_eval), then the fixed-order
@@ -32,13 +32,17 @@
 #include <vector>
 
 #include "../../include/svnicp_b200.h"
+#include "block_scan.cuh"
 #include "kernels.h"
+#include "voxel_hash.cuh"
 
 namespace {
 
-constexpr unsigned long long EMPTY_KEY = ~0ull;
+using svn::EMPTY_KEY;
+using svn::SCAN_BLOCK;
+using svn::block_exclusive_scan;
+
 constexpr int MAX_CAP = 32;
-constexpr int SCAN_BLOCK = 1024;
 
 struct MapTable {
   unsigned long long *keys;  // [slots]
@@ -51,42 +55,14 @@ struct MapDev {
   int *head, *walker;        // [slots] per-batch list head / elected walker (restored to -1 / INT_MAX after every batch)
   long long *counters;       // [0] voxels, [1] points, [2] far voxels (scratch), [3] dropped (table full)
   int slots_mask, cap;
-  float inv_guard;           // unused
   float voxel_size_f;
 };
-
-__device__ __forceinline__ unsigned long long pack_key(int vx, int vy, int vz) {
-  const unsigned long long B = 1ull << 20;
-  return ((unsigned long long)(vx + (long long)B) & 0x1FFFFFull) | (((unsigned long long)(vy + (long long)B) & 0x1FFFFFull) << 21) |
-         (((unsigned long long)(vz + (long long)B) & 0x1FFFFFull) << 42);
-}
-__device__ __forceinline__ unsigned hash_key(unsigned long long k) {
-  k ^= k >> 33; k *= 0xff51afd7ed558ccdull; k ^= k >> 33; k *= 0xc4ceb9fe1a85ec53ull; k ^= k >> 33;
-  return (unsigned)k;
-}
 
 // The voxel a stored point belongs to (VoxelHashMap.cpp:30): (int)(p / float(voxel_size)) per axis -- truncation toward zero,
 // so (-v, v) is voxel 0, and NaN converts to 0 -- packed.  k_map_insert_link files points with it and svnicp_map_import checks
 // membership with it, so the two cannot drift.
 __device__ __forceinline__ unsigned long long voxel_key(const float q[3], float voxel_size_f) {
-  return pack_key((int)(q[0] / voxel_size_f), (int)(q[1] / voxel_size_f), (int)(q[2] / voxel_size_f));
-}
-
-// find-or-create; returns the slot or -1 when the table is full
-__device__ int find_or_create(const MapDev &m, unsigned long long key, bool *created) {
-  unsigned slot = hash_key(key) & (unsigned)m.slots_mask;
-  *created = false;
-  for (int probe = 0; probe <= m.slots_mask; probe++) {
-    const unsigned long long k = m.tab.keys[slot];
-    if (k == key) return (int)slot;
-    if (k == EMPTY_KEY) {
-      const unsigned long long old = atomicCAS(&m.tab.keys[slot], EMPTY_KEY, key);
-      if (old == EMPTY_KEY) { *created = true; return (int)slot; }
-      if (old == key) return (int)slot;
-    }
-    slot = (slot + 1) & (unsigned)m.slots_mask;
-  }
-  return -1;
+  return svn::pack_voxel_key((int)(q[0] / voxel_size_f), (int)(q[1] / voxel_size_f), (int)(q[2] / voxel_size_f));
 }
 
 // pass 1: transform (VoxelHashMap.cpp:23-26), voxel index (:30), slot lookup, link into the voxel's batch list
@@ -101,7 +77,7 @@ __global__ void k_map_insert_link(MapDev m, const T *xyz, int n, const double *R
 #pragma unroll
   for (int r = 0; r < 3; r++) wxyz[3 * (size_t)i + r] = q[r];
   bool created;
-  const int slot = find_or_create(m, voxel_key(q, m.voxel_size_f), &created);
+  const int slot = svn::hash_insert(m.tab.keys, (unsigned)m.slots_mask, voxel_key(q, m.voxel_size_f), &created);
   pt_slot[i] = slot;
   if (slot < 0) { atomicAdd((unsigned long long *)&m.counters[3], 1ull); return; }
   if (created) atomicAdd((unsigned long long *)&m.counters[0], 1ull);
@@ -167,7 +143,7 @@ __global__ void k_map_rebuild(MapDev old, MapDev neu, const double *pos, double 
   int slot = 0;
   if (lane == 0) {
     bool created;
-    slot = find_or_create(neu, key, &created);
+    slot = svn::hash_insert(neu.tab.keys, (unsigned)neu.slots_mask, key, &created);
     if (slot >= 0) {
       neu.tab.count[slot] = cnt;
       atomicAdd((unsigned long long *)&neu.counters[0], 1ull);
@@ -190,60 +166,7 @@ __device__ __forceinline__ int slot_emit_count(const MapDev &m, int s, const dou
 }
 
 __global__ void __launch_bounds__(SCAN_BLOCK) k_getmap_count(MapDev m, const double *pos, double r2, int all, int *block_sums) {
-  __shared__ int s_w[32];
-  const int s = blockIdx.x * SCAN_BLOCK + threadIdx.x;
-  int c = slot_emit_count(m, s, pos, r2, all);
-  for (int o = 16; o > 0; o >>= 1) c += __shfl_xor_sync(0xffffffffu, c, o);
-  if ((threadIdx.x & 31) == 0) s_w[threadIdx.x >> 5] = c;
-  __syncthreads();
-  if (threadIdx.x < 32) {
-    int v = s_w[threadIdx.x];
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    if (threadIdx.x == 0) block_sums[blockIdx.x] = v;
-  }
-}
-
-template <typename T>
-__device__ T block_exclusive_scan(T v, T *total) {  // SCAN_BLOCK threads; int, or long long for point offsets
-  __shared__ T s_w[32];
-  __shared__ T s_tot;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  T incl = v;
-  for (int o = 1; o < 32; o <<= 1) {
-    const T u = __shfl_up_sync(0xffffffffu, incl, o);
-    if (lane >= o) incl += u;
-  }
-  if (lane == 31) s_w[warp] = incl;
-  __syncthreads();
-  if (warp == 0) {
-    T x = s_w[lane], xi = x;
-    for (int o = 1; o < 32; o <<= 1) {
-      const T u = __shfl_up_sync(0xffffffffu, xi, o);
-      if (lane >= o) xi += u;
-    }
-    s_w[lane] = xi - x;
-    if (lane == 31) s_tot = xi;
-  }
-  __syncthreads();
-  const T r = s_w[warp] + incl - v;
-  if (total) *total = s_tot;
-  __syncthreads();
-  return r;
-}
-
-template <typename T>
-__global__ void __launch_bounds__(SCAN_BLOCK) k_getmap_scan(T *block_sums, int n_blocks, long long *total_out) {
-  // one block, looping over the sums SCAN_BLOCK at a time (GetMap: n_blocks <= SCAN_BLOCK * 8)
-  T carry = 0;
-  for (int base = 0; base < n_blocks; base += SCAN_BLOCK) {
-    const int i = base + threadIdx.x;
-    const T v = i < n_blocks ? block_sums[i] : 0;
-    T tot;
-    const T ex = block_exclusive_scan(v, &tot);
-    if (i < n_blocks) block_sums[i] = carry + ex;
-    carry += tot;
-  }
-  if (threadIdx.x == 0) *total_out = carry;
+  svn::block_sum_int(slot_emit_count(m, blockIdx.x * SCAN_BLOCK + threadIdx.x, pos, r2, all), &block_sums[blockIdx.x]);
 }
 
 __global__ void __launch_bounds__(SCAN_BLOCK) k_getmap_emit(MapDev m, const double *pos, double r2, int all, const int *block_offs, double *out) {
@@ -402,7 +325,7 @@ __device__ __forceinline__ void snap_flag(unsigned long long *err, long long i, 
   atomicMin(err, ((unsigned long long)i << 3) | (unsigned long long)reason);
 }
 
-// One warp per snapshot voxel into the (cleared) twin table: find_or_create, count, points; every point's membership is
+// One warp per snapshot voxel into the (cleared) twin table: hash_insert, count, points; every point's membership is
 // checked with voxel_key.  words: [0] lowest (voxel << 3 | reason) of the count and index errors, [2] voxels refused by a full
 // table, [3] lowest of the duplicate and membership errors (meaningful only when the counts are valid and sum to N, since the
 // point offsets come from them).  Each voxel's slot goes to slot_of (-1 when not inserted) and the lowest voxel index per slot
@@ -416,14 +339,14 @@ __global__ void k_map_import(MapDev neu, const int32_t *voxels, const int32_t *c
   const int lim = 1 << 20;
   const bool count_ok = c >= 1 && c <= neu.cap;
   const bool index_ok = vx >= -lim && vx < lim && vy >= -lim && vy < lim && vz >= -lim && vz < lim;
-  const unsigned long long key = pack_key(vx, vy, vz);
+  const unsigned long long key = svn::pack_voxel_key(vx, vy, vz);
   int slot = -1;
   if (lane == 0) {
     if (!count_ok) snap_flag(words, i, SNAP_BAD_COUNT);
     else if (!index_ok) snap_flag(words, i, SNAP_BAD_INDEX);
     else {
       bool created;
-      slot = find_or_create(neu, key, &created);
+      slot = svn::hash_insert(neu.tab.keys, (unsigned)neu.slots_mask, key, &created);
       if (slot < 0) atomicAdd(&words[2], 1ull);
       else {
         atomicMin(&neu.walker[slot], (int)i);
@@ -471,14 +394,8 @@ constexpr double MEV_MARGIN = 1.0 + 1e-12;       // search radii exceed sqrt(d^2
 // Read-only probe: the slot holding key, or -1 when the voxel is absent or holds no point.  There are no tombstones (far voxels
 // leave by a rebuild into the twin table), so the walk may stop at the first empty slot.
 __device__ __forceinline__ int map_find(const MapTable &t, int slots_mask, unsigned long long key) {
-  unsigned slot = hash_key(key) & (unsigned)slots_mask;
-  for (int probe = 0; probe <= slots_mask; probe++) {
-    const unsigned long long k = __ldg(t.keys + slot);
-    if (k == key) return __ldg(t.count + slot) > 0 ? (int)slot : -1;
-    if (k == EMPTY_KEY) return -1;
-    slot = (slot + 1) & (unsigned)slots_mask;
-  }
-  return -1;
+  const int slot = svn::hash_find(t.keys, (unsigned)slots_mask, key);
+  return slot < 0 || __ldg(t.count + slot) > 0 ? slot : -1;
 }
 
 // Per pose of a block, x = [t ; omega] relative to T0 = (R0, t0): R~ = R0 Exp(omega), t~ = t0 + R0 t -> Rt [MB][12], and
@@ -553,7 +470,7 @@ __device__ __forceinline__ void map_nearest(const MapDev &m, double r, NearestSt
   int own[3];
 #pragma unroll
   for (int a = 0; a < 3; a++) own[a] = (int)__fdiv_rn(__double2float_rn(s.q[a]), v);
-  int slot = map_find(m.tab, m.slots_mask, pack_key(own[0], own[1], own[2]));
+  int slot = map_find(m.tab, m.slots_mask, svn::pack_voxel_key(own[0], own[1], own[2]));
   if (slot >= 0) visit_slot(m.tab, m.cap, slot, s);
   if (s.found) {
     const double rb = fmin(r, sqrt(s.bd) * MEV_MARGIN);
@@ -564,7 +481,7 @@ __device__ __forceinline__ void map_nearest(const MapDev &m, double r, NearestSt
     for (int y = lo[1]; y <= hi[1]; y++)
       for (int x = lo[0]; x <= hi[0]; x++) {
         if (x == own[0] && y == own[1] && z == own[2]) continue;
-        slot = map_find(m.tab, m.slots_mask, pack_key(x, y, z));
+        slot = map_find(m.tab, m.slots_mask, svn::pack_voxel_key(x, y, z));
         if (slot >= 0) visit_slot(m.tab, m.cap, slot, s);
       }
 }
@@ -705,7 +622,7 @@ static MapDev dev_view(svnicp_map m, int which) {
   MapDev d;
   d.tab = m->tab[which];
   d.head = m->head; d.walker = m->walker; d.counters = m->counters;
-  d.slots_mask = (int)(m->slots - 1); d.cap = m->cap; d.inv_guard = 0.f;
+  d.slots_mask = (int)(m->slots - 1); d.cap = m->cap;
   d.voxel_size_f = (float)m->voxel_size;  // Eigen promotes the double scalar to the vector's float (VoxelHashMap.cpp:30)
   return d;
 }
@@ -881,7 +798,7 @@ int svnicp_map_get(svnicp_map m, const double position[3], double max_range, con
   const int n_blocks = (int)((m->slots + SCAN_BLOCK - 1) / SCAN_BLOCK);
   const double r2 = max_range * max_range;
   k_getmap_count<<<n_blocks, SCAN_BLOCK, 0, m->stream>>>(d, m->d_pose + 12, r2, all, m->block_sums);
-  k_getmap_scan<int><<<1, SCAN_BLOCK, 0, m->stream>>>(m->block_sums, n_blocks, m->counters + 2);
+  svn::k_scan_block_sums<int><<<1, SCAN_BLOCK, 0, m->stream>>>(m->block_sums, n_blocks, m->counters + 2);
   k_getmap_emit<<<n_blocks, SCAN_BLOCK, 0, m->stream>>>(d, m->d_pose + 12, r2, all, m->block_sums, m->out);
   MCU(cudaGetLastError());
   int rc = sync_counters(m);
@@ -1015,7 +932,7 @@ static void launch_point_offsets(svnicp_map m, const int32_t *counts, const int 
   const int nb = (int)((V + SCAN_BLOCK - 1) / SCAN_BLOCK);
   long long *psum = (long long *)m->sn[SN_PSUM], *off = (long long *)m->sn[SN_OFF];
   k_snap_pts_count<<<nb, SCAN_BLOCK, 0, m->stream>>>(counts, slots, tab_count, m->cap, V, psum);
-  k_getmap_scan<long long><<<1, SCAN_BLOCK, 0, m->stream>>>(psum, nb, total);
+  svn::k_scan_block_sums<long long><<<1, SCAN_BLOCK, 0, m->stream>>>(psum, nb, total);
   k_snap_pts_offsets<<<nb, SCAN_BLOCK, 0, m->stream>>>(counts, slots, tab_count, m->cap, V, psum, off);
 }
 
@@ -1048,11 +965,11 @@ extern "C" int svnicp_map_export(svnicp_map m, int32_t *voxels, int32_t *counts,
   MCU(cudaMemsetAsync(words, 0, 4 * sizeof(long long), st));
   const MapDev d = dev_view(m, m->cur);
   k_snap_count<<<slot_blocks, SCAN_BLOCK, 0, st>>>(d, hist);
-  k_getmap_scan<int><<<1, SCAN_BLOCK, 0, st>>>(hist, slot_blocks, words);
+  svn::k_scan_block_sums<int><<<1, SCAN_BLOCK, 0, st>>>(hist, slot_blocks, words);
   k_snap_emit<<<slot_blocks, SCAN_BLOCK, 0, st>>>(d, hist, V, key[0], slot[0]);
   for (int shift = 0, a = 0; shift < CANON_BITS; shift += RADIX_BITS, a ^= 1) {
     k_radix_hist<<<n_tiles, RADIX_THREADS, 0, st>>>(key[a], (int)V, shift, n_tiles, hist);
-    k_getmap_scan<int><<<1, SCAN_BLOCK, 0, st>>>(hist, RADIX_DIGITS * n_tiles, words + 3);
+    svn::k_scan_block_sums<int><<<1, SCAN_BLOCK, 0, st>>>(hist, RADIX_DIGITS * n_tiles, words + 3);
     k_radix_scatter<<<n_tiles, RADIX_THREADS, 0, st>>>(key[a], slot[a], key[a ^ 1], slot[a ^ 1], (int)V, shift, n_tiles, hist);
   }
   launch_point_offsets(m, nullptr, slot[0], d.tab.count, V, words + 1);
