@@ -272,6 +272,25 @@ int svnicp_map_size(svnicp_map m, int64_t *voxels, int64_t *points);
 int svnicp_map_evaluate(svnicp_map m, const void *source, int64_t n, int dtype_f64, int on_device, const double R0[9],
                         const double t0[3], int n_poses, const double *poses_6xM, double max_dist, double *out_stats,
                         double *out_H, double *out_b, uint8_t *out_mask, float *out_nearest);
+/* Exhaustive search of a scan against the map over a regular grid of poses (no reference counterpart): relocalisation,
+ * loop-closure checks, recovery from a lost track.  Pose convention, source, max_dist, the search-radius limit and the inlier
+ * test are those of svnicp_map_evaluate.
+ * Grid: axis a = 0..5 of x = [t ; omega] has counts[a] >= 1 values x_a(i) = ((double)i - 0.5 * (double)(counts[a] - 1)) * steps[a],
+ *   i = 0 .. counts[a]-1 (centred on T0; steps finite and >= 0).  M = prod(counts) <= 2^31 - 1.  Flat grid index
+ *   g = i0 + counts[0] * (i1 + counts[1] * (i2 + ...)), axis 0 (t_x) fastest.
+ * Score of a pose = its inlier count: source points with a stored map point at d^2 < max_dist -- the count svnicp_map_evaluate
+ *   returns for the same pose, bit for bit.
+ * Ranking: count descending, then g ascending (a total order: the result does not depend on scheduling or slot layout).
+ *   out_index [k] int64  the winners' g, best first
+ *   out_poses [6][k]     their grid values, to pass on to svnicp_map_evaluate or svnicp_set_initial_mean (through T0)
+ *   out_stats [k][3]     svnicp_map_evaluate's {count, fraction, RMSE} of each winner, bit for bit
+ *   out_counts [M] int32 (may be NULL)  the score of every grid pose, in g order
+ * Host outputs.  Blocking, on the map's stream; changes no state of the map.  SVNICP_ERR_INVALID: svnicp_map_evaluate's argument
+ * errors, null counts / steps / outputs, a count < 1, a negative or non-finite step, M > 2^31 - 1, top_k outside
+ * [1, min(M, 1024)]. */
+int svnicp_map_search(svnicp_map m, const void *source, int64_t n, int dtype_f64, int on_device, const double R0[9], const double t0[3],
+                      const int32_t counts[6], const double steps[6], double max_dist, int top_k, int64_t *out_index,
+                      double *out_poses_6xK, double *out_stats, int32_t *out_counts);
 /* Snapshot of the map's content (no reference counterpart), to save a map and restore it bit for bit with svnicp_map_import:
  *   voxels [V][3] int32  voxel indices (vx, vy, vz) in ascending lexicographic order
  *   counts [V]    int32  points per voxel, 1 <= count <= max_pointscount

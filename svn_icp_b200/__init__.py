@@ -95,8 +95,8 @@ EXPORTS = [
     "svnicp_get_median_paths", "svnicp_get_timing", "svnicp_get_slice", "svnicp_get_launch_count", "svnicp_set_profiling", "svnicp_get_phase_times",
     "svnicp_get_scan_info", "svnicp_get_tail_stamps", "svnicp_evaluate",
     "svnicp_map_create", "svnicp_map_destroy", "svnicp_map_last_error", "svnicp_map_clear", "svnicp_map_add_cloud", "svnicp_map_get",
-    "svnicp_map_download", "svnicp_map_size", "svnicp_map_evaluate", "svnicp_map_export", "svnicp_map_import",
-    "svnicp_pre_create", "svnicp_pre_destroy", "svnicp_pre_last_error", "svnicp_pre_crop", "svnicp_pre_downsample_uniform",
+    "svnicp_map_download", "svnicp_map_size", "svnicp_map_evaluate", "svnicp_map_search", "svnicp_map_export",
+    "svnicp_map_import", "svnicp_pre_create", "svnicp_pre_destroy", "svnicp_pre_last_error", "svnicp_pre_crop", "svnicp_pre_downsample_uniform",
     "svnicp_pre_to_f64", "svnicp_pre_download", "svnicp_pre_deskew", "svnicp_pose_compose",
     "svnicp_batch_create", "svnicp_batch_destroy", "svnicp_batch_last_error", "svnicp_batch_size", "svnicp_batch_stream", "svnicp_batch_align",
 ]
@@ -158,7 +158,7 @@ def _ARGTYPES(V, I, L, D):
         "svnicp_map_create": [V, D, D, I, L, I], "svnicp_map_clear": [V], "svnicp_map_add_cloud": [V, V, L, I, I, V, V],
         "svnicp_map_get": [V, V, D, V, V], "svnicp_map_download": [V, V, L], "svnicp_map_size": [V, V, V],
         "svnicp_map_evaluate": [V, V, L, I, I, V, V, I, V, D, V, V, V, V, V], "svnicp_map_export": [V, V, V, V, L, L, I],
-        "svnicp_map_import": [V, V, V, V, L, L, I],
+        "svnicp_map_search": [V, V, L, I, I, V, V, V, V, D, I, V, V, V, V], "svnicp_map_import": [V, V, V, V, L, L, I],
         "svnicp_pre_create": [V, L, I], "svnicp_pre_crop": [V, V, L, I, D, D, V, V, V],
         "svnicp_pre_downsample_uniform": [V, V, L, I, D, V, V], "svnicp_pre_to_f64": [V, V, L, V], "svnicp_pre_download": [V, V, L, V],
         "svnicp_pre_deskew": [V, V, L, I, V, I, I, V, V, V, V, V, V], "svnicp_pose_compose": [V, V, V, V, V],
@@ -584,6 +584,20 @@ def read_map_snapshot(path: str) -> MapSnapshot:
     return MapSnapshot(float(h["voxel_size"]), float(h["max_range"]), int(h["max_pointscount"]), vox, cnt, pts)
 
 
+def search_grid_poses(counts, steps, g) -> np.ndarray:
+    """Poses [6, k] of flat grid indices g (svnicp_map_search's grid; no GPU): axis a has counts[a] values
+    x_a(i) = (i - 0.5 (counts[a] - 1)) * steps[a], and g = i0 + counts[0] * (i1 + counts[1] * (i2 + ...)), axis 0 fastest."""
+    counts = np.asarray(counts, dtype=np.int64).reshape(6)
+    steps = np.asarray(steps, dtype=np.float64).reshape(6)
+    g = np.asarray(g, dtype=np.int64).reshape(-1).copy()
+    out = np.zeros((6, len(g)))
+    for a in range(6):
+        i = g % counts[a]
+        g //= counts[a]
+        out[a] = (i.astype(np.float64) - 0.5 * float(counts[a] - 1)) * steps[a]
+    return out
+
+
 class VoxelHashMap:
     """Drop-in for svnicp::VoxelHashMap (VoxelHashMap.h:28-72, VoxelHashMap.cpp:22-101), device resident: the local map the
     node keeps between scans (OdometryPipeline.cpp:577-581, :630).  Same method names; poses are (R [3,3], t [3])."""
@@ -696,6 +710,36 @@ class VoxelHashMap:
             if v is not None:
                 out[k] = v
         return {k: v[0] for k, v in out.items()} if single else out
+
+    def Search(self, source, R0, t0, counts, steps, max_dist: float, top_k: int = 1, want_counts: bool = False) -> dict:
+        """Exhaustive search of a scan over a grid of poses around T0 = (R0, t0) (svnicp_map_search; no reference counterpart):
+        relocalisation, loop-closure checks.  counts [6] values per axis of x = [t ; omega], steps [6] their spacing, centred on
+        T0 (search_grid_poses gives the poses).  Score = inlier count of Evaluate; ranked by count descending, then grid index.
+        Returns index [k] int64, poses [6, k], count [k] int64, fitness [k], rmse [k] (Evaluate's values for the winners), and
+        counts (the score of every grid pose, shaped [counts[5], ..., counts[0]] so that counts[..., i0] runs along t_x) or None.
+        source: [n,3] float32 or float64 sensor-frame points, host.  Changes no state of the map."""
+        a = np.asarray(source)
+        f64 = a.dtype != np.float32
+        a = np.ascontiguousarray(a, dtype=np.float64 if f64 else np.float32).reshape(-1, 3)
+        return self._search(_p(a), len(a), f64, False, R0, t0, counts, steps, max_dist, top_k, want_counts)
+
+    def SearchDevice(self, ptr: int, n: int, f64: bool, R0, t0, counts, steps, max_dist: float, top_k: int = 1,
+                     want_counts: bool = False) -> dict:
+        """Search for a device cloud: ptr to [n,3] float32 (f64 = False, e.g. a ScanPreprocessor output) or float64."""
+        return self._search(C.c_void_p(ptr), n, f64, True, R0, t0, counts, steps, max_dist, top_k, want_counts)
+
+    def _search(self, src, n, f64, on_device, R0, t0, counts, steps, max_dist, top_k, want_counts):
+        cnt = np.ascontiguousarray(counts, dtype=np.int32).reshape(6)
+        stp = _f64(steps).reshape(6)
+        k = int(top_k)
+        M = int(np.prod([int(c) for c in cnt])) if (cnt >= 1).all() else 0  # Python ints: no wrap-around
+        index, poses, stats = np.zeros(max(k, 1), dtype=np.int64), np.zeros((6, max(k, 1))), np.zeros((max(k, 1), 3))
+        grid = np.zeros(M, dtype=np.int32) if want_counts and 0 < M < 2 ** 31 else None
+        self._check(self._lib.svnicp_map_search(self._m, src, C.c_int64(n), C.c_int(int(f64)), C.c_int(int(on_device)),
+                                                _p(_f64(R0).reshape(9)), _p(_f64(t0).reshape(3)), _p(cnt), _p(stp),
+                                                C.c_double(max_dist), C.c_int(k), _p(index), _p(poses), _p(stats), _p(grid)), "Search")
+        return dict(index=index, poses=poses, count=stats[:, 0].astype(np.int64), fitness=stats[:, 1].copy(), rmse=stats[:, 2].copy(),
+                    counts=grid.reshape(tuple(int(c) for c in cnt[::-1])) if grid is not None else None)
 
     # -- snapshots (svnicp_map_export / svnicp_map_import; no reference counterpart) --------------
     def Export(self) -> MapSnapshot:

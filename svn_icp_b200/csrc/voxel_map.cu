@@ -18,6 +18,10 @@
 // nearest-map-point search per (source point, pose) by read-only probes of the same hash (k_map_eval), then the fixed-order
 // reduction of svnicp_evaluate (k_eval_fin, eval_kernels.cu).
 //
+// svnicp_map_search (DESIGN.md section 10d) ranks a regular grid of poses by the same inlier count: an existence test per
+// (source point, pose) with an early exit (k_map_search_count), integer counts per pose and a deterministic running top k
+// (k_map_search_topk); the winners' statistics come from svnicp_map_evaluate itself.
+//
 // svnicp_map_export / svnicp_map_import (DESIGN.md section 10c) save and restore the content in canonical form -- voxels in
 // ascending (vx, vy, vz), each voxel's points in stored order -- independent of the slot layout: a radix sort of the live keys
 // on the way out, a rebuild into the twin table with full validation on the way in.
@@ -398,17 +402,13 @@ __device__ __forceinline__ int map_find(const MapTable &t, int slots_mask, unsig
   return slot < 0 || __ldg(t.count + slot) > 0 ? slot : -1;
 }
 
-// Per pose of a block, x = [t ; omega] relative to T0 = (R0, t0): R~ = R0 Exp(omega), t~ = t0 + R0 t -> Rt [MB][12], and
-// R_p = Exp(omega) -> Rp [MB][9] for gn_assemble.  x = 0 gives R_p = I exactly, and (R0, t0) is stored as given, so the
-// query of a pose x = 0 is q0 bit for bit (the products would turn a -0 entry of R0 into +0).
-__global__ void k_map_eval_prep(const double *x6 /*[MB][6]*/, int MB, svn::ScanConst sc, double *Rt, double *Rp) {
-  const int p = threadIdx.x;
-  if (p >= MB) return;
-  const double *x = x6 + 6 * p;
-  double R[9];
+// One pose x = [t ; omega] relative to T0 = (R0, t0): R~ = R0 Exp(omega), t~ = t0 + R0 t -> o [12] (R~ row-major, t~), and
+// R_p = Exp(omega) -> R [9].  x = 0 gives R_p = I exactly, and (R0, t0) is stored as given, so the query of a pose x = 0 is
+// q0 bit for bit (the products would turn a -0 entry of R0 into +0).  The one place this is computed: svnicp_map_evaluate
+// (k_map_eval_prep) and svnicp_map_search (k_map_search_prep) cannot drift apart.
+__device__ __forceinline__ void map_pose(const double *x, const svn::ScanConst &sc, double *o, double R[9]) {
   svn::so3_exp(x + 3, R, nullptr);
   const bool zero = x[0] == 0.0 && x[1] == 0.0 && x[2] == 0.0 && x[3] == 0.0 && x[4] == 0.0 && x[5] == 0.0;
-  double *o = Rt + 12 * p;
 #pragma unroll
   for (int r = 0; r < 3; r++) {
 #pragma unroll
@@ -416,6 +416,14 @@ __global__ void k_map_eval_prep(const double *x6 /*[MB][6]*/, int MB, svn::ScanC
       o[3 * r + c] = zero ? sc.R0[3 * r + c] : sc.R0[3 * r] * R[c] + sc.R0[3 * r + 1] * R[3 + c] + sc.R0[3 * r + 2] * R[6 + c];
     o[9 + r] = zero ? sc.t0[r] : sc.t0[r] + (sc.R0[3 * r] * x[0] + sc.R0[3 * r + 1] * x[1] + sc.R0[3 * r + 2] * x[2]);
   }
+}
+
+// Per pose of a block: Rt [MB][12] and Rp [MB][9] (for gn_assemble) by map_pose
+__global__ void k_map_eval_prep(const double *x6 /*[MB][6]*/, int MB, svn::ScanConst sc, double *Rt, double *Rp) {
+  const int p = threadIdx.x;
+  if (p >= MB) return;
+  double R[9];
+  map_pose(x6 + 6 * p, sc, Rt + 12 * p, R);
 #pragma unroll
   for (int i = 0; i < 9; i++) Rp[9 * p + i] = R[i];
 }
@@ -565,6 +573,178 @@ __global__ void __launch_bounds__(MEV_THREADS, SYS ? 4 : 8) k_map_eval(MapDev m,
   }
 }
 
+// ---- svnicp_map_search (DESIGN.md section 10d) -------------------------------------------------------------------------------
+// Per chunk of grid poses: k_map_search_prep (grid value -> R~ t~ by map_pose) -> k_map_search_count (inlier count per pose)
+// -> k_map_search_topk (running top k of the keys ((n - count) << 32) | g).
+constexpr int MS_CHUNK = 16384;      // poses per chunk at most (scratch: 100 B per pose); fewer for large scans, see svnicp_map_search
+constexpr int MS_MAX_K = 1024;       // top_k limit: the winners are sorted in one block of MS_TOPK_THREADS
+constexpr int MS_TOPK_THREADS = 1024;
+
+// Grid value i of an axis with `count` values and step `step`: ((double)i - 0.5 (count - 1)) * step.  The difference is exact
+// (half integers below 2^31), so the one rounding is the product's, as in search_grid_poses of the Python mirror and the host
+// decode in svnicp_map_search.
+__host__ __device__ __forceinline__ double grid_value(int i, int count, double step) {
+  return ((double)i - 0.5 * (double)(count - 1)) * step;
+}
+
+struct GridSpec {
+  int counts[6];
+  double steps[6];
+};
+
+// R~ t~ of grid poses g0 .. g0 + Mc - 1 -> Rt [Mc][12], the bits k_map_eval_prep gives the same x
+__global__ void k_map_search_prep(GridSpec gs, long long g0, int Mc, svn::ScanConst sc, double *Rt) {
+  const int p = blockIdx.x * blockDim.x + threadIdx.x;
+  if (p >= Mc) return;
+  long long g = g0 + p;
+  double x[6], R[9];
+#pragma unroll
+  for (int a = 0; a < 6; a++) {
+    const int i = (int)(g % gs.counts[a]);
+    g /= gs.counts[a];
+    x[a] = grid_value(i, gs.counts[a], gs.steps[a]);
+  }
+  map_pose(x, sc, Rt + 12 * (size_t)p, R);
+}
+
+// Does the voxel hold a point with d^2 < max_dist?
+__device__ __forceinline__ bool slot_any_within(const MapTable &t, int cap, int slot, const double q[3], double max_dist) {
+  const int c = __ldg(t.count + slot);
+  const float *p = t.pts + (size_t)slot * cap * 3;
+  for (int k = 0; k < c; k++) {
+    const double mp[3] = {(double)__ldg(p + 3 * k), (double)__ldg(p + 3 * k + 1), (double)__ldg(p + 3 * k + 2)};
+    if (svn::dist2(q, mp) < max_dist) return true;
+  }
+  return false;
+}
+
+// Is there a stored point with d^2 < max_dist for the finite query q?  The box, the probes and dist2 are map_nearest's, but the
+// walk stops at the first such point and the box never shrinks.  This is map_nearest's `found`, bit for bit: map_nearest sets
+// found exactly when it visits a point with dist2 < max_dist (its running bound starts at max_dist), and both walks visit every
+// voxel of the initial box until then -- map_nearest shrinks the box only once found is set.  By the box argument of box_axis,
+// the initial box (radius r = sqrt(max_dist) * MEV_MARGIN) holds every point whose dist2 can fall below max_dist, dist2's
+// rounding being far below the margin.  So both are "some stored point has dist2(q, p) < max_dist", evaluated on the same q
+// with the same dist2: the inlier count svnicp_map_evaluate reports.
+__device__ __forceinline__ bool map_any_within(const MapDev &m, double r, double max_dist, const double q[3]) {
+  const float v = m.voxel_size_f;
+  int lo[3], hi[3];
+  bool wide = false;
+#pragma unroll
+  for (int a = 0; a < 3; a++) {
+    box_axis(q[a], r, v, lo[a], hi[a]);
+    wide |= (long long)hi[a] - lo[a] >= MEV_SPAN;
+  }
+  if (wide) {  // map_nearest's sweep of the whole table, with the early exit
+    for (int slot = 0; slot <= m.slots_mask; slot++)
+      if (__ldg(m.tab.keys + slot) != EMPTY_KEY && slot_any_within(m.tab, m.cap, slot, q, max_dist)) return true;
+    return false;
+  }
+  int own[3];
+#pragma unroll
+  for (int a = 0; a < 3; a++) own[a] = (int)__fdiv_rn(__double2float_rn(q[a]), v);
+  int slot = map_find(m.tab, m.slots_mask, svn::pack_voxel_key(own[0], own[1], own[2]));
+  if (slot >= 0 && slot_any_within(m.tab, m.cap, slot, q, max_dist)) return true;
+  for (int z = lo[2]; z <= hi[2]; z++)
+    for (int y = lo[1]; y <= hi[1]; y++)
+      for (int x = lo[0]; x <= hi[0]; x++) {
+        if (x == own[0] && y == own[1] && z == own[2]) continue;
+        slot = map_find(m.tab, m.slots_mask, svn::pack_voxel_key(x, y, z));
+        if (slot >= 0 && slot_any_within(m.tab, m.cap, slot, q, max_dist)) return true;
+      }
+  return false;
+}
+
+// Flat over (pose, point): warp w of the chunk holds 32 consecutive source points of pose w / wpp (wpp = warps per pose), as
+// k_map_eval's warps, so that neighbouring lanes probe the same voxels; a 900-point scan gives 29 warps per pose and a chunk
+// of 16 k poses fills the GPU.  q in k_map_eval's fma order; a non-finite q is not an inlier.  Integer counts: one
+// warp-aggregated atomicAdd per warp, the same sum in any order.
+template <typename T>
+__global__ void __launch_bounds__(MEV_THREADS) k_map_search_count(MapDev m, const T *__restrict__ src, int n, int wpp, int Mc,
+                                                                 const double *__restrict__ Rt, double max_dist, double r, int *cnt) {
+  const long long w = ((long long)blockIdx.x * MEV_THREADS + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  const int p = (int)(w / wpp);
+  if (p >= Mc) return;  // whole warps: MEV_THREADS is a multiple of 32
+  const int i = (int)(w - (long long)p * wpp) * 32 + lane;
+  bool in = false;
+  if (i < n) {
+    const double *P = Rt + 12 * (size_t)p;
+    double Rtl[9], ttl[3];
+#pragma unroll
+    for (int k = 0; k < 9; k++) Rtl[k] = __ldg(P + k);
+#pragma unroll
+    for (int k = 0; k < 3; k++) ttl[k] = __ldg(P + 9 + k);
+    const double x = (double)src[3 * (size_t)i], y = (double)src[3 * (size_t)i + 1], z = (double)src[3 * (size_t)i + 2];
+    double q[3];
+#pragma unroll
+    for (int a = 0; a < 3; a++) q[a] = svn::affine_row_fma(Rtl, ttl, a, x, y, z);
+    if (isfinite(q[0]) && isfinite(q[1]) && isfinite(q[2])) in = map_any_within(m, r, max_dist, q);
+  }
+  const unsigned b = __ballot_sync(0xffffffffu, in);
+  if (lane == 0 && b) atomicAdd(cnt + p, __popc(b));
+}
+
+// The running top k: the kk = min(k, n_best + Mc) smallest of the carried keys best [n_best] (sorted) and the chunk's keys
+// ((n - cnt[p]) << 32) | (g0 + p), sorted ascending back into best.  Keys are unique (g is), so the kk smallest are one set:
+// an MSB-first radix select over 8-bit digits finds the kk-th smallest key T exactly (integer histograms: no order dependence),
+// the keys <= T are compacted (exactly kk of them, in any order) and a bitonic sort in shared memory orders them.
+__device__ __forceinline__ unsigned long long search_key(const int *cnt, int p, long long g0, long long n) {
+  return ((unsigned long long)(n - cnt[p]) << 32) | (unsigned long long)(g0 + p);
+}
+
+__global__ void __launch_bounds__(MS_TOPK_THREADS) k_map_search_topk(const int *cnt, int Mc, long long g0, long long n,
+                                                                     unsigned long long *best, int n_best, int k) {
+  __shared__ int s_hist[RADIX_DIGITS];
+  __shared__ unsigned long long s_sel[MS_TOPK_THREADS];
+  __shared__ unsigned long long s_prefix, s_mask;
+  __shared__ int s_need, s_n;
+  const int tid = threadIdx.x, total = n_best + Mc, kk = total < k ? total : k;
+  auto key = [&](int j) { return j < n_best ? best[j] : search_key(cnt, j - n_best, g0, n); };
+  if (tid == 0) { s_prefix = 0; s_mask = 0; s_need = kk; s_n = 0; }
+  __syncthreads();
+  if (kk < total) {
+    for (int shift = 64 - RADIX_BITS; shift >= 0; shift -= RADIX_BITS) {
+      for (int d = tid; d < RADIX_DIGITS; d += MS_TOPK_THREADS) s_hist[d] = 0;
+      __syncthreads();
+      const unsigned long long prefix = s_prefix, mask = s_mask;
+      for (int j = tid; j < total; j += MS_TOPK_THREADS) {
+        const unsigned long long kj = key(j);
+        if ((kj & mask) == prefix) atomicAdd(&s_hist[(kj >> shift) & (RADIX_DIGITS - 1)], 1);
+      }
+      __syncthreads();
+      if (tid == 0) {  // the digit of the need-th smallest key among those matching the prefix
+        int need = s_need, d = 0;
+        while (s_hist[d] < need) need -= s_hist[d++];
+        s_need = need;
+        s_prefix = prefix | ((unsigned long long)d << shift);
+        s_mask = mask | ((unsigned long long)(RADIX_DIGITS - 1) << shift);
+      }
+      __syncthreads();
+    }
+  } else if (tid == 0) {
+    s_prefix = ~0ull;  // every candidate is kept
+  }
+  __syncthreads();
+  const unsigned long long T = s_prefix;
+  for (int j = tid; j < total; j += MS_TOPK_THREADS) {
+    const unsigned long long kj = key(j);
+    if (kj <= T) s_sel[atomicAdd(&s_n, 1)] = kj;
+  }
+  __syncthreads();
+  if (tid >= s_n) s_sel[tid] = ~0ull;  // s_n == kk <= MS_TOPK_THREADS
+  __syncthreads();
+  for (int size = 2; size <= MS_TOPK_THREADS; size <<= 1)
+    for (int stride = size >> 1; stride > 0; stride >>= 1) {
+      const int j = tid ^ stride;
+      if (j > tid) {
+        const unsigned long long a = s_sel[tid], b = s_sel[j];
+        if ((a > b) == ((tid & size) == 0)) { s_sel[tid] = b; s_sel[j] = a; }
+      }
+      __syncthreads();
+    }
+  if (tid < kk) best[tid] = s_sel[tid];
+}
+
 }  // namespace
 
 struct svnicp_map_t {
@@ -595,6 +775,11 @@ struct svnicp_map_t {
   uint8_t *ev_mask = nullptr;
   float *ev_near = nullptr;
   size_t ev_src_cap = 0, ev_part_cap = 0, ev_mask_cap = 0, ev_near_cap = 0;
+  // svnicp_map_search scratch (grown on demand): R~ t~ [chunk][12], counts [chunk], the running top k [MS_MAX_K]
+  double *ms_rt = nullptr;
+  int *ms_cnt = nullptr;
+  unsigned long long *ms_best = nullptr;
+  size_t ms_rt_cap = 0, ms_cnt_cap = 0, ms_best_cap = 0;
   // svnicp_map_export / svnicp_map_import scratch (grown on demand; nothing above is touched by it), indexed by SN_*
   void *sn[11] = {};
   size_t sn_cap[11] = {};
@@ -689,6 +874,7 @@ void svnicp_map_destroy(svnicp_map m) {
   cudaFree(m->head); cudaFree(m->walker); cudaFree(m->counters); cudaFree(m->d_pose); cudaFree(m->block_sums);
   cudaFree(m->batch_in); cudaFree(m->wxyz); cudaFree(m->pt_slot); cudaFree(m->next); cudaFree(m->out);
   cudaFree(m->ev_src); cudaFree(m->ev_pose); cudaFree(m->ev_part); cudaFree(m->ev_out); cudaFree(m->ev_mask); cudaFree(m->ev_near);
+  cudaFree(m->ms_rt); cudaFree(m->ms_cnt); cudaFree(m->ms_best);
   for (void *p : m->sn) cudaFree(p);
   if (m->h_counters) cudaFreeHost(m->h_counters);
   if (m->stream) cudaStreamDestroy(m->stream);
@@ -837,6 +1023,26 @@ static int ev_grow(svnicp_map m, void **p, size_t *cap, size_t bytes) {
   return SVNICP_OK;
 }
 
+// The scan and threshold checks shared by svnicp_map_evaluate and svnicp_map_search: n, max_dist and the search-radius limit
+static int check_scan_args(svnicp_map m, const char *fn, int64_t n, double max_dist) {
+  char buf[256];
+  if (n < 1 || n > (1ll << 30)) {
+    snprintf(buf, sizeof(buf), "%s: need 1 <= n <= 2^30 source points", fn);
+    return mfail(m, SVNICP_ERR_INVALID, buf);
+  }
+  if (!isfinite(max_dist) || !(max_dist > 0)) {
+    snprintf(buf, sizeof(buf), "%s: max_dist must be finite and > 0", fn);
+    return mfail(m, SVNICP_ERR_INVALID, buf);
+  }
+  const double r = sqrt(max_dist);
+  if (ceil(r / m->voxel_size) > MEV_MAX_REACH) {
+    snprintf(buf, sizeof(buf), "%s: search radius sqrt(max_dist) = %g m spans %g voxels of %g m on each side of the "
+             "query; at most %d are supported", fn, r, ceil(r / m->voxel_size), m->voxel_size, MEV_MAX_REACH);
+    return mfail(m, SVNICP_ERR_INVALID, buf);
+  }
+  return SVNICP_OK;
+}
+
 template <bool SYS>
 static void go_map_eval(const MapDev &d, const void *src, int dtype_f64, dim3 grid, int n, const double *Rt, const svn::ScanConst &sc,
                         double max_dist, double r, double *part, uint8_t *mask, float *nearest, cudaStream_t st) {
@@ -855,16 +1061,10 @@ extern "C" int svnicp_map_evaluate(svnicp_map m, const void *source, int64_t n, 
   if (!m) return SVNICP_ERR_INVALID;
   if (!source || !R0 || !t0 || !poses_6xM || !out_stats)
     return mfail(m, SVNICP_ERR_INVALID, "svnicp_map_evaluate: null source, R0, t0, poses or out_stats");
-  if (n < 1 || n > (1ll << 30)) return mfail(m, SVNICP_ERR_INVALID, "svnicp_map_evaluate: need 1 <= n <= 2^30 source points");
+  int rc = check_scan_args(m, "svnicp_map_evaluate", n, max_dist);
+  if (rc) return rc;
   if (n_poses < 1) return mfail(m, SVNICP_ERR_INVALID, "svnicp_map_evaluate: n_poses must be >= 1");
-  if (!isfinite(max_dist) || !(max_dist > 0)) return mfail(m, SVNICP_ERR_INVALID, "svnicp_map_evaluate: max_dist must be finite and > 0");
   const double r = sqrt(max_dist);
-  if (ceil(r / m->voxel_size) > MEV_MAX_REACH) {
-    char buf[256];
-    snprintf(buf, sizeof(buf), "svnicp_map_evaluate: search radius sqrt(max_dist) = %g m spans %g voxels of %g m on each side of the "
-             "query; at most %d are supported", r, ceil(r / m->voxel_size), m->voxel_size, MEV_MAX_REACH);
-    return mfail(m, SVNICP_ERR_INVALID, buf);
-  }
   MCU(cudaSetDevice(m->device));
   cudaStream_t st = m->stream;
   const int ni = (int)n, M = n_poses;
@@ -872,7 +1072,6 @@ extern "C" int svnicp_map_evaluate(svnicp_map m, const void *source, int64_t n, 
   int parts = (int)((n + MEV_THREADS - 1) / MEV_THREADS);
   if (parts > m->sm_count * MEV_CTAS_PER_SM) parts = m->sm_count * MEV_CTAS_PER_SM;
   const size_t esz = dtype_f64 ? sizeof(double) : sizeof(float);
-  int rc;
   if ((rc = ev_grow(m, (void **)&m->ev_part, &m->ev_part_cap, (size_t)parts * mb_max * EV_NS * sizeof(double))) ||
       (!on_device && (rc = ev_grow(m, &m->ev_src, &m->ev_src_cap, (size_t)n * 3 * esz))) ||
       (out_mask && (rc = ev_grow(m, (void **)&m->ev_mask, &m->ev_mask_cap, (size_t)mb_max * n))) ||
@@ -918,6 +1117,82 @@ extern "C" int svnicp_map_evaluate(svnicp_map m, const void *source, int64_t n, 
     }
   }
   return SVNICP_OK;
+}
+
+// ---- svnicp_map_search --------------------------------------------------------------------------------------------------------
+extern "C" int svnicp_map_search(svnicp_map m, const void *source, int64_t n, int dtype_f64, int on_device, const double R0[9],
+                                 const double t0[3], const int32_t counts[6], const double steps[6], double max_dist, int top_k,
+                                 int64_t *out_index, double *out_poses_6xK, double *out_stats, int32_t *out_counts) {
+  if (!m) return SVNICP_ERR_INVALID;
+  if (!source || !R0 || !t0 || !counts || !steps || !out_index || !out_poses_6xK || !out_stats)
+    return mfail(m, SVNICP_ERR_INVALID, "svnicp_map_search: null source, R0, t0, counts, steps, out_index, out_poses or out_stats");
+  int rc = check_scan_args(m, "svnicp_map_search", n, max_dist);
+  if (rc) return rc;
+  long long M = 1;
+  for (int a = 0; a < 6; a++) {
+    if (counts[a] < 1) return mfail(m, SVNICP_ERR_INVALID, "svnicp_map_search: every grid count must be >= 1");
+    if (!isfinite(steps[a]) || !(steps[a] >= 0)) return mfail(m, SVNICP_ERR_INVALID, "svnicp_map_search: every grid step must be finite and >= 0");
+    M *= counts[a];
+    if (M > INT_MAX) return mfail(m, SVNICP_ERR_INVALID, "svnicp_map_search: the grid holds more than 2^31 - 1 poses");
+  }
+  if (top_k < 1 || top_k > MS_MAX_K || top_k > M) {
+    char buf[160];
+    snprintf(buf, sizeof(buf), "svnicp_map_search: top_k = %d is outside [1, min(%lld grid poses, %d)]", top_k, M, MS_MAX_K);
+    return mfail(m, SVNICP_ERR_INVALID, buf);
+  }
+  MCU(cudaSetDevice(m->device));
+  cudaStream_t st = m->stream;
+  // poses per chunk: at most MS_CHUNK, and about 2^27 queries for large scans (one pose at least)
+  const long long by_n = (1ll << 27) / n;
+  const int chunk = (int)(by_n < 1 ? 1 : by_n < MS_CHUNK ? by_n : MS_CHUNK);
+  const int wpp = (int)((n + 31) / 32);
+  const size_t esz = dtype_f64 ? sizeof(double) : sizeof(float);
+  if ((rc = ev_grow(m, (void **)&m->ms_rt, &m->ms_rt_cap, (size_t)chunk * 12 * sizeof(double))) ||
+      (rc = ev_grow(m, (void **)&m->ms_cnt, &m->ms_cnt_cap, (size_t)chunk * sizeof(int))) ||
+      (rc = ev_grow(m, (void **)&m->ms_best, &m->ms_best_cap, (size_t)MS_MAX_K * sizeof(unsigned long long))) ||
+      (!on_device && (rc = ev_grow(m, &m->ev_src, &m->ev_src_cap, (size_t)n * 3 * esz))))
+    return rc;
+  const void *src = source;
+  if (!on_device) {
+    MCU(cudaMemcpyAsync(m->ev_src, source, (size_t)n * 3 * esz, cudaMemcpyHostToDevice, st));
+    src = m->ev_src;
+  }
+  svn::ScanConst sc;
+  memcpy(sc.R0, R0, sizeof(sc.R0));
+  memcpy(sc.t0, t0, sizeof(sc.t0));
+  GridSpec gs;
+  memcpy(gs.counts, counts, sizeof(gs.counts));
+  memcpy(gs.steps, steps, sizeof(gs.steps));
+  const MapDev d = dev_view(m, m->cur);
+  const double r = sqrt(max_dist) * MEV_MARGIN;  // k_map_eval's radius
+  int n_best = 0;
+  for (long long g0 = 0; g0 < M; g0 += chunk) {
+    const int Mc = (int)(M - g0 < chunk ? M - g0 : chunk);
+    k_map_search_prep<<<(Mc + 127) / 128, 128, 0, st>>>(gs, g0, Mc, sc, m->ms_rt);
+    MCU(cudaMemsetAsync(m->ms_cnt, 0, (size_t)Mc * sizeof(int), st));
+    const unsigned blocks = (unsigned)(((long long)Mc * wpp + MEV_THREADS / 32 - 1) / (MEV_THREADS / 32));
+    if (dtype_f64)
+      k_map_search_count<double><<<blocks, MEV_THREADS, 0, st>>>(d, (const double *)src, (int)n, wpp, Mc, m->ms_rt, max_dist, r, m->ms_cnt);
+    else
+      k_map_search_count<float><<<blocks, MEV_THREADS, 0, st>>>(d, (const float *)src, (int)n, wpp, Mc, m->ms_rt, max_dist, r, m->ms_cnt);
+    k_map_search_topk<<<1, MS_TOPK_THREADS, 0, st>>>(m->ms_cnt, Mc, g0, n, m->ms_best, n_best, top_k);
+    MCU(cudaGetLastError());
+    if (out_counts) MCU(cudaMemcpyAsync(out_counts + g0, m->ms_cnt, (size_t)Mc * sizeof(int), cudaMemcpyDeviceToHost, st));
+    n_best = n_best + Mc < top_k ? n_best + Mc : top_k;
+  }
+  std::vector<unsigned long long> best((size_t)top_k);
+  MCU(cudaMemcpyAsync(best.data(), m->ms_best, (size_t)top_k * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+  MCU(cudaStreamSynchronize(st));
+  for (int j = 0; j < top_k; j++) {
+    long long g = (long long)(best[j] & 0xFFFFFFFFull);
+    out_index[j] = g;
+    for (int a = 0; a < 6; a++) {
+      out_poses_6xK[(size_t)a * top_k + j] = grid_value((int)(g % counts[a]), counts[a], steps[a]);
+      g /= counts[a];
+    }
+  }
+  // the winners' statistics are svnicp_map_evaluate's by construction: the same call on the grid values (source already on device)
+  return svnicp_map_evaluate(m, src, n, dtype_f64, 1, R0, t0, top_k, out_poses_6xK, max_dist, out_stats, nullptr, nullptr, nullptr, nullptr);
 }
 
 // ---- svnicp_map_export / svnicp_map_import -----------------------------------------------------------------------------------

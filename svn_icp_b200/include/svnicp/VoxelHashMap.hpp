@@ -166,6 +166,44 @@ struct VoxelHashMap {
     return r;
   }
 
+  /** Result of Search: the k winners, best first (index = flat grid index g, poses [6][k] the grid values relative to T0,
+   *  count / fitness / rmse Evaluate's values for them), and with want_counts the score of every grid pose in g order. */
+  struct SearchResult {
+    int k = 0;
+    std::vector<int64_t> index;
+    std::vector<double> poses;
+    std::vector<int64_t> count;
+    std::vector<double> fitness, rmse;
+    std::vector<int32_t> counts;
+  };
+  /** Exhaustive search of a scan over a grid of poses around T0 (svnicp_map_search; no reference counterpart): counts[a] values
+   *  x_a(i) = (i - 0.5 (counts[a] - 1)) steps[a] per axis of x = [t ; omega], flat index g with axis 0 fastest.  Score = the
+   *  inlier count of Evaluate; ranked by count descending, then g ascending.  Changes no state of the map. */
+  SearchResult Search(const float *xyz, int64_t n, const InitialMean &T0, const int32_t (&counts)[6], const double (&steps)[6],
+                      double max_dist, int top_k = 1, bool want_counts = false, bool on_device = false) {
+    int64_t M = 1;  // capped at 2^31: the ABI refuses larger grids
+    for (int a = 0; a < 6; a++) {
+      M *= counts[a] > 0 ? counts[a] : 0;
+      if (M > INT32_MAX) M = (int64_t)INT32_MAX + 1;
+    }
+    if (top_k < 1 || (int64_t)top_k > M) throw Error("Search: need 1 <= top_k <= the number of grid poses");
+    SearchResult r;
+    r.k = top_k;
+    r.index.resize((size_t)top_k);
+    r.poses.resize(6 * (size_t)top_k);
+    std::vector<double> stats(3 * (size_t)top_k);
+    if (want_counts && M <= INT32_MAX) r.counts.resize((size_t)M);
+    check(svnicp_map_search(m_, xyz, n, 0, on_device, T0.R.data(), T0.t.data(), counts, steps, max_dist, top_k, r.index.data(),
+                            r.poses.data(), stats.data(), want_counts ? r.counts.data() : nullptr),
+          "Search");
+    for (int j = 0; j < top_k; j++) {
+      r.count.push_back((int64_t)stats[3 * j]);
+      r.fitness.push_back(stats[3 * j + 1]);
+      r.rmse.push_back(stats[3 * j + 2]);
+    }
+    return r;
+  }
+
   using Snapshot = MapSnapshot;
   /** The content in canonical form (svnicp_map_export; no reference counterpart) */
   Snapshot Export() const {
