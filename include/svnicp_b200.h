@@ -287,10 +287,18 @@ int svnicp_map_evaluate(svnicp_map m, const void *source, int64_t n, int dtype_f
  *   out_counts [M] int32 (may be NULL)  the score of every grid pose, in g order
  * Host outputs.  Blocking, on the map's stream; changes no state of the map.  SVNICP_ERR_INVALID: svnicp_map_evaluate's argument
  * errors, null counts / steps / outputs, a count < 1, a negative or non-finite step, M > 2^31 - 1, top_k outside
- * [1, min(M, 1024)]. */
+ * [1, min(M, 1024)].
+ * Path: with out_counts == NULL, a grid of at least 16 * top_k poses whose translation axes can be cut into blocks takes a
+ * branch-and-bound path that counts only the blocks whose inlier bound can still reach the k-th count; every other call counts
+ * every pose.  Both return the same bits (svnicp_map_search_info reports which ran). */
 int svnicp_map_search(svnicp_map m, const void *source, int64_t n, int dtype_f64, int on_device, const double R0[9], const double t0[3],
                       const int32_t counts[6], const double steps[6], double max_dist, int top_k, int64_t *out_index,
                       double *out_poses_6xK, double *out_stats, int32_t *out_counts);
+/* The work done by the last svnicp_map_search on this map that returned SVNICP_OK (SVNICP_ERR_INVALID before the first one):
+ *   out8 = {path (0 every pose counted, 1 pruned), grid poses M, poses per full block, blocks, blocks counted, poses counted
+ *           exactly, bound queries (blocks * n), bound violations (a pose counting more than its block's bound: always 0)}
+ * On path 0: poses per block 0, blocks 0, blocks counted 0, poses counted M, bound queries 0, violations -1. */
+int svnicp_map_search_info(svnicp_map m, int64_t out8[8]);
 /* Snapshot of the map's content (no reference counterpart), to save a map and restore it bit for bit with svnicp_map_import:
  *   voxels [V][3] int32  voxel indices (vx, vy, vz) in ascending lexicographic order
  *   counts [V]    int32  points per voxel, 1 <= count <= max_pointscount

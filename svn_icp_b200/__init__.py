@@ -95,7 +95,7 @@ EXPORTS = [
     "svnicp_get_median_paths", "svnicp_get_timing", "svnicp_get_slice", "svnicp_get_launch_count", "svnicp_set_profiling", "svnicp_get_phase_times",
     "svnicp_get_scan_info", "svnicp_get_tail_stamps", "svnicp_evaluate",
     "svnicp_map_create", "svnicp_map_destroy", "svnicp_map_last_error", "svnicp_map_clear", "svnicp_map_add_cloud", "svnicp_map_get",
-    "svnicp_map_download", "svnicp_map_size", "svnicp_map_evaluate", "svnicp_map_search", "svnicp_map_export",
+    "svnicp_map_download", "svnicp_map_size", "svnicp_map_evaluate", "svnicp_map_search", "svnicp_map_search_info", "svnicp_map_export",
     "svnicp_map_import", "svnicp_pre_create", "svnicp_pre_destroy", "svnicp_pre_last_error", "svnicp_pre_crop", "svnicp_pre_downsample_uniform",
     "svnicp_pre_to_f64", "svnicp_pre_download", "svnicp_pre_deskew", "svnicp_pose_compose",
     "svnicp_batch_create", "svnicp_batch_destroy", "svnicp_batch_last_error", "svnicp_batch_size", "svnicp_batch_stream", "svnicp_batch_align",
@@ -158,7 +158,8 @@ def _ARGTYPES(V, I, L, D):
         "svnicp_map_create": [V, D, D, I, L, I], "svnicp_map_clear": [V], "svnicp_map_add_cloud": [V, V, L, I, I, V, V],
         "svnicp_map_get": [V, V, D, V, V], "svnicp_map_download": [V, V, L], "svnicp_map_size": [V, V, V],
         "svnicp_map_evaluate": [V, V, L, I, I, V, V, I, V, D, V, V, V, V, V], "svnicp_map_export": [V, V, V, V, L, L, I],
-        "svnicp_map_search": [V, V, L, I, I, V, V, V, V, D, I, V, V, V, V], "svnicp_map_import": [V, V, V, V, L, L, I],
+        "svnicp_map_search": [V, V, L, I, I, V, V, V, V, D, I, V, V, V, V], "svnicp_map_search_info": [V, V],
+        "svnicp_map_import": [V, V, V, V, L, L, I],
         "svnicp_pre_create": [V, L, I], "svnicp_pre_crop": [V, V, L, I, D, D, V, V, V],
         "svnicp_pre_downsample_uniform": [V, V, L, I, D, V, V], "svnicp_pre_to_f64": [V, V, L, V], "svnicp_pre_download": [V, V, L, V],
         "svnicp_pre_deskew": [V, V, L, I, V, I, I, V, V, V, V, V, V], "svnicp_pose_compose": [V, V, V, V, V],
@@ -712,12 +713,13 @@ class VoxelHashMap:
         return {k: v[0] for k, v in out.items()} if single else out
 
     def Search(self, source, R0, t0, counts, steps, max_dist: float, top_k: int = 1, want_counts: bool = False) -> dict:
-        """Exhaustive search of a scan over a grid of poses around T0 = (R0, t0) (svnicp_map_search; no reference counterpart):
+        """Exact search of a scan over a grid of poses around T0 = (R0, t0) (svnicp_map_search; no reference counterpart):
         relocalisation, loop-closure checks.  counts [6] values per axis of x = [t ; omega], steps [6] their spacing, centred on
         T0 (search_grid_poses gives the poses).  Score = inlier count of Evaluate; ranked by count descending, then grid index.
         Returns index [k] int64, poses [6, k], count [k] int64, fitness [k], rmse [k] (Evaluate's values for the winners), and
         counts (the score of every grid pose, shaped [counts[5], ..., counts[0]] so that counts[..., i0] runs along t_x) or None.
-        source: [n,3] float32 or float64 sensor-frame points, host.  Changes no state of the map."""
+        source: [n,3] float32 or float64 sensor-frame points, host.  Changes no state of the map.  Without want_counts a grid
+        with translation blocks is searched by branch and bound (SearchInfo), with the same result."""
         a = np.asarray(source)
         f64 = a.dtype != np.float32
         a = np.ascontiguousarray(a, dtype=np.float64 if f64 else np.float32).reshape(-1, 3)
@@ -740,6 +742,17 @@ class VoxelHashMap:
                                                 C.c_double(max_dist), C.c_int(k), _p(index), _p(poses), _p(stats), _p(grid)), "Search")
         return dict(index=index, poses=poses, count=stats[:, 0].astype(np.int64), fitness=stats[:, 1].copy(), rmse=stats[:, 2].copy(),
                     counts=grid.reshape(tuple(int(c) for c in cnt[::-1])) if grid is not None else None)
+
+    SEARCH_INFO_FIELDS = ("path", "grid_poses", "poses_per_block", "blocks", "blocks_counted", "poses_counted", "bound_queries",
+                          "violations")
+
+    def SearchInfo(self) -> dict:
+        """The work of the last successful Search (svnicp_map_search_info): path 0 counted every pose, path 1 pruned by block
+        bounds; poses_counted of grid_poses were counted exactly; violations (poses above their block's bound) is always 0 on
+        path 1 and -1 on path 0."""
+        out = np.zeros(8, dtype=np.int64)
+        self._check(self._lib.svnicp_map_search_info(self._m, _p(out)), "SearchInfo")
+        return {k: int(v) for k, v in zip(self.SEARCH_INFO_FIELDS, out)}
 
     # -- snapshots (svnicp_map_export / svnicp_map_import; no reference counterpart) --------------
     def Export(self) -> MapSnapshot:

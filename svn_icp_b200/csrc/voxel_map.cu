@@ -582,8 +582,9 @@ constexpr int MS_TOPK_THREADS = 1024;
 
 // Grid value i of an axis with `count` values and step `step`: ((double)i - 0.5 (count - 1)) * step.  The difference is exact
 // (half integers below 2^31), so the one rounding is the product's, as in search_grid_poses of the Python mirror and the host
-// decode in svnicp_map_search.
-__host__ __device__ __forceinline__ double grid_value(int i, int count, double step) {
+// decode in svnicp_map_search.  A 64-bit i is the pruned path's virtual block end, which may lie past the axis (below 2^32).
+template <typename I>
+__host__ __device__ __forceinline__ double grid_value(I i, int count, double step) {
   return ((double)i - 0.5 * (double)(count - 1)) * step;
 }
 
@@ -688,18 +689,26 @@ __global__ void __launch_bounds__(MEV_THREADS) k_map_search_count(MapDev m, cons
 // ((n - cnt[p]) << 32) | (g0 + p), sorted ascending back into best.  Keys are unique (g is), so the kk smallest are one set:
 // an MSB-first radix select over 8-bit digits finds the kk-th smallest key T exactly (integer histograms: no order dependence),
 // the keys <= T are compacted (exactly kk of them, in any order) and a bitonic sort in shared memory orders them.
-__device__ __forceinline__ unsigned long long search_key(const int *cnt, int p, long long g0, long long n) {
+// LIST (the pruned path): pose p of the chunk is grid pose gl[p], or no pose at all when gl[p] < 0 (a slot of a partial edge
+// block).  Such a slot's key is MS_NO_POSE, above every real key (n - cnt < 2^31); it may repeat, so the compaction skips it:
+// the real keys are still unique, at most kk of them are <= T, and the rest of best is padded with MS_NO_POSE.
+constexpr unsigned long long MS_NO_POSE = ~0ull;
+
+template <bool LIST>
+__device__ __forceinline__ unsigned long long search_key(const int *cnt, const int *gl, int p, long long g0, long long n) {
+  if (LIST) return gl[p] < 0 ? MS_NO_POSE : ((unsigned long long)(n - cnt[p]) << 32) | (unsigned long long)gl[p];
   return ((unsigned long long)(n - cnt[p]) << 32) | (unsigned long long)(g0 + p);
 }
 
+template <bool LIST>
 __global__ void __launch_bounds__(MS_TOPK_THREADS) k_map_search_topk(const int *cnt, int Mc, long long g0, long long n,
-                                                                     unsigned long long *best, int n_best, int k) {
+                                                                     unsigned long long *best, int n_best, int k, const int *gl) {
   __shared__ int s_hist[RADIX_DIGITS];
   __shared__ unsigned long long s_sel[MS_TOPK_THREADS];
   __shared__ unsigned long long s_prefix, s_mask;
   __shared__ int s_need, s_n;
   const int tid = threadIdx.x, total = n_best + Mc, kk = total < k ? total : k;
-  auto key = [&](int j) { return j < n_best ? best[j] : search_key(cnt, j - n_best, g0, n); };
+  auto key = [&](int j) { return j < n_best ? best[j] : search_key<LIST>(cnt, gl, j - n_best, g0, n); };
   if (tid == 0) { s_prefix = 0; s_mask = 0; s_need = kk; s_n = 0; }
   __syncthreads();
   if (kk < total) {
@@ -728,7 +737,7 @@ __global__ void __launch_bounds__(MS_TOPK_THREADS) k_map_search_topk(const int *
   const unsigned long long T = s_prefix;
   for (int j = tid; j < total; j += MS_TOPK_THREADS) {
     const unsigned long long kj = key(j);
-    if (kj <= T) s_sel[atomicAdd(&s_n, 1)] = kj;
+    if (kj <= T && (!LIST || kj != MS_NO_POSE)) s_sel[atomicAdd(&s_n, 1)] = kj;
   }
   __syncthreads();
   if (tid >= s_n) s_sel[tid] = ~0ull;  // s_n == kk <= MS_TOPK_THREADS
@@ -743,6 +752,113 @@ __global__ void __launch_bounds__(MS_TOPK_THREADS) k_map_search_topk(const int *
       __syncthreads();
     }
   if (tid < kk) best[tid] = s_sel[tid];
+}
+
+// ---- svnicp_map_search, pruned path (DESIGN.md section 10e) ----------------------------------------------------------------
+// The translation axes are cut into blocks of b[0] x b[1] x b[2] consecutive grid indices; a block is (block coordinates, one
+// rotation index), id = c0 + nb[0] (c1 + nb[1] (c2 + nb[2] rot)), with rot the flat index of (i3, i4, i5) -- so g and id agree on
+// the rotation.  Edge blocks are partial: every block is treated as the virtual full block starting at c_a b[a].
+// k_map_search_bound_prep (R~ t~ of each block's centre) -> k_map_search_count at the bound radius (an upper bound of every
+// count in the block, see svnicp_map_search) -> k_map_search_keys + the export's LSD radix sort (best bound first) ->
+// per chunk of whole blocks: k_map_search_expand (grid poses) -> k_map_search_count -> k_map_search_violations -> the running top k.
+struct BlockSpec {
+  int b[3];   // grid indices per block on axes 0..2
+  int nb[3];  // blocks per axis: ceil(counts[a] / b[a])
+};
+
+// Centre of each block id0 .. id0 + Mc - 1: per translation axis the fp64 midpoint of the virtual block's first and last grid
+// values, the rotation's grid values, then map_pose -> Rt [Mc][12]
+__global__ void k_map_search_bound_prep(GridSpec gs, BlockSpec bs, long long id0, int Mc, svn::ScanConst sc, double *Rt) {
+  const int p = blockIdx.x * blockDim.x + threadIdx.x;
+  if (p >= Mc) return;
+  long long id = id0 + p;
+  double x[6], R[9];
+#pragma unroll
+  for (int a = 0; a < 3; a++) {
+    const long long first = (id % bs.nb[a]) * bs.b[a], last = first + bs.b[a] - 1;
+    id /= bs.nb[a];
+    x[a] = 0.5 * (grid_value(first, gs.counts[a], gs.steps[a]) + grid_value(last, gs.counts[a], gs.steps[a]));
+  }
+#pragma unroll
+  for (int a = 3; a < 6; a++) {
+    x[a] = grid_value((int)(id % gs.counts[a]), gs.counts[a], gs.steps[a]);
+    id /= gs.counts[a];
+  }
+  map_pose(x, sc, Rt + 12 * (size_t)p, R);
+}
+
+// Sort keys ((n - bound) << id_bits) | id, unique and ascending in (bound descending, id ascending); the values are the ids
+__global__ void k_map_search_keys(const int *bound, int B, long long n, int id_bits, unsigned long long *keys, int *ids) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= B) return;
+  keys[i] = ((unsigned long long)(n - bound[i]) << id_bits) | (unsigned long long)i;
+  ids[i] = i;
+}
+
+// The grid poses of the chunk's blocks ids[0 .. Mc / ppb): slot p = j ppb + l0 + b0 (l1 + b1 l2) of block ids[j].  A pose
+// inside the grid gets gl[p] = g and the R~ t~ k_map_search_prep gives that g (the same integers into the same arithmetic); a
+// slot past the edge of a partial block gets gl[p] = -1 and a NaN translation, so that k_map_search_count finds no inlier for it
+// without a probe.  The number of real poses is added to *counted.
+__global__ void k_map_search_expand(GridSpec gs, BlockSpec bs, const int *ids, int Mc, int ppb, svn::ScanConst sc, double *Rt, int *gl,
+                                    unsigned long long *counted) {
+  const int p = blockIdx.x * blockDim.x + threadIdx.x;
+  bool real = false;
+  if (p < Mc) {
+    const int j = p / ppb;
+    int l = p - j * ppb;
+    long long id = ids[j], g = 0, stride = 1;
+    double x[6], R[9];
+    real = true;
+#pragma unroll
+    for (int a = 0; a < 3; a++) {
+      const long long i = (id % bs.nb[a]) * bs.b[a] + l % bs.b[a];
+      id /= bs.nb[a];
+      l /= bs.b[a];
+      real &= i < gs.counts[a];
+      x[a] = grid_value(i, gs.counts[a], gs.steps[a]);
+      g += i * stride;
+      stride *= gs.counts[a];
+    }
+    g += id * stride;  // id is now the rotation index
+#pragma unroll
+    for (int a = 3; a < 6; a++) {
+      x[a] = grid_value((int)(id % gs.counts[a]), gs.counts[a], gs.steps[a]);
+      id /= gs.counts[a];
+    }
+    double *o = Rt + 12 * (size_t)p;
+    if (real) {
+      map_pose(x, sc, o, R);
+    } else {
+#pragma unroll
+      for (int c = 0; c < 12; c++) o[c] = __longlong_as_double(0x7FF8000000000000ll);  // NaN
+    }
+    gl[p] = real ? (int)g : -1;
+  }
+  const int c = __syncthreads_count(real);
+  if (threadIdx.x == 0 && c) atomicAdd(counted, (unsigned long long)c);
+}
+
+// The self-check of the bound: a counted pose whose count exceeds its block's bound (keys in walk order, from the chunk's first)
+__global__ void k_map_search_violations(const int *cnt, const int *gl, const unsigned long long *keys, int Mc, int ppb, long long n, int id_bits,
+                                        unsigned long long *violations) {
+  const int p = blockIdx.x * blockDim.x + threadIdx.x;
+  const bool bad = p < Mc && gl[p] >= 0 && cnt[p] > n - (long long)(keys[p / ppb] >> id_bits);
+  const int c = __syncthreads_count(bad);
+  if (threadIdx.x == 0 && c) atomicAdd(violations, (unsigned long long)c);
+}
+
+// max |coordinate| over the finite coordinates of the scan, as the bits of a non-negative double (ordered like the values).  A
+// point with a non-finite coordinate has a non-finite query at every pose and is an inlier nowhere, so it does not enter the slack.
+template <typename T>
+__global__ void k_max_abs_finite(const T *src, long long n3, unsigned long long *out) {
+  double v = 0.0;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n3; i += (long long)gridDim.x * blockDim.x) {
+    const double a = fabs((double)src[i]);
+    if (isfinite(a) && a > v) v = a;
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v = fmax(v, __shfl_xor_sync(0xffffffffu, v, o));
+  if ((threadIdx.x & 31) == 0 && v > 0.0) atomicMax(out, (unsigned long long)__double_as_longlong(v));
 }
 
 }  // namespace
@@ -780,6 +896,12 @@ struct svnicp_map_t {
   int *ms_cnt = nullptr;
   unsigned long long *ms_best = nullptr;
   size_t ms_rt_cap = 0, ms_cnt_cap = 0, ms_best_cap = 0;
+  // ... and of its pruned path, indexed by MP_*: the block bounds, the sort's key and id buffers and histograms, the chunk's
+  // grid indices, and device words; with the work done by the last successful call (svnicp_map_search_info)
+  void *mp[8] = {};
+  size_t mp_cap[8] = {};
+  long long ms_info[8] = {};
+  bool ms_info_valid = false;
   // svnicp_map_export / svnicp_map_import scratch (grown on demand; nothing above is touched by it), indexed by SN_*
   void *sn[11] = {};
   size_t sn_cap[11] = {};
@@ -875,6 +997,7 @@ void svnicp_map_destroy(svnicp_map m) {
   cudaFree(m->batch_in); cudaFree(m->wxyz); cudaFree(m->pt_slot); cudaFree(m->next); cudaFree(m->out);
   cudaFree(m->ev_src); cudaFree(m->ev_pose); cudaFree(m->ev_part); cudaFree(m->ev_out); cudaFree(m->ev_mask); cudaFree(m->ev_near);
   cudaFree(m->ms_rt); cudaFree(m->ms_cnt); cudaFree(m->ms_best);
+  for (void *p : m->mp) cudaFree(p);
   for (void *p : m->sn) cudaFree(p);
   if (m->h_counters) cudaFreeHost(m->h_counters);
   if (m->stream) cudaStreamDestroy(m->stream);
@@ -1120,6 +1243,213 @@ extern "C" int svnicp_map_evaluate(svnicp_map m, const void *source, int64_t n, 
 }
 
 // ---- svnicp_map_search --------------------------------------------------------------------------------------------------------
+// Scratch of the pruned path (DESIGN.md section 10e), grown on demand: 28 B per block (the bound, two key and two id buffers of
+// the sort) + 4 B per 16 blocks of radix histogram + 4 B per chunk pose + 32 B of words.
+enum { MP_BOUND, MP_KEY0, MP_KEY1, MP_ID0, MP_ID1, MP_HIST, MP_GL, MP_WORDS, MP_COUNT };
+static_assert(MP_COUNT == sizeof(svnicp_map_t::mp) / sizeof(void *), "one scratch buffer per MP_* index");
+// Selection rule: a grid of fewer than MS_POSES_PER_K * top_k poses takes the exhaustive path.  The walk cannot stop before k
+// poses are counted and stops only on a bound below the k-th count, which a k that large keeps low: on the 143 k-point scan
+// with k = 1024 of 3 969 poses nothing was pruned and the bound pass made the call 2 % slower (DESIGN.md section 10e).  The
+// define is for A/B builds through SVNICP_NVCC_DEFS, as the other SVN_* switches (0: every grid with blocks is pruned).
+#ifndef SVN_MS_POSES_PER_K
+#define SVN_MS_POSES_PER_K 16
+#endif
+constexpr long long MS_POSES_PER_K = SVN_MS_POSES_PER_K;
+
+static int mp_grow(svnicp_map m, int k, size_t bytes) { return ev_grow(m, &m->mp[k], &m->mp_cap[k], bytes > 0 ? bytes : 1); }
+
+static void launch_search_count(const MapDev &d, const void *src, int dtype_f64, int n, int wpp, int Mc, const double *Rt, double max_dist,
+                                double r, int *cnt, cudaStream_t st) {
+  const unsigned blocks = (unsigned)(((long long)Mc * wpp + MEV_THREADS / 32 - 1) / (MEV_THREADS / 32));
+  if (dtype_f64) k_map_search_count<double><<<blocks, MEV_THREADS, 0, st>>>(d, (const double *)src, n, wpp, Mc, Rt, max_dist, r, cnt);
+  else k_map_search_count<float><<<blocks, MEV_THREADS, 0, st>>>(d, (const float *)src, n, wpp, Mc, Rt, max_dist, r, cnt);
+}
+
+struct BlockPlan {
+  BlockSpec bs;
+  int ppb;            // poses per full block
+  long long B;        // blocks
+  double max_dist_b;  // the bound's threshold r_B^2, rounded up
+  double r_b;         // its box radius sqrt(max_dist_b) * MEV_MARGIN
+};
+
+// rho = max |R0 d| over the corners d = (+-h0, +-h1, +-h2) of the block's translation box, in fp64.  |R0 d| is convex in d, so
+// its maximum over the box is at a corner; R0 need not be orthonormal (nothing checks it).
+static double corner_radius(const double R0[9], const double h[3]) {
+  double rho = 0.0;
+  for (int c = 0; c < 8; c++) {
+    const double dv[3] = {c & 1 ? h[0] : -h[0], c & 2 ? h[1] : -h[1], c & 4 ? h[2] : -h[2]};
+    double s = 0.0;
+    for (int r = 0; r < 3; r++) {
+      const double v = R0[3 * r] * dv[0] + R0[3 * r + 1] * dv[1] + R0[3 * r + 2] * dv[2];
+      s += v * v;
+    }
+    rho = fmax(rho, sqrt(s));
+  }
+  return rho;
+}
+
+// Why no pose of a block counts more inliers than the block's bound.  Let c be the block's centre and x one of its poses; they
+// share omega, so map_pose gives them the same R~ (as values: x = 0 stores R0 itself, which equals R0 Exp(0) up to the sign
+// of zeros), and t~_x - t~_c = R0 (t_x - t_c) up to the rounding of map_pose.  t_x - t_c lies in the box [-h, h], h_a =
+// 0.5 (b_a - 1) steps[a], up to the rounding of grid_value and of the midpoint, so |R0 (t_x - t_c)| <= rho.  The queries of a
+// source point s, q_x and q_c, are formed by the same affine_row_fma from the same R~ and s, so |q_x - q_c| <= rho + delta,
+// where delta bounds every rounding above: each is a few ulp of |t0|, ||R0|| max|t| or ||R~ s|| <= ||R0|| |s| (fp64, relative
+// 2^-53 each), and delta = 1e-9 (1 + |t0| + ||R0||_F max|t| + ||R0||_F sqrt(3) max|s|) exceeds their sum by a factor of about
+// 10^6 (max|t| over the virtual blocks, which end at most 1.5 (counts - 1) steps from the centre; max|s| over the finite
+// coordinates: a point with a non-finite one has no finite query anywhere).  If s is an inlier of x, a stored p has
+// dist2(q_x, p) < max_dist; dist2 is within 4 ulp of |q_x - p|^2, so |q_x - p| < sqrt(max_dist) MEV_MARGIN and
+//   |q_c - p| <= |q_c - q_x| + |q_x - p| < sqrt(max_dist) MEV_MARGIN + rho + delta = r_B.
+// With max_dist_B = r_B^2 MEV_MARGIN, dist2(q_c, p) < max_dist_B (dist2 again within 4 ulp), and map_any_within at that
+// threshold with its box at sqrt(max_dist_B) MEV_MARGIN finds such a point (map_any_within's own argument): s is an inlier of
+// the bound query at c.  So count(x) <= bound(block), for every x of the block.  k_map_search_violations checks it on every
+// counted pose.
+//
+// Block sizes: equal metric half-extents H on the translation axes with counts > 1, b_a = min(counts[a], 1 + floor(2 H /
+// steps[a])) (a zero step adds nothing to rho and takes the finest positive step as its unit), and the largest H for which
+// ceil(box radius / voxel_size) <= MEV_MAX_REACH -- so the bound queries never reach map_any_within's whole-table sweep -- and a
+// block fits one chunk.  rho and the block count grow with H, so a bisection finds it.  False: the grid gets no blocks (every
+// b_a = 1) and takes the exhaustive path.
+static bool plan_blocks(double voxel_size, const int32_t counts[6], const double steps[6], const double R0[9], const double t0[3],
+                        double max_dist, double max_abs_s, int chunk, BlockPlan *pl) {
+  double nR = 0.0, tmax = 0.0, t0n = 0.0;
+  for (int i = 0; i < 9; i++) nR += R0[i] * R0[i];
+  for (int a = 0; a < 3; a++) {
+    const double e = 1.5 * (double)(counts[a] - 1) * steps[a];
+    tmax += e * e;
+    t0n += t0[a] * t0[a];
+  }
+  nR = sqrt(nR);
+  const double delta = 1e-9 * (1.0 + sqrt(t0n) + nR * sqrt(tmax) + nR * sqrt(3.0) * max_abs_s);
+  const double base = sqrt(max_dist) * MEV_MARGIN + delta;
+  if (!isfinite(base)) return false;
+  double s_ref = 0.0;
+  for (int a = 0; a < 3; a++)
+    if (counts[a] > 1 && steps[a] > 0 && (s_ref == 0.0 || steps[a] < s_ref)) s_ref = steps[a];
+  if (s_ref == 0.0) s_ref = voxel_size;
+  auto sizes = [&](double H, BlockPlan &q) {  // true when the bound's box stays within MEV_MAX_REACH and a block fits a chunk
+    double h[3];
+    long long ppb = 1;
+    for (int a = 0; a < 3; a++) {
+      const double f = 2.0 * H / (steps[a] > 0 ? steps[a] : s_ref);
+      const long long b = f >= (double)(counts[a] - 1) ? counts[a] : 1 + (long long)floor(f);
+      q.bs.b[a] = (int)b;
+      q.bs.nb[a] = (int)((counts[a] + b - 1) / b);
+      h[a] = 0.5 * (double)(b - 1) * steps[a];
+      ppb *= b;
+    }
+    const double rb = base + corner_radius(R0, h);
+    q.ppb = (int)(ppb < chunk ? ppb : chunk);
+    q.max_dist_b = rb * rb * MEV_MARGIN;
+    q.r_b = sqrt(q.max_dist_b) * MEV_MARGIN;
+    return ppb <= chunk && isfinite(q.r_b) && ceil(q.r_b / voxel_size) <= MEV_MAX_REACH;
+  };
+  double lo = 0.0, hi = 0.0;
+  for (int a = 0; a < 3; a++) hi = fmax(hi, (double)counts[a] * (steps[a] > 0 ? steps[a] : s_ref));
+  BlockPlan q;
+  if (!sizes(lo, q)) return false;
+  if (sizes(hi, q)) lo = hi;
+  for (int it = 0; it < 100 && lo < hi; it++) {
+    const double mid = 0.5 * (lo + hi);
+    if (mid <= lo || mid >= hi) break;
+    (sizes(mid, q) ? lo : hi) = mid;
+  }
+  sizes(lo, q);
+  if (q.ppb == 1) return false;
+  q.B = (long long)q.bs.nb[0] * q.bs.nb[1] * q.bs.nb[2] * counts[3] * counts[4] * counts[5];
+  *pl = q;
+  return true;
+}
+
+// The exhaustive path: every grid pose, in chunks of g
+static int search_exhaustive(svnicp_map m, const MapDev &d, const void *src, int dtype_f64, int n, int wpp, int chunk, const GridSpec &gs,
+                             const svn::ScanConst &sc, long long M, double max_dist, double r, int top_k, int32_t *out_counts,
+                             long long info[8]) {
+  cudaStream_t st = m->stream;
+  int n_best = 0;
+  for (long long g0 = 0; g0 < M; g0 += chunk) {
+    const int Mc = (int)(M - g0 < chunk ? M - g0 : chunk);
+    k_map_search_prep<<<(Mc + 127) / 128, 128, 0, st>>>(gs, g0, Mc, sc, m->ms_rt);
+    MCU(cudaMemsetAsync(m->ms_cnt, 0, (size_t)Mc * sizeof(int), st));
+    launch_search_count(d, src, dtype_f64, n, wpp, Mc, m->ms_rt, max_dist, r, m->ms_cnt, st);
+    k_map_search_topk<false><<<1, MS_TOPK_THREADS, 0, st>>>(m->ms_cnt, Mc, g0, n, m->ms_best, n_best, top_k, nullptr);
+    MCU(cudaGetLastError());
+    if (out_counts) MCU(cudaMemcpyAsync(out_counts + g0, m->ms_cnt, (size_t)Mc * sizeof(int), cudaMemcpyDeviceToHost, st));
+    n_best = n_best + Mc < top_k ? n_best + Mc : top_k;
+  }
+  const long long w[8] = {0, M, 0, 0, 0, M, 0, -1};
+  memcpy(info, w, sizeof(w));
+  return SVNICP_OK;
+}
+
+// The pruned path: block bounds, blocks sorted by bound, exact counts block by block until the next bound is below the k-th count
+static int search_pruned(svnicp_map m, const MapDev &d, const void *src, int dtype_f64, int n, int wpp, int chunk, const GridSpec &gs,
+                         const svn::ScanConst &sc, long long M, const BlockPlan &pl, double max_dist, double r, int top_k,
+                         long long info[8]) {
+  cudaStream_t st = m->stream;
+  const long long B = pl.B;
+  int id_bits = 1, n_bits = 1;
+  while ((1ll << id_bits) < B) id_bits++;
+  while ((1ll << n_bits) <= n) n_bits++;  // n - bound lies in [0, n]
+  const int n_tiles = (int)((B + RADIX_TILE - 1) / RADIX_TILE);
+  int rc;
+  if ((rc = mp_grow(m, MP_BOUND, B * 4)) || (rc = mp_grow(m, MP_KEY0, B * 8)) || (rc = mp_grow(m, MP_KEY1, B * 8)) ||
+      (rc = mp_grow(m, MP_ID0, B * 4)) || (rc = mp_grow(m, MP_ID1, B * 4)) || (rc = mp_grow(m, MP_HIST, (size_t)RADIX_DIGITS * n_tiles * 4)) ||
+      (rc = mp_grow(m, MP_GL, (size_t)chunk * 4)))
+    return rc;
+  int *bound = (int *)m->mp[MP_BOUND], *gl = (int *)m->mp[MP_GL], *hist = (int *)m->mp[MP_HIST];
+  unsigned long long *key[2] = {(unsigned long long *)m->mp[MP_KEY0], (unsigned long long *)m->mp[MP_KEY1]};
+  int *id[2] = {(int *)m->mp[MP_ID0], (int *)m->mp[MP_ID1]};
+  unsigned long long *words = (unsigned long long *)m->mp[MP_WORDS];  // [0] violations, [1] poses counted, [3] sink of the scans
+  MCU(cudaMemsetAsync(words, 0, 2 * sizeof(unsigned long long), st));
+  for (long long c0 = 0; c0 < B; c0 += chunk) {
+    const int Mc = (int)(B - c0 < chunk ? B - c0 : chunk);
+    k_map_search_bound_prep<<<(Mc + 127) / 128, 128, 0, st>>>(gs, pl.bs, c0, Mc, sc, m->ms_rt);
+    MCU(cudaMemsetAsync(bound + c0, 0, (size_t)Mc * sizeof(int), st));
+    launch_search_count(d, src, dtype_f64, n, wpp, Mc, m->ms_rt, pl.max_dist_b, pl.r_b, bound + c0, st);
+  }
+  k_map_search_keys<<<(unsigned)((B + 255) / 256), 256, 0, st>>>(bound, (int)B, n, id_bits, key[0], id[0]);
+  int a = 0;
+  for (int shift = 0; shift < id_bits + n_bits; shift += RADIX_BITS, a ^= 1) {
+    k_radix_hist<<<n_tiles, RADIX_THREADS, 0, st>>>(key[a], (int)B, shift, n_tiles, hist);
+    svn::k_scan_block_sums<int><<<1, SCAN_BLOCK, 0, st>>>(hist, RADIX_DIGITS * n_tiles, (long long *)words + 3);
+    k_radix_scatter<<<n_tiles, RADIX_THREADS, 0, st>>>(key[a], id[a], key[a ^ 1], id[a ^ 1], (int)B, shift, n_tiles, hist);
+  }
+  MCU(cudaGetLastError());
+  const unsigned long long *keys = key[a];
+  const int *ids = id[a];
+  // Stop rule: once k poses are counted, stop before the next block if its bound is strictly below the k-th count.  The blocks
+  // left have bounds no higher, so none of their poses can reach the k-th count; on an equal bound a pose with that count and a
+  // lower g might follow, so an equal bound does not stop the walk.
+  const int per = chunk / pl.ppb;
+  long long pos = 0;
+  int n_best = 0;
+  while (pos < B) {
+    const int nbc = (int)(B - pos < per ? B - pos : per), Mc = nbc * pl.ppb;
+    k_map_search_expand<<<(Mc + 127) / 128, 128, 0, st>>>(gs, pl.bs, ids + pos, Mc, pl.ppb, sc, m->ms_rt, gl, words + 1);
+    MCU(cudaMemsetAsync(m->ms_cnt, 0, (size_t)Mc * sizeof(int), st));
+    launch_search_count(d, src, dtype_f64, n, wpp, Mc, m->ms_rt, max_dist, r, m->ms_cnt, st);
+    k_map_search_violations<<<(Mc + 127) / 128, 128, 0, st>>>(m->ms_cnt, gl, keys + pos, Mc, pl.ppb, n, id_bits, words);
+    k_map_search_topk<true><<<1, MS_TOPK_THREADS, 0, st>>>(m->ms_cnt, Mc, 0, n, m->ms_best, n_best, top_k, gl);
+    MCU(cudaGetLastError());
+    n_best = n_best + Mc < top_k ? n_best + Mc : top_k;
+    pos += nbc;
+    if (pos < B && n_best == top_k) {
+      unsigned long long h[2];  // the next block's key, the k-th best key (MS_NO_POSE until k real poses are counted)
+      MCU(cudaMemcpyAsync(h, keys + pos, sizeof(h[0]), cudaMemcpyDeviceToHost, st));
+      MCU(cudaMemcpyAsync(h + 1, m->ms_best + top_k - 1, sizeof(h[1]), cudaMemcpyDeviceToHost, st));
+      MCU(cudaStreamSynchronize(st));
+      if (h[1] != MS_NO_POSE && n - (long long)(h[0] >> id_bits) < n - (long long)(h[1] >> 32)) break;
+    }
+  }
+  unsigned long long w[2];
+  MCU(cudaMemcpyAsync(w, words, sizeof(w), cudaMemcpyDeviceToHost, st));
+  MCU(cudaStreamSynchronize(st));
+  const long long v[8] = {1, M, pl.ppb, B, pos, (long long)w[1], B * n, (long long)w[0]};
+  memcpy(info, v, sizeof(v));
+  return SVNICP_OK;
+}
+
 extern "C" int svnicp_map_search(svnicp_map m, const void *source, int64_t n, int dtype_f64, int on_device, const double R0[9],
                                  const double t0[3], const int32_t counts[6], const double steps[6], double max_dist, int top_k,
                                  int64_t *out_index, double *out_poses_6xK, double *out_stats, int32_t *out_counts) {
@@ -1165,21 +1495,29 @@ extern "C" int svnicp_map_search(svnicp_map m, const void *source, int64_t n, in
   memcpy(gs.steps, steps, sizeof(gs.steps));
   const MapDev d = dev_view(m, m->cur);
   const double r = sqrt(max_dist) * MEV_MARGIN;  // k_map_eval's radius
-  int n_best = 0;
-  for (long long g0 = 0; g0 < M; g0 += chunk) {
-    const int Mc = (int)(M - g0 < chunk ? M - g0 : chunk);
-    k_map_search_prep<<<(Mc + 127) / 128, 128, 0, st>>>(gs, g0, Mc, sc, m->ms_rt);
-    MCU(cudaMemsetAsync(m->ms_cnt, 0, (size_t)Mc * sizeof(int), st));
-    const unsigned blocks = (unsigned)(((long long)Mc * wpp + MEV_THREADS / 32 - 1) / (MEV_THREADS / 32));
-    if (dtype_f64)
-      k_map_search_count<double><<<blocks, MEV_THREADS, 0, st>>>(d, (const double *)src, (int)n, wpp, Mc, m->ms_rt, max_dist, r, m->ms_cnt);
-    else
-      k_map_search_count<float><<<blocks, MEV_THREADS, 0, st>>>(d, (const float *)src, (int)n, wpp, Mc, m->ms_rt, max_dist, r, m->ms_cnt);
-    k_map_search_topk<<<1, MS_TOPK_THREADS, 0, st>>>(m->ms_cnt, Mc, g0, n, m->ms_best, n_best, top_k);
+  // Path: the per-pose counts need every pose counted; without them a grid with blocks takes the pruned path.  Both return the
+  // same bits.
+  BlockPlan pl;
+  bool pruned = false;
+  if (!out_counts && (counts[0] > 1 || counts[1] > 1 || counts[2] > 1) && M >= MS_POSES_PER_K * top_k) {
+    if ((rc = mp_grow(m, MP_WORDS, 4 * sizeof(unsigned long long)))) return rc;
+    unsigned long long *words = (unsigned long long *)m->mp[MP_WORDS], max_abs_bits;
+    MCU(cudaMemsetAsync(words + 2, 0, sizeof(unsigned long long), st));
+    const long long n3 = 3 * n;
+    const unsigned grid = (unsigned)(n3 < 256ll * m->sm_count * 4 ? (n3 + 255) / 256 : m->sm_count * 4);
+    if (dtype_f64) k_max_abs_finite<double><<<grid, 256, 0, st>>>((const double *)src, n3, words + 2);
+    else k_max_abs_finite<float><<<grid, 256, 0, st>>>((const float *)src, n3, words + 2);
     MCU(cudaGetLastError());
-    if (out_counts) MCU(cudaMemcpyAsync(out_counts + g0, m->ms_cnt, (size_t)Mc * sizeof(int), cudaMemcpyDeviceToHost, st));
-    n_best = n_best + Mc < top_k ? n_best + Mc : top_k;
+    MCU(cudaMemcpyAsync(&max_abs_bits, words + 2, sizeof(max_abs_bits), cudaMemcpyDeviceToHost, st));
+    MCU(cudaStreamSynchronize(st));
+    double max_abs_s;
+    memcpy(&max_abs_s, &max_abs_bits, sizeof(max_abs_s));
+    pruned = plan_blocks(m->voxel_size, counts, steps, R0, t0, max_dist, max_abs_s, chunk, &pl);
   }
+  long long info[8];
+  rc = pruned ? search_pruned(m, d, src, dtype_f64, (int)n, wpp, chunk, gs, sc, M, pl, max_dist, r, top_k, info)
+              : search_exhaustive(m, d, src, dtype_f64, (int)n, wpp, chunk, gs, sc, M, max_dist, r, top_k, out_counts, info);
+  if (rc) return rc;
   std::vector<unsigned long long> best((size_t)top_k);
   MCU(cudaMemcpyAsync(best.data(), m->ms_best, (size_t)top_k * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
   MCU(cudaStreamSynchronize(st));
@@ -1192,7 +1530,19 @@ extern "C" int svnicp_map_search(svnicp_map m, const void *source, int64_t n, in
     }
   }
   // the winners' statistics are svnicp_map_evaluate's by construction: the same call on the grid values (source already on device)
-  return svnicp_map_evaluate(m, src, n, dtype_f64, 1, R0, t0, top_k, out_poses_6xK, max_dist, out_stats, nullptr, nullptr, nullptr, nullptr);
+  rc = svnicp_map_evaluate(m, src, n, dtype_f64, 1, R0, t0, top_k, out_poses_6xK, max_dist, out_stats, nullptr, nullptr, nullptr, nullptr);
+  if (rc) return rc;
+  memcpy(m->ms_info, info, sizeof(info));  // svnicp_map_search_info: the last call that succeeded
+  m->ms_info_valid = true;
+  return SVNICP_OK;
+}
+
+extern "C" int svnicp_map_search_info(svnicp_map m, int64_t out8[8]) {
+  if (!m) return SVNICP_ERR_INVALID;
+  if (!out8) return mfail(m, SVNICP_ERR_INVALID, "svnicp_map_search_info: null output");
+  if (!m->ms_info_valid) return mfail(m, SVNICP_ERR_INVALID, "svnicp_map_search_info: no svnicp_map_search has succeeded on this map yet");
+  for (int i = 0; i < 8; i++) out8[i] = m->ms_info[i];
+  return SVNICP_OK;
 }
 
 // ---- svnicp_map_export / svnicp_map_import -----------------------------------------------------------------------------------

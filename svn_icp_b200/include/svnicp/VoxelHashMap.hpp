@@ -176,9 +176,10 @@ struct VoxelHashMap {
     std::vector<double> fitness, rmse;
     std::vector<int32_t> counts;
   };
-  /** Exhaustive search of a scan over a grid of poses around T0 (svnicp_map_search; no reference counterpart): counts[a] values
+  /** Exact search of a scan over a grid of poses around T0 (svnicp_map_search; no reference counterpart): counts[a] values
    *  x_a(i) = (i - 0.5 (counts[a] - 1)) steps[a] per axis of x = [t ; omega], flat index g with axis 0 fastest.  Score = the
-   *  inlier count of Evaluate; ranked by count descending, then g ascending.  Changes no state of the map. */
+   *  inlier count of Evaluate; ranked by count descending, then g ascending.  Changes no state of the map.  Without want_counts
+   *  a grid with translation blocks is searched by branch and bound (SearchInfo), with the same result. */
   SearchResult Search(const float *xyz, int64_t n, const InitialMean &T0, const int32_t (&counts)[6], const double (&steps)[6],
                       double max_dist, int top_k = 1, bool want_counts = false, bool on_device = false) {
     int64_t M = 1;  // capped at 2^31: the ABI refuses larger grids
@@ -202,6 +203,17 @@ struct VoxelHashMap {
       r.rmse.push_back(stats[3 * j + 2]);
     }
     return r;
+  }
+
+  /** The work of the last successful Search (svnicp_map_search_info): path 0 counted every pose, path 1 pruned by block bounds */
+  struct SearchWork {
+    int64_t path = 0, grid_poses = 0, poses_per_block = 0, blocks = 0, blocks_counted = 0, poses_counted = 0, bound_queries = 0,
+            violations = 0;
+  };
+  SearchWork SearchInfo() const {
+    int64_t v[8];
+    check(svnicp_map_search_info(m_, v), "SearchInfo");
+    return SearchWork{v[0], v[1], v[2], v[3], v[4], v[5], v[6], v[7]};
   }
 
   using Snapshot = MapSnapshot;
