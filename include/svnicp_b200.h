@@ -299,6 +299,25 @@ int svnicp_map_search(svnicp_map m, const void *source, int64_t n, int dtype_f64
  *           exactly, bound queries (blocks * n), bound violations (a pose counting more than its block's bound: always 0)}
  * On path 0: poses per block 0, blocks 0, blocks counted 0, poses counted M, bound queries 0, violations -1. */
 int svnicp_map_search_info(svnicp_map m, int64_t out8[8]);
+/* Gauss-Newton refinement of M pose hypotheses of one scan against the map (no reference counterpart): the continuous step after
+ * svnicp_map_search, whose out_poses may be passed in unchanged.  Source, pose convention, correspondences (exact nearest stored
+ * point with d^2 < max_dist), max_dist as the robust scale and the search-radius limit are those of svnicp_map_evaluate.
+ * One iteration of one pose (the single-particle SVN-ICP step, SVNICP.cpp:41-114 with P = 1, :268-279):
+ *   H, b = svnicp_map_evaluate's system at x (the same bits); delta = -H^-1 b (LDL^T, H carries + 1e-6 I);
+ *   R' = Exp(omega) Exp(delta_w), t' = R' J_l(delta_w) delta_t + t with J_l = I at delta_w = 0 exactly (the reference gives NaN);
+ *   x' = [t' ; Log(R')] with the principal Log (|omega| <= pi, accurate at pi); an exactly zero delta leaves x unchanged.
+ * A pose stops after the update with |delta|_2 < tol, or after `iterations` updates (tol = 0 runs them all); poses are independent.
+ *   out_poses [6][M]      the final x (may alias poses)
+ *   out_iterations [M]    updates applied
+ *   out_step [M]          |delta|_2 of the last update (may be NULL)
+ *   out_stats [M][3], out_H [M][36], out_b [M][6]  svnicp_map_evaluate at the final x, bit for bit (H, b may be NULL)
+ * Each pose's outputs are the same bits whatever M, its position, the call or the slot layout.  The loop runs on the map's
+ * stream without host round trips; blocking; changes no state of the map.  SVNICP_ERR_INVALID: svnicp_map_evaluate's argument
+ * errors, null poses / out_poses / out_iterations / out_stats, n_poses outside [1, 65536], iterations outside [1, 1000], a
+ * negative or non-finite tol. */
+int svnicp_map_refine(svnicp_map m, const void *source, int64_t n, int dtype_f64, int on_device, const double R0[9], const double t0[3],
+                      int n_poses, const double *poses_6xM, double max_dist, int iterations, double tol, double *out_poses_6xM,
+                      int32_t *out_iterations, double *out_step, double *out_stats, double *out_H, double *out_b);
 /* Snapshot of the map's content (no reference counterpart), to save a map and restore it bit for bit with svnicp_map_import:
  *   voxels [V][3] int32  voxel indices (vx, vy, vz) in ascending lexicographic order
  *   counts [V]    int32  points per voxel, 1 <= count <= max_pointscount

@@ -96,7 +96,7 @@ EXPORTS = [
     "svnicp_get_scan_info", "svnicp_get_tail_stamps", "svnicp_evaluate",
     "svnicp_map_create", "svnicp_map_destroy", "svnicp_map_last_error", "svnicp_map_clear", "svnicp_map_add_cloud", "svnicp_map_get",
     "svnicp_map_download", "svnicp_map_size", "svnicp_map_evaluate", "svnicp_map_search", "svnicp_map_search_info", "svnicp_map_export",
-    "svnicp_map_import", "svnicp_pre_create", "svnicp_pre_destroy", "svnicp_pre_last_error", "svnicp_pre_crop", "svnicp_pre_downsample_uniform",
+    "svnicp_map_import", "svnicp_map_refine", "svnicp_pre_create", "svnicp_pre_destroy", "svnicp_pre_last_error", "svnicp_pre_crop", "svnicp_pre_downsample_uniform",
     "svnicp_pre_to_f64", "svnicp_pre_download", "svnicp_pre_deskew", "svnicp_pose_compose",
     "svnicp_batch_create", "svnicp_batch_destroy", "svnicp_batch_last_error", "svnicp_batch_size", "svnicp_batch_stream", "svnicp_batch_align",
 ]
@@ -160,6 +160,7 @@ def _ARGTYPES(V, I, L, D):
         "svnicp_map_evaluate": [V, V, L, I, I, V, V, I, V, D, V, V, V, V, V], "svnicp_map_export": [V, V, V, V, L, L, I],
         "svnicp_map_search": [V, V, L, I, I, V, V, V, V, D, I, V, V, V, V], "svnicp_map_search_info": [V, V],
         "svnicp_map_import": [V, V, V, V, L, L, I],
+        "svnicp_map_refine": [V, V, L, I, I, V, V, I, V, D, I, D, V, V, V, V, V, V],
         "svnicp_pre_create": [V, L, I], "svnicp_pre_crop": [V, V, L, I, D, D, V, V, V],
         "svnicp_pre_downsample_uniform": [V, V, L, I, D, V, V], "svnicp_pre_to_f64": [V, V, L, V], "svnicp_pre_download": [V, V, L, V],
         "svnicp_pre_deskew": [V, V, L, I, V, I, I, V, V, V, V, V, V], "svnicp_pose_compose": [V, V, V, V, V],
@@ -742,6 +743,45 @@ class VoxelHashMap:
                                                 C.c_double(max_dist), C.c_int(k), _p(index), _p(poses), _p(stats), _p(grid)), "Search")
         return dict(index=index, poses=poses, count=stats[:, 0].astype(np.int64), fitness=stats[:, 1].copy(), rmse=stats[:, 2].copy(),
                     counts=grid.reshape(tuple(int(c) for c in cnt[::-1])) if grid is not None else None)
+
+    def Refine(self, source, R0, t0, poses, max_dist: float, iterations: int = 30, tol: float = SteinICPParam.convergence_threshold,
+               want_system: bool = False) -> dict:
+        """Gauss-Newton refinement of pose hypotheses of a scan against this map (svnicp_map_refine; no reference counterpart):
+        the continuous step after Search, whose poses may be passed in unchanged.  poses: (6,) or (6, M) x = [t ; omega]
+        relative to T0 = (R0, t0), as in Evaluate.  Each pose takes up to `iterations` single-particle SVN-ICP steps on exact
+        correspondences (delta = -H^-1 b, the update of SVNICP.cpp:268-279 with J_l = I at a zero rotation step, the principal
+        Log) and stops after the first step with |delta| < tol (tol = 0 runs every iteration).  Returns poses [6, M],
+        iterations [M] int64, step [M] (|delta| of the last step) and Evaluate's inliers, fitness, rmse at the final poses,
+        with want_system also H [M, 6, 6], b [M, 6], bit for bit.  A (6,) pose drops the M axis.  Changes no state of the map."""
+        a = np.asarray(source)
+        f64 = a.dtype != np.float32
+        a = np.ascontiguousarray(a, dtype=np.float64 if f64 else np.float32).reshape(-1, 3)
+        return self._refine(_p(a), len(a), f64, False, R0, t0, poses, max_dist, iterations, tol, want_system)
+
+    def RefineDevice(self, ptr: int, n: int, f64: bool, R0, t0, poses, max_dist: float, iterations: int = 30,
+                     tol: float = SteinICPParam.convergence_threshold, want_system: bool = False) -> dict:
+        """Refine for a device cloud: ptr to [n,3] float32 (f64 = False, e.g. a ScanPreprocessor output) or float64."""
+        return self._refine(C.c_void_p(ptr), n, f64, True, R0, t0, poses, max_dist, iterations, tol, want_system)
+
+    def _refine(self, src, n, f64, on_device, R0, t0, poses, max_dist, iterations, tol, want_system):
+        x = np.asarray(poses, dtype=np.float64)
+        single = x.ndim == 1
+        x = np.ascontiguousarray(x.reshape(6, -1))
+        M = x.shape[1]
+        out_x, its, step, stats = np.zeros((6, M)), np.zeros(M, dtype=np.int32), np.zeros(M), np.zeros((M, 3))
+        H = np.zeros((M, 6, 6)) if want_system else None
+        b = np.zeros((M, 6)) if want_system else None
+        self._check(self._lib.svnicp_map_refine(self._m, src, C.c_int64(n), C.c_int(int(f64)), C.c_int(int(on_device)),
+                                                _p(_f64(R0).reshape(9)), _p(_f64(t0).reshape(3)), C.c_int(M), _p(x),
+                                                C.c_double(max_dist), C.c_int(int(iterations)), C.c_double(tol), _p(out_x), _p(its),
+                                                _p(step), _p(stats), _p(H), _p(b)), "Refine")
+        out = dict(poses=out_x, iterations=its.astype(np.int64), step=step, inliers=stats[:, 0].astype(np.int64),
+                   fitness=stats[:, 1].copy(), rmse=stats[:, 2].copy())
+        if want_system:
+            out["H"], out["b"] = H, b
+        if single:
+            out = {k: (v[:, 0] if k == "poses" else v[0]) for k, v in out.items()}
+        return out
 
     SEARCH_INFO_FIELDS = ("path", "grid_poses", "poses_per_block", "blocks", "blocks_counted", "poses_counted", "bound_queries",
                           "violations")

@@ -190,6 +190,33 @@ __device__ inline void so3_log(const double R[9], double w[3]) {
   }
 }
 
+// Principal SO(3) Log, accurate up to and including an angle of pi (svnicp_map_refine; the scan path keeps so3_log and its
+// reference quirks).  a = atan2(|skew part| / 2, (tr R - 1) / 2) in [0, pi].  Up to pi / 2 the axis comes from the skew part
+// (R - R^T) / 2 = sin(a) [n]x; beyond it from the symmetric part (R + R^T) / 2 - cos(a) I = (1 - cos a) n n^T, whose largest
+// diagonal entry is at least (1 - cos a) / 3 >= 1 / 3, with the sign of n taken from the skew part.  |w| <= pi; at exactly pi
+// either sign is the same rotation.  tests/map_refine_oracle.c restates it.
+__device__ inline void so3_log_principal(const double R[9], double w[3]) {
+  const double v[3] = {R[7] - R[5], R[2] - R[6], R[3] - R[1]};  // 2 sin(a) n
+  const double s = 0.5 * sqrt(v[0] * v[0] + v[1] * v[1] + v[2] * v[2]);
+  const double c = 0.5 * (R[0] + R[4] + R[8] - 1.0);
+  const double a = atan2(s, c);
+  if (c >= 0.0) {
+    const double f = s > 0.0 ? 0.5 * a / s : 0.5;  // a / sin(a) -> 1 as a -> 0
+    w[0] = f * v[0]; w[1] = f * v[1]; w[2] = f * v[2];
+    return;
+  }
+  const double B[9] = {R[0] - c, 0.5 * (R[1] + R[3]), 0.5 * (R[2] + R[6]),
+                       0.5 * (R[1] + R[3]), R[4] - c, 0.5 * (R[5] + R[7]),
+                       0.5 * (R[2] + R[6]), 0.5 * (R[5] + R[7]), R[8] - c};
+  const int k = (B[0] >= B[4] && B[0] >= B[8]) ? 0 : (B[4] >= B[8] ? 1 : 2);
+  double n[3];  // row k: (1 - cos a) n_k n
+#pragma unroll
+  for (int j = 0; j < 3; j++) n[j] = k == 0 ? B[j] : (k == 1 ? B[3 + j] : B[6 + j]);
+  const double nn = sqrt(n[0] * n[0] + n[1] * n[1] + n[2] * n[2]);
+  const double f = ((n[0] * v[0] + n[1] * v[1] + n[2] * v[2]) < 0.0 ? -a : a) / nn;
+  w[0] = f * n[0]; w[1] = f * n[1]; w[2] = f * n[2];
+}
+
 // ZYX Euler angles x6[3..5] = (roll, pitch, yaw) -> R, exactly as SVGDICP::to_rotation_tensor (SVGDICP.cpp:226-260)
 __device__ __forceinline__ void euler_R(const double *x6, double *R) {
   double sr, cr, sp, cp, sy, cy;

@@ -22,6 +22,10 @@
 // (source point, pose) with an early exit (k_map_search_count), integer counts per pose and a deterministic running top k
 // (k_map_search_topk); the winners' statistics come from svnicp_map_evaluate itself.
 //
+// svnicp_map_refine (DESIGN.md section 10f) runs Gauss-Newton steps of many poses against the table: k_map_refine_eval (the
+// sums of k_map_eval, each search seeded with the previous iteration's map point), k_eval_fin, k_map_refine_step (solve and
+// update), the whole loop enqueued without a host round trip; the final statistics come from svnicp_map_evaluate itself.
+//
 // svnicp_map_export / svnicp_map_import (DESIGN.md section 10c) save and restore the content in canonical form -- voxels in
 // ascending (vx, vy, vz), each voxel's points in stored order -- independent of the slot layout: a radix sort of the live keys
 // on the way out, a rebuild into the twin table with full validation on the way in.
@@ -32,6 +36,7 @@
 #include <stdio.h>
 #include <string.h>
 
+#include <algorithm>
 #include <string>
 #include <vector>
 
@@ -573,6 +578,181 @@ __global__ void __launch_bounds__(MEV_THREADS, SYS ? 4 : 8) k_map_eval(MapDev m,
   }
 }
 
+// ---- svnicp_map_refine (DESIGN.md section 10f) --------------------------------------------------------------------------------
+// Per pose block and iteration: k_map_refine_eval (k_map_eval<T, true>'s sums of the active poses) -> k_eval_fin (the fixed-order
+// sum and gn_assemble of svnicp_map_evaluate, unchanged) -> k_map_refine_step (solve, update, stop rule, next R~ t~).
+// Seeding (SVN_RF_SEED, default on; the A/B measurement is in DESIGN.md section 10f): each (pose, point) keeps the map point it
+// chose last iteration and starts the next search from it.
+#ifndef SVN_RF_SEED
+#define SVN_RF_SEED 1
+#endif
+constexpr bool RF_SEED = SVN_RF_SEED != 0;
+constexpr int RF_MAX_BLOCK = 1024;              // poses per block at most (k_map_eval_prep runs one thread per pose)
+constexpr size_t RF_BLOCK_BYTES = 64ull << 20;  // partials + seeds of one pose block, at most (one pose exceeds it only beyond ~5 M points)
+
+// k_map_refine_eval's share of one source point in the per-pose sums, once its nearest point s is settled: the arithmetic of
+// k_map_eval's loop body, which keeps its own copy so that its SASS stays as measured in DESIGN.md section 10b (a shared helper
+// changes its instruction schedule).
+// Queries without a correspondence (no point with d^2 < max_dist, or a non-finite query) add only +1 to W (Q2).
+template <bool SYS>
+__device__ __forceinline__ void map_eval_accum(const NearestState &s, double x, double y, double z, const double Rtl[9],
+                                               const svn::ScanConst &sc, double D, double (&acc)[svn::EV_NS]) {
+  if (!s.found) {
+    if (SYS) acc[0] += 1.0;  // masked: +1 on the translation block (Q2); nothing else, so a NaN never reaches the sums
+    return;
+  }
+  acc[16] += 1.0;
+  acc[17] += s.bd;
+  if (SYS) {
+    double sp[3], w[3];
+#pragma unroll
+    for (int a = 0; a < 3; a++) {
+      sp[a] = fma(sc.R0[3 * a], x, fma(sc.R0[3 * a + 1], y, sc.R0[3 * a + 2] * z));  // s' = R0 s
+      w[a] = fma(Rtl[3 * a], x, fma(Rtl[3 * a + 1], y, Rtl[3 * a + 2] * z));        // R~ s
+    }
+    const double e[3] = {s.q[0] - (double)s.bx, s.q[1] - (double)s.by, s.q[2] - (double)s.bz};
+    const double wq = D / (D + 3.0 * sqrt(s.bd));
+    const double rho = wq * wq;  // (D / (D + 3 |e|))^2, SVNICP.cpp:120-122
+    acc[0] += rho;
+    const double g[3] = {rho * sp[0], rho * sp[1], rho * sp[2]};
+    acc[1] += g[0]; acc[2] += g[1]; acc[3] += g[2];
+    acc[4] += g[0] * sp[0]; acc[5] += g[0] * sp[1]; acc[6] += g[0] * sp[2];
+    acc[7] += g[1] * sp[1]; acc[8] += g[1] * sp[2]; acc[9] += g[2] * sp[2];
+    const double f[3] = {rho * e[0], rho * e[1], rho * e[2]};
+    acc[10] += f[0]; acc[11] += f[1]; acc[12] += f[2];
+    acc[13] += w[1] * f[2] - w[2] * f[1];
+    acc[14] += w[2] * f[0] - w[0] * f[2];
+    acc[15] += w[0] * f[1] - w[1] * f[0];
+  }
+}
+
+// The CTA's partial slot of pose p, in k_map_eval's order: a fixed butterfly per warp, then the warps in ascending order
+__device__ __forceinline__ void map_eval_store(const double (&acc)[svn::EV_NS], double (&s_w)[MEV_THREADS / 32][svn::EV_NS], double *part,
+                                               int p, int MB) {
+  using svn::EV_NS;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+  for (int j = 0; j < EV_NS; j++) {
+    const double v = svn::warp_sum(acc[j]);
+    if (lane == 0) s_w[warp][j] = v;
+  }
+  __syncthreads();
+  if (threadIdx.x < EV_NS) {
+    double t = 0.0;
+#pragma unroll
+    for (int w = 0; w < MEV_THREADS / 32; w++) t += s_w[w][threadIdx.x];
+    part[((size_t)blockIdx.x * MB + p) * EV_NS + threadIdx.x] = t;
+  }
+}
+
+// The seeded search gives map_nearest's result bit for bit.  The seed is a stored point (the map does not change during a
+// call).  When its d^2 at the new query is < max_dist, it starts the search as the current best, and the box radius becomes
+// sqrt(d^2_seed) * MEV_MARGIN.  Then:
+//  - The true nearest point p* has d^2(p*) <= d^2_seed.  By the box argument of box_axis, which holds for any radius that bounds
+//    the nearest distance with the margin over dist2's rounding, the box holds p*.  map_nearest itself relies on the same
+//    argument when it shrinks the box to the best distance found in the query's own voxel.
+//  - Every visit compares (d^2, lexicographic (x, y, z)), a total order on the data alone, and keeps the smaller; the seed's
+//    own voxel lies inside the box, so revisiting the seed leaves an exact tie with itself unchanged.  The result is the
+//    minimum of the visited set plus the seed, which contains p*: p* itself.
+//  - A seed with d^2 >= max_dist, NaN (no point last iteration: the store writes NaN) or a non-finite query is not used, and
+//    the search is map_nearest's from max_dist.
+// The inlier bit, d^2 and the chosen point are therefore those of k_map_eval, and so are the sums.
+template <typename T>
+__global__ void __launch_bounds__(MEV_THREADS, 4) k_map_refine_eval(MapDev m, const T *__restrict__ src, int n, const double *__restrict__ Rt,
+                                                                    svn::ScanConst sc, double max_dist, double r, const int *__restrict__ active,
+                                                                    double *part, float *seed) {
+  using svn::EV_NS;
+  __shared__ double s_w[MEV_THREADS / 32][EV_NS];
+  const int p = blockIdx.y, MB = gridDim.y;
+  if (!active[p]) return;  // the whole CTA: the pose stopped
+  const double *P = Rt + 12 * p;
+  double Rtl[9], ttl[3];
+#pragma unroll
+  for (int i = 0; i < 9; i++) Rtl[i] = P[i];
+#pragma unroll
+  for (int i = 0; i < 3; i++) ttl[i] = P[9 + i];
+  double acc[EV_NS];
+#pragma unroll
+  for (int j = 0; j < EV_NS; j++) acc[j] = 0.0;
+  for (int i = blockIdx.x * MEV_THREADS + threadIdx.x; i < n; i += gridDim.x * MEV_THREADS) {
+    const double x = (double)src[3 * (size_t)i], y = (double)src[3 * (size_t)i + 1], z = (double)src[3 * (size_t)i + 2];
+    NearestState s;
+#pragma unroll
+    for (int a = 0; a < 3; a++) s.q[a] = svn::affine_row_fma(Rtl, ttl, a, x, y, z);
+    s.bd = max_dist;
+    s.bx = s.by = s.bz = 0.f;
+    s.found = false;
+    float *sd = RF_SEED ? seed + ((size_t)p * n + i) * 3 : nullptr;
+    if (isfinite(s.q[0]) && isfinite(s.q[1]) && isfinite(s.q[2])) {
+      double rs = r;
+      if (RF_SEED) {
+        const float px = sd[0], py = sd[1], pz = sd[2];
+        const double mp[3] = {(double)px, (double)py, (double)pz};
+        const double d = svn::dist2(s.q, mp);
+        if (d < max_dist) {
+          s.bd = d; s.bx = px; s.by = py; s.bz = pz; s.found = true;
+          rs = fmin(r, sqrt(d) * MEV_MARGIN);
+        }
+      }
+      map_nearest(m, rs, s);
+    }
+    if (RF_SEED) {
+      const float nan = __int_as_float(0x7fffffff);
+      sd[0] = s.found ? s.bx : nan; sd[1] = s.found ? s.by : nan; sd[2] = s.found ? s.bz : nan;
+    }
+    map_eval_accum<true>(s, x, y, z, Rtl, sc, max_dist, acc);
+  }
+  map_eval_store(acc, s_w, part, p, MB);
+}
+
+// One thread per pose of the block: delta = -H^-1 b from k_eval_fin's H and b (ldl_solve6_reg), the update of SVNICP.cpp:268-279
+// in tail2.cu's operation order with J_l = I at delta_omega = 0 (not the reference's NaN, Q7), x' = [t' ; so3_log_principal(R')],
+// |delta| in the order of tail2.cu, then the stop rule (update, then test) and R~ t~, R_p of x' for the next iteration.
+// An exactly zero delta (e.g. no inlier: b = 0) leaves x as it is, bit for bit.
+__global__ void k_map_refine_step(const double *__restrict__ ev, int MB, svn::ScanConst sc, int iterations, double tol, int *active,
+                                  int *iters, double *step, double *x6, double *Rt, double *Rp) {
+  using svn::EV_OUT;
+  const int p = blockIdx.x * blockDim.x + threadIdx.x;
+  if (p >= MB || !active[p]) return;
+  const double *o = ev + (size_t)EV_OUT * p;
+  double A[36], d[6];
+#pragma unroll
+  for (int i = 0; i < 36; i++) A[i] = o[3 + i];
+#pragma unroll
+  for (int i = 0; i < 6; i++) d[i] = o[39 + i];
+  svn::ldl_solve6_reg(A, d);
+#pragma unroll
+  for (int i = 0; i < 6; i++) d[i] = -d[i];
+  double *x = x6 + 6 * p;
+  const bool zero = d[0] == 0.0 && d[1] == 0.0 && d[2] == 0.0 && d[3] == 0.0 && d[4] == 0.0 && d[5] == 0.0;
+  if (!zero) {
+    double dR[9], Jl[9], Rn[9], dt[3], t[3], w[3];
+    const double *R = Rp + 9 * p;  // Exp(omega) of the current x (map_pose)
+    svn::so3_exp(d + 3, dR, Jl);
+    const bool rot0 = d[3] == 0.0 && d[4] == 0.0 && d[5] == 0.0;
+#pragma unroll
+    for (int r = 0; r < 3; r++) dt[r] = rot0 ? d[r] : Jl[3 * r] * d[0] + Jl[3 * r + 1] * d[1] + Jl[3 * r + 2] * d[2];
+#pragma unroll
+    for (int r = 0; r < 3; r++)
+#pragma unroll
+      for (int c = 0; c < 3; c++) Rn[3 * r + c] = R[3 * r] * dR[c] + R[3 * r + 1] * dR[3 + c] + R[3 * r + 2] * dR[6 + c];
+#pragma unroll
+    for (int r = 0; r < 3; r++) t[r] = (Rn[3 * r] * dt[0] + Rn[3 * r + 1] * dt[1] + Rn[3 * r + 2] * dt[2]) + x[r];
+    svn::so3_log_principal(Rn, w);
+#pragma unroll
+    for (int q = 0; q < 3; q++) { x[q] = t[q]; x[3 + q] = w[q]; }
+  }
+  const double dn = sqrt(d[0] * d[0] + d[1] * d[1] + d[2] * d[2] + d[3] * d[3] + d[4] * d[4] + d[5] * d[5]);
+  const int it = iters[p] + 1;
+  iters[p] = it;
+  step[p] = dn;
+  if (dn < tol || it >= iterations) active[p] = 0;
+  double R[9];
+  map_pose(x, sc, Rt + 12 * p, R);
+#pragma unroll
+  for (int i = 0; i < 9; i++) Rp[9 * p + i] = R[i];
+}
+
 // ---- svnicp_map_search (DESIGN.md section 10d) -------------------------------------------------------------------------------
 // Per chunk of grid poses: k_map_search_prep (grid value -> R~ t~ by map_pose) -> k_map_search_count (inlier count per pose)
 // -> k_map_search_topk (running top k of the keys ((n - count) << 32) | g).
@@ -905,6 +1085,9 @@ struct svnicp_map_t {
   // svnicp_map_export / svnicp_map_import scratch (grown on demand; nothing above is touched by it), indexed by SN_*
   void *sn[11] = {};
   size_t sn_cap[11] = {};
+  // svnicp_map_refine scratch (grown on demand; nothing above is touched by it), indexed by RF_*
+  void *rf[9] = {};
+  size_t rf_cap[9] = {};
   int sm_count = 148;
   cudaStream_t stream = nullptr;
   std::string err;
@@ -999,6 +1182,7 @@ void svnicp_map_destroy(svnicp_map m) {
   cudaFree(m->ms_rt); cudaFree(m->ms_cnt); cudaFree(m->ms_best);
   for (void *p : m->mp) cudaFree(p);
   for (void *p : m->sn) cudaFree(p);
+  for (void *p : m->rf) cudaFree(p);
   if (m->h_counters) cudaFreeHost(m->h_counters);
   if (m->stream) cudaStreamDestroy(m->stream);
   delete m;
@@ -1543,6 +1727,94 @@ extern "C" int svnicp_map_search_info(svnicp_map m, int64_t out8[8]) {
   if (!m->ms_info_valid) return mfail(m, SVNICP_ERR_INVALID, "svnicp_map_search_info: no svnicp_map_search has succeeded on this map yet");
   for (int i = 0; i < 8; i++) out8[i] = m->ms_info[i];
   return SVNICP_OK;
+}
+
+// ---- svnicp_map_refine ----------------------------------------------------------------------------------------------------------
+// Scratch per pose block of MB poses: x [MB][6], R~ t~ [MB][12], R_p [MB][9], k_eval_fin's output [MB][EV_OUT], the active flags,
+// iteration counts and last |delta| (about 640 B per pose), the partials [parts][MB][EV_NS] and the seeds [MB][n][3] float.
+enum { RF_X, RF_RT, RF_RP, RF_OUT, RF_ACTIVE, RF_ITERS, RF_STEP, RF_PART, RF_SEEDS, RF_COUNT };
+static_assert(RF_COUNT == sizeof(svnicp_map_t::rf) / sizeof(void *), "one scratch buffer per RF_* index");
+
+static int rf_grow(svnicp_map m, int k, size_t bytes) { return ev_grow(m, &m->rf[k], &m->rf_cap[k], bytes > 0 ? bytes : 1); }
+
+extern "C" int svnicp_map_refine(svnicp_map m, const void *source, int64_t n, int dtype_f64, int on_device, const double R0[9],
+                                 const double t0[3], int n_poses, const double *poses_6xM, double max_dist, int iterations, double tol,
+                                 double *out_poses_6xM, int32_t *out_iterations, double *out_step, double *out_stats, double *out_H,
+                                 double *out_b) {
+  using svn::EV_BLOCK;
+  using svn::EV_NS;
+  using svn::EV_OUT;
+  if (!m) return SVNICP_ERR_INVALID;
+  if (!source || !R0 || !t0 || !poses_6xM || !out_poses_6xM || !out_iterations || !out_stats)
+    return mfail(m, SVNICP_ERR_INVALID, "svnicp_map_refine: null source, R0, t0, poses, out_poses, out_iterations or out_stats");
+  int rc = check_scan_args(m, "svnicp_map_refine", n, max_dist);
+  if (rc) return rc;
+  if (n_poses < 1 || n_poses > 65536) return mfail(m, SVNICP_ERR_INVALID, "svnicp_map_refine: n_poses must be in [1, 65536]");
+  if (iterations < 1 || iterations > 1000) return mfail(m, SVNICP_ERR_INVALID, "svnicp_map_refine: iterations must be in [1, 1000]");
+  if (!isfinite(tol) || tol < 0) return mfail(m, SVNICP_ERR_INVALID, "svnicp_map_refine: tol must be finite and >= 0");
+  MCU(cudaSetDevice(m->device));
+  cudaStream_t st = m->stream;
+  const int ni = (int)n, M = n_poses;
+  int parts = (int)((n + MEV_THREADS - 1) / MEV_THREADS);  // svnicp_map_evaluate's partial slots: the same sums
+  if (parts > m->sm_count * MEV_CTAS_PER_SM) parts = m->sm_count * MEV_CTAS_PER_SM;
+  const size_t per_pose = (size_t)parts * EV_NS * sizeof(double) + (RF_SEED ? (size_t)n * 3 * sizeof(float) : 0);
+  const size_t by_bytes = RF_BLOCK_BYTES / per_pose;
+  const int mb_max = (int)std::min<size_t>({(size_t)M, (size_t)RF_MAX_BLOCK, std::max<size_t>(by_bytes, 1)});
+  const size_t esz = dtype_f64 ? sizeof(double) : sizeof(float);
+  const size_t mb = (size_t)mb_max;
+  if ((rc = rf_grow(m, RF_X, mb * 6 * sizeof(double))) || (rc = rf_grow(m, RF_RT, mb * 12 * sizeof(double))) ||
+      (rc = rf_grow(m, RF_RP, mb * 9 * sizeof(double))) || (rc = rf_grow(m, RF_OUT, mb * EV_OUT * sizeof(double))) ||
+      (rc = rf_grow(m, RF_ACTIVE, mb * sizeof(int))) || (rc = rf_grow(m, RF_ITERS, mb * sizeof(int))) ||
+      (rc = rf_grow(m, RF_STEP, mb * sizeof(double))) || (rc = rf_grow(m, RF_PART, (size_t)parts * mb * EV_NS * sizeof(double))) ||
+      (RF_SEED && (rc = rf_grow(m, RF_SEEDS, mb * (size_t)n * 3 * sizeof(float)))) ||
+      (!on_device && (rc = ev_grow(m, &m->ev_src, &m->ev_src_cap, (size_t)n * 3 * esz))))
+    return rc;
+  const void *src = source;
+  if (!on_device) {
+    MCU(cudaMemcpyAsync(m->ev_src, source, (size_t)n * 3 * esz, cudaMemcpyHostToDevice, st));
+    src = m->ev_src;
+  }
+  svn::ScanConst sc;
+  memcpy(sc.R0, R0, sizeof(sc.R0));
+  memcpy(sc.t0, t0, sizeof(sc.t0));
+  const MapDev d = dev_view(m, m->cur);
+  const double r = sqrt(max_dist) * MEV_MARGIN;  // k_map_eval's radius
+  double *x = (double *)m->rf[RF_X], *Rt = (double *)m->rf[RF_RT], *Rp = (double *)m->rf[RF_RP], *ev = (double *)m->rf[RF_OUT];
+  double *part = (double *)m->rf[RF_PART], *step = (double *)m->rf[RF_STEP];
+  int *active = (int *)m->rf[RF_ACTIVE], *iters = (int *)m->rf[RF_ITERS];
+  float *seed = (float *)m->rf[RF_SEEDS];
+  std::vector<double> hx(mb * 6), hstep(mb);
+  std::vector<int> hit(mb);
+  for (int m0 = 0; m0 < M; m0 += mb_max) {
+    const int MB = M - m0 < mb_max ? M - m0 : mb_max;
+    for (int j = 0; j < MB; j++)
+      for (int c = 0; c < 6; c++) hx[(size_t)6 * j + c] = poses_6xM[(size_t)c * M + m0 + j];
+    MCU(cudaMemcpyAsync(x, hx.data(), (size_t)6 * MB * sizeof(double), cudaMemcpyHostToDevice, st));
+    MCU(cudaMemsetAsync(iters, 0, (size_t)MB * sizeof(int), st));
+    if (RF_SEED) MCU(cudaMemsetAsync(seed, 0xFF, (size_t)MB * n * 3 * sizeof(float), st));  // NaN: no seed
+    k_fill_i32<<<(MB + 255) / 256, 256, 0, st>>>(active, 1, (size_t)MB);
+    for (int j = 0; j < MB; j += EV_BLOCK)
+      k_map_eval_prep<<<1, EV_BLOCK, 0, st>>>(x + 6 * j, MB - j < EV_BLOCK ? MB - j : EV_BLOCK, sc, Rt + 12 * j, Rp + 9 * j);
+    const dim3 grid((unsigned)parts, (unsigned)MB);
+    for (int it = 0; it < iterations; it++) {
+      if (dtype_f64) k_map_refine_eval<double><<<grid, MEV_THREADS, 0, st>>>(d, (const double *)src, ni, Rt, sc, max_dist, r, active, part, seed);
+      else k_map_refine_eval<float><<<grid, MEV_THREADS, 0, st>>>(d, (const float *)src, ni, Rt, sc, max_dist, r, active, part, seed);
+      svn::launch_eval_fin(part, parts, MB, ni, sc, Rp, ev, st);  // a stopped pose's row is stale and unread
+      k_map_refine_step<<<(MB + 127) / 128, 128, 0, st>>>(ev, MB, sc, iterations, tol, active, iters, step, x, Rt, Rp);
+    }
+    MCU(cudaGetLastError());
+    MCU(cudaMemcpyAsync(hx.data(), x, (size_t)6 * MB * sizeof(double), cudaMemcpyDeviceToHost, st));
+    MCU(cudaMemcpyAsync(hit.data(), iters, (size_t)MB * sizeof(int), cudaMemcpyDeviceToHost, st));
+    MCU(cudaMemcpyAsync(hstep.data(), step, (size_t)MB * sizeof(double), cudaMemcpyDeviceToHost, st));
+    MCU(cudaStreamSynchronize(st));  // the host block buffers are refilled next
+    for (int j = 0; j < MB; j++) {
+      for (int c = 0; c < 6; c++) out_poses_6xM[(size_t)c * M + m0 + j] = hx[(size_t)6 * j + c];
+      out_iterations[m0 + j] = hit[j];
+      if (out_step) out_step[m0 + j] = hstep[j];
+    }
+  }
+  // the statistics and the system at the final poses are svnicp_map_evaluate's by construction: the same call (source on device)
+  return svnicp_map_evaluate(m, src, n, dtype_f64, 1, R0, t0, M, out_poses_6xM, max_dist, out_stats, out_H, out_b, nullptr, nullptr);
 }
 
 // ---- svnicp_map_export / svnicp_map_import -----------------------------------------------------------------------------------

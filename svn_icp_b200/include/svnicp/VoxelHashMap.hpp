@@ -205,6 +205,43 @@ struct VoxelHashMap {
     return r;
   }
 
+  /** Result of Refine, per pose in input order: the final x (poses [6][M]), the updates applied, |delta| of the last one, and
+   *  Evaluate's inliers / fitness / rmse (and with want_system H [M][36], b [M][6]) at the final x, bit for bit. */
+  struct RefineResult {
+    int n_poses = 0;
+    std::vector<double> poses;
+    std::vector<int32_t> iterations;
+    std::vector<double> step;
+    std::vector<int64_t> inliers;
+    std::vector<double> fitness, rmse, H, b;
+  };
+  /** Gauss-Newton refinement of M pose hypotheses of a scan against this map (svnicp_map_refine; no reference counterpart): up
+   *  to `iterations` single-particle SVN-ICP steps per pose on exact correspondences, stopping after the first step with
+   *  |delta| < tol.  poses_6xM: [6][M] x relative to T0, as in Evaluate; Search's poses may be passed in unchanged.  Chain two
+   *  calls to tighten max_dist.  Changes no state of the map. */
+  RefineResult Refine(const float *xyz, int64_t n, const InitialMean &T0, const std::vector<double> &poses_6xM, double max_dist,
+                      int iterations = 30, double tol = 1e-5, bool want_system = false, bool on_device = false) {
+    if (poses_6xM.empty() || poses_6xM.size() % 6 != 0) throw Error("Refine: poses must hold 6*M doubles");
+    RefineResult r;
+    r.n_poses = (int)(poses_6xM.size() / 6);
+    const size_t M = (size_t)r.n_poses;
+    r.poses.resize(6 * M);
+    r.iterations.resize(M);
+    r.step.resize(M);
+    std::vector<double> stats(3 * M);
+    if (want_system) { r.H.resize(36 * M); r.b.resize(6 * M); }
+    check(svnicp_map_refine(m_, xyz, n, 0, on_device, T0.R.data(), T0.t.data(), r.n_poses, poses_6xM.data(), max_dist, iterations, tol,
+                            r.poses.data(), r.iterations.data(), r.step.data(), stats.data(), want_system ? r.H.data() : nullptr,
+                            want_system ? r.b.data() : nullptr),
+          "Refine");
+    for (size_t m = 0; m < M; m++) {
+      r.inliers.push_back((int64_t)stats[3 * m]);
+      r.fitness.push_back(stats[3 * m + 1]);
+      r.rmse.push_back(stats[3 * m + 2]);
+    }
+    return r;
+  }
+
   /** The work of the last successful Search (svnicp_map_search_info): path 0 counted every pose, path 1 pruned by block bounds */
   struct SearchWork {
     int64_t path = 0, grid_poses = 0, poses_per_block = 0, blocks = 0, blocks_counted = 0, poses_counted = 0, bound_queries = 0,
